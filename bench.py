@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the SoW training hot path on B200 (contract: see the task's bench.py section).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Metric (BASELINE.json): SoW Llama-350M r=50 bf16 pre-training tokens/s (reference definition, simple_train.py:
@@ -51,7 +51,37 @@ def parse_args():
     ap.add_argument("--no-extra-rows", action="store_true", help="skip the batch-16/64 and torch.compile rows")
     ap.add_argument("--no-fused-optimizer", action="store_true")
     ap.add_argument("--profile-steps", type=int, default=3)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32): its loss and "
+                         "every parameter after the optimizer update, at most 64 MB in all")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+DUMP_BYTES = 60_000_000          # float32 data; with the .npy headers a dump stays under 64 MB
+
+
+def dump_outputs(out_dir, loss, model):
+    """The results of the last timed step as float32 .npy files: the loss it returned and the parameters its optimizer
+    update left behind.  A parameter larger than its share of DUMP_BYTES is sampled at positions drawn from a fixed seed.
+    The inputs (weights, token batches) are seeded too, so two builds run with the same arguments can be compared output
+    for output."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    params = [(n, p) for n, p in model.named_parameters() if p.numel()]
+    per_param = DUMP_BYTES // 4 // (len(params) + 1)
+    gen = torch.Generator().manual_seed(0)
+    for name, p in params:
+        flat = p.detach().reshape(-1)
+        if flat.numel() > per_param:
+            flat = flat[torch.randint(flat.numel(), (per_param,), generator=gen).to(flat.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), flat.float().cpu().numpy())
 
 
 def load_traffic():
@@ -307,6 +337,8 @@ def main():
     tokens_per_step = B * S * world
     value = tokens_per_step * K / (ms_max / 1e3)
     final_loss = float(loss)
+    if args.dump_outputs and rank == 0:                  # replicas hold identical parameters
+        dump_outputs(args.dump_outputs, loss, trainer.model)
 
     # ---- timed region 2: end to end through the public API with HOST buffers -------------------------------
     barrier()

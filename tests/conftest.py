@@ -63,3 +63,14 @@ def rel_err(a, b):
     a = np.asarray(a, dtype=np.float64)
     b = np.asarray(b, dtype=np.float64)
     return float(np.linalg.norm(a - b) / (np.linalg.norm(b) + 1e-300))
+
+
+def tt_matrix(g, case):
+    """Input of a from_matrix / to_matrix case of tt.npz, which keeps only its shape and SHA-256: drawn again as
+    tests/golden/make_golden.py drew it (torch.randn on the CPU after seed 0) and checked bit for bit."""
+    import hashlib
+    import torch
+    shape = [int(d) for d in g[f"tt/{case}/shape"]]
+    mat = torch.randn(*shape, generator=torch.Generator().manual_seed(0)).numpy()
+    assert hashlib.sha256(mat.tobytes()).hexdigest() == str(g[f"tt/{case}/matrix_sha256"]), case
+    return mat

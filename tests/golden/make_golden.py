@@ -8,6 +8,7 @@ The reference imports four packages that are not installed here (peft, opt_einsu
 are shimmed below (SURVEY.md 8c).  Nothing from the reference is copied: only its *outputs* on seeded inputs are
 stored, as small .npz files next to this script.
 """
+import hashlib
 import os
 import sys
 import types
@@ -17,6 +18,7 @@ import torch
 
 REF_ROOT = os.environ.get("SOW_REFERENCE_ROOT", "/root/reference")
 HERE = os.path.dirname(os.path.abspath(__file__))
+TT_ROW_STEP = 4       # of each from_matrix / to_matrix reconstruction every 4th row is stored: keeps tt.npz under 1 MB
 
 
 def install_shims():
@@ -243,6 +245,18 @@ def make_qr_cases(ref_utils, out):
     out["qr/bf16/w"], out["qr/bf16/Q"], out["qr/bf16/R"], out["qr/bf16/rank"] = npy(wb), npy(Q), npy(R), np.int32(8)
 
 
+def store_tt_matrix_case(out, name, mat, ranks, back, rel_err, core_shapes):
+    """One from_matrix / to_matrix case.  The input (torch.manual_seed(0); torch.randn(M, N)) is stored as its shape and
+    SHA-256: the tests draw it again and check it bit for bit.  The reconstruction is stored as every TT_ROW_STEP-th
+    row; ``rel_err`` is the reference's error over the full matrices."""
+    out[f"tt/{name}/shape"] = np.array(mat.shape, dtype=np.int32)
+    out[f"tt/{name}/matrix_sha256"] = np.array(hashlib.sha256(np.ascontiguousarray(mat).tobytes()).hexdigest())
+    out[f"tt/{name}/ranks"] = np.array(ranks, dtype=np.int32)
+    out[f"tt/{name}/to_matrix_rows"] = np.ascontiguousarray(back[::TT_ROW_STEP])
+    out[f"tt/{name}/rel_err"] = np.float64(rel_err)
+    out[f"tt/{name}/core_shapes"] = np.array(core_shapes, dtype=np.int32)
+
+
 def make_tt_cases(ref_tt, ref_utils, ref_ttadam, ref_ttsgd, out):
     TT = ref_tt.TensorTrain
     # --- tests/tt_test.py KAT: arange tensor, ranks [1,4,4,1]
@@ -271,16 +285,14 @@ def make_tt_cases(ref_tt, ref_utils, ref_ttadam, ref_ttsgd, out):
     cases = [("m81_r4", 81, 81, [1, 4, 4, 4, 1]), ("m81_r9", 81, 81, [1, 9, 9, 9, 1]), ("m100x60", 100, 60, [1, 16, 1]),
              ("m256_o3", 256, 256, [1, 8, 8, 1]), ("m300x200", 300, 200, [1, 12, 12, 1]),
              ("m256x192", 256, 192, [1, 32, 1]), ("m130x70_pad", 130, 70, [1, 10, 1])]
+    out["tt/to_matrix_row_step"] = np.int32(TT_ROW_STEP)
     for name, M, N, ranks in cases:
         torch.manual_seed(0)
         mat = torch.randn(M, N)
         tt = TT.from_matrix(mat, list(ranks))
         back = tt.to_matrix((M, N))
-        out[f"tt/{name}/matrix"] = npy(mat)
-        out[f"tt/{name}/ranks"] = np.array(ranks, dtype=np.int32)
-        out[f"tt/{name}/to_matrix"] = npy(back)
-        out[f"tt/{name}/rel_err"] = np.float64((back - mat).norm() / mat.norm())
-        out[f"tt/{name}/core_shapes"] = np.array([list(c.shape) for c in tt.cores], dtype=np.int32)
+        store_tt_matrix_case(out, name, npy(mat), ranks, npy(back), (back - mat).norm() / mat.norm(),
+                             [list(c.shape) for c in tt.cores])
 
     # --- tests/tt_adam_update.py KATs (seed 0; "cuda" -> "cpu")
     from opt_einsum import contract
