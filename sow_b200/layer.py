@@ -213,14 +213,18 @@ class SharedInputGroup:
         self.cache = None            # (x, x._version, grad_mode, {member index: parked output})
         self.misses = 0
         self.enabled = True
+        # a member's factors enter the group call concatenated (rank * n_iter columns); too wide a group runs its members
+        # one by one, each of which fits on its own
+        self.rank_fits = ops.group_rank_fits(m.rank * m.n_iter for m in self.members)
 
     def usable_traced(self) -> bool:
         ms = self.members
-        return self.enabled and 2 <= len(ms) <= 4 and all(m.n_iter == 1 and m.acc_upweight.numel() == 0 for m in ms)
+        return (self.enabled and self.rank_fits and 2 <= len(ms) <= 4
+                and all(m.n_iter == 1 and m.acc_upweight.numel() == 0 for m in ms))
 
     def usable(self) -> bool:
         ms = self.members
-        if not self.enabled or len(ms) < 2 or len(ms) > 4:
+        if not self.enabled or not self.rank_fits or len(ms) < 2 or len(ms) > 4:
             return False
         m0 = ms[0]
         n_dense = 0

@@ -72,6 +72,17 @@ def rank_pad(r: int) -> int:
     return (r + 63) // 64 * 64
 
 
+# Widest concatenated padded rank R = sum_i rank_pad(r_i) one sow_group_fwd / sow_group_bwd call takes: the skinny GEMM
+# keeps one scale per 64 columns of t_cat in a table of kMaxAlphaBlocks = 16 entries (csrc/gemm.cuh), and group_layout
+# (csrc/linear.cu) rejects anything wider.
+MAX_GROUP_RANK = 64 * 16
+
+
+def group_rank_fits(ranks) -> bool:
+    """True when projections of these ranks can run as ONE group call (sum of their padded ranks <= MAX_GROUP_RANK)."""
+    return sum(rank_pad(int(r)) for r in ranks) <= MAX_GROUP_RANK
+
+
 # ---------------------------------------------------------------------------------------------------------
 # SoW linear
 # ---------------------------------------------------------------------------------------------------------

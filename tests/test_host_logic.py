@@ -148,3 +148,16 @@ def test_colorized_str_runs():
     from tn_gradient.utils import __colorized_str__
     s = __colorized_str__(MLP())
     assert "fc1" in s and "trainable" in s
+
+
+@pytest.mark.parametrize("rank,n_iter,fits", [(128, 4, False), (384, 1, False), (320, 1, True), (128, 2, True)])
+def test_shared_input_group_runs_members_alone_above_the_group_rank_limit(rank, n_iter, fits):
+    """One group call takes a concatenated padded rank of at most ops.MAX_GROUP_RANK = 1024; a wider q/k/v group must run
+    its members one by one instead of failing."""
+    from sow_b200 import ops
+    from sow_b200.layer import SharedInputGroup, SoWLinear
+    ms = [SoWLinear(64, 64, rank=rank, n_iter=n_iter, init_method="normal") for _ in range(3)]
+    grp = SharedInputGroup(ms)
+    assert ops.MAX_GROUP_RANK == 1024
+    assert grp.usable() == fits
+    assert grp.usable_traced() == (fits and n_iter == 1)
