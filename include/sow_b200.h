@@ -14,7 +14,11 @@
  *    issued concurrently from several host threads (autograd runs backward on its own thread).
  *  - Scratch memory is provided by the caller: ask sow_workspace_bytes() first.
  *  - Matrices are dense row-major.  W is (in,out) -- the reference layout (tn_gradient/layer/sow.py:28,74-79),
- *    i.e. the transpose of nn.Linear.  dtype codes: SOWB_BF16 / SOWB_F32.
+ *    i.e. the transpose of nn.Linear.  dtype codes: SOWB_BF16 / SOWB_F32 / SOWB_F16.
+ *  - 16-bit modes (SOWB_BF16, SOWB_F16): every 2-byte tensor of a call has the mode's type; products accumulate in fp32
+ *    and every output element is rounded once to the 16-bit type (round to nearest even).  In SOWB_F16, values past
+ *    65504 become +-inf and inf / NaN propagate (IEEE fp16, as torch's fp16 matmul; no saturation).
+ *  - The tensor-train entry points (tt_*) take SOWB_BF16 / SOWB_F32 only and reject SOWB_F16 with SOWB_EINVAL.
  *  - Alignment: device pointers 16-byte aligned; `in` and `out` multiples of 8 (TMA row pitch rule).
  */
 #ifndef SOW_B200_H_
@@ -35,6 +39,7 @@ extern "C" {
 
 #define SOWB_BF16 0
 #define SOWB_F32 1
+#define SOWB_F16 2   /* IEEE binary16 (torch.float16) */
 
 enum sowb_op {
   SOWB_OP_LINEAR_FWD = 0,
@@ -61,7 +66,8 @@ int sow_rank_pad(int r);
 
 /*
  * One projection of a GROUP of SoW linears that read the same input x[T,in] (q/k/v or gate/up of a transformer block;
- * a lone projection is a group of one).  All matrices bf16 row-major.  Members may differ in `out`, `r` and `scale`.
+ * a lone projection is a group of one).  All matrices row-major, of the call's dtype (the 2-byte tensors of SOWB_F32 are
+ * bf16 pieces).  Members may differ in `out`, `r` and `scale`.
  */
 typedef struct sowb_group_member {
   const void* W;    /* (in,out) frozen accumulation acc_downweight, or NULL before the first merge (sow.py:69-70) */
@@ -88,10 +94,12 @@ size_t sow_group_workspace_bytes(int op, int64_t T, int in, const sowb_group_mem
  * in 2 + n launches: the factors are packed into A_cat[in,R] = [A_0|0|A_1|0|...] (each member zero-padded to
  * sow_rank_pad(r_i) columns, R = their sum), ONE skinny GEMM computes t_cat[T,R] = scale_i * x . A_cat for all members
  * (x is read once instead of n times), and each y_i is one tcgen05 GEMM with the t_i . B_i product fused in as an extra
- * K-segment.  A_cat and t_cat (caller-allocated bf16) are what autograd saves for sow_group_bwd.
+ * K-segment.  A_cat and t_cat (caller-allocated, bf16 in SOWB_BF16 / SOWB_F32, fp16 in SOWB_F16) are what autograd
+ * saves for sow_group_bwd.
  * W_i may be NULL (pre-merge phase) -> rank-r term only.  1 <= n <= 4.
  *
- * dtype SOWB_BF16: everything bf16.  dtype SOWB_F32 (fp32 modules -- the reference's GLUE scripts never set a dtype,
+ * dtype SOWB_BF16: everything bf16.  dtype SOWB_F16: everything fp16 (x, W, A, B, bias, y, A_cat, t_cat); x_lo and W_lo
+ * must be NULL.  dtype SOWB_F32 (fp32 modules -- the reference's GLUE scripts never set a dtype,
  * run_glue.py:386-388,508-514): the fp32 operands arrive split into two bf16 pieces each (sow_split_bf16x2: v ~ hi + lo,
  * relative error 2^-17), x = (x, x_lo), W_i = (W, W_lo), and the base product runs as the bf16x3 contraction
  * x.W + x.W_lo + x_lo.W on the tensor cores with fp32 accumulation (fp32-faithful: ~1e-5 relative, vs 4e-3 for plain bf16
@@ -112,7 +120,8 @@ int sow_split_bf16x2(const float* src, void* hi, void* lo, int64_t n, void* stre
  *     dbias_i = sum_T dY_i                 (if non-NULL)
  * The full in x out weight gradient is never formed (W is frozen: sow.py:69-70, prepare.py:142,150).  All reductions
  * across CTAs go through fp32 partials summed in a fixed order: results are bit-reproducible run to run.
- * dt_cat[T,R] bf16 is caller-allocated scratch.  At most 4 (SOWB_F32: 3) members may carry a dense W.
+ * dt_cat[T,R] (bf16, fp16 in SOWB_F16) is caller-allocated scratch.  At most 4 (SOWB_F32: 3) members may carry a dense W.
+ * SOWB_F16: x, A_cat, t_cat, W, B, dY, dt_cat, dX, dA, dB and dbias are fp16; dy_lo and W_lo must be NULL.
  * SOWB_F32: dY_i = (dy, dy_lo) and W_i = (W, W_lo) are bf16 pieces, dX is fp32 (bf16x3 products); the factor gradients
  * are computed from the high pieces and written in bf16.
  */
@@ -134,7 +143,9 @@ typedef struct sowb_merge_entry {
 } sowb_merge_entry;
 
 /* Grouped merge over n entries in ONE launch.  table_dev: device scratch of n * sow_merge_table_stride() bytes.
- * dtype SOWB_BF16: W, A, B bf16, the rank-r product on tcgen05, fp32 accumulate, one bf16 rounding of W.
+ * dtype SOWB_BF16: W, A, B bf16, the rank-r product on tcgen05, fp32 accumulate, one bf16 rounding of W per 64-wide
+ *                  rank chunk.
+ * dtype SOWB_F16 : the same with W, A, B fp16 and one fp16 rounding of W per rank chunk.
  * dtype SOWB_F32 : W, A, B fp32, exact fp32 FMA (fp32 modules keep their pretrained weights at full precision). */
 size_t sow_merge_table_stride(void);
 int sow_merge_grouped(const sowb_merge_entry* entries_host, int n, int dtype, void* table_dev,
@@ -279,7 +290,8 @@ int tt_adam_dense(void* p, const void* g, float* m, float* v, int64_t numel, dou
  * Multi-tensor Adam / AdamW: one launch over a device table of chunks
  *     struct { void* p; const void* g; void* m; void* v; int64_t n; }   (40 bytes, n <= sow_adam_chunk_elems())
  * covering all tensors of a param group (torch.optim.AdamW at scripts/simple_train.py:502-506).  Moments have
- * the parameter dtype (model.to(bf16): simple_train.py:425-426); math is fp32 in registers.  Bias corrections
+ * the parameter dtype (model.to(bf16): simple_train.py:425-426; torch.optim.AdamW keeps fp16 state for fp16 parameters
+ * too); math is fp32 in registers.  dtype: SOWB_BF16, SOWB_F16 or SOWB_F32.  Bias corrections
  * are computed by the caller so `state["step"]` semantics (reset_optimizer, training_utils.py:257-277) stay on
  * the host side.  Hyper-parameters are doubles so that 1-beta is formed without float cancellation.
  * decoupled != 0 -> AdamW (p *= 1 - lr*wd), else L2 (g += wd*p).

@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "libsow_b200.so")
 
 SOWB_BF16 = 0
 SOWB_F32 = 1
+SOWB_F16 = 2
 
 OP_LINEAR_FWD = 0
 OP_LINEAR_BWD = 1

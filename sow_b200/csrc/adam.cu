@@ -9,6 +9,8 @@
 // the host side re-resolves the pointers whenever they change.
 #include "common.cuh"
 
+#include <cuda_fp16.h>
+
 namespace sowb {
 
 struct AdamChunk {   // 40 bytes; the host passes an int64[n_chunks][5] table with exactly this layout
@@ -49,14 +51,38 @@ __device__ __forceinline__ AdamHyper with_device_step(AdamHyper h, const float* 
   return h;
 }
 
+// 16-bit parameter types (bf16, fp16): conversions of one element and of a packed pair, round to nearest even
+template <typename H>
+struct Half16;
+template <>
+struct Half16<__nv_bfloat16> {
+  using H2 = __nv_bfloat162;
+  static __device__ __forceinline__ float2 to_f2(H2 v) { return __bfloat1622float2(v); }
+  static __device__ __forceinline__ H2 from_f2(float a, float b) { return __floats2bfloat162_rn(a, b); }
+  static __device__ __forceinline__ float to_f(__nv_bfloat16 v) { return __bfloat162float(v); }
+  static __device__ __forceinline__ __nv_bfloat16 from_f(float v) { return __float2bfloat16(v); }
+};
+template <>
+struct Half16<__half> {
+  using H2 = __half2;
+  static __device__ __forceinline__ float2 to_f2(H2 v) { return __half22float2(v); }
+  static __device__ __forceinline__ H2 from_f2(float a, float b) { return __floats2half2_rn(a, b); }
+  static __device__ __forceinline__ float to_f(__half v) { return __half2float(v); }
+  static __device__ __forceinline__ __half from_f(float v) { return __float2half_rn(v); }
+};
+
+// p, g, m, v of type H (bf16 or fp16): 16-byte vector accesses (8 elements) when all four are 16-byte aligned
+template <typename H>
 __global__ void __launch_bounds__(256)
-adam_multi_bf16_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0, const float* __restrict__ step_dev) {
+adam_multi_16bit_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0, const float* __restrict__ step_dev) {
+  using C = Half16<H>;
+  using H2 = typename C::H2;
   const AdamHyper h = with_device_step(h0, step_dev);
   const AdamChunk c = chunks[blockIdx.x];
-  __nv_bfloat16* p = static_cast<__nv_bfloat16*>(c.p);
-  const __nv_bfloat16* g = static_cast<const __nv_bfloat16*>(c.g);
-  __nv_bfloat16* m = static_cast<__nv_bfloat16*>(c.m);
-  __nv_bfloat16* v = static_cast<__nv_bfloat16*>(c.v);
+  H* p = static_cast<H*>(c.p);
+  const H* g = static_cast<const H*>(c.g);
+  H* m = static_cast<H*>(c.m);
+  H* v = static_cast<H*>(c.v);
   const bool aligned = ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) |
                          reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15) == 0;
   int64_t done = 0;
@@ -67,19 +93,19 @@ adam_multi_bf16_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0,
       const uint4 gg = reinterpret_cast<const uint4*>(g)[i];
       uint4 mm = reinterpret_cast<uint4*>(m)[i];
       uint4 vv = reinterpret_cast<uint4*>(v)[i];
-      __nv_bfloat162* p2 = reinterpret_cast<__nv_bfloat162*>(&pp);
-      const __nv_bfloat162* g2 = reinterpret_cast<const __nv_bfloat162*>(&gg);
-      __nv_bfloat162* m2 = reinterpret_cast<__nv_bfloat162*>(&mm);
-      __nv_bfloat162* v2 = reinterpret_cast<__nv_bfloat162*>(&vv);
+      H2* p2 = reinterpret_cast<H2*>(&pp);
+      const H2* g2 = reinterpret_cast<const H2*>(&gg);
+      H2* m2 = reinterpret_cast<H2*>(&mm);
+      H2* v2 = reinterpret_cast<H2*>(&vv);
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
-        float2 pf = __bfloat1622float2(p2[j]), gf = __bfloat1622float2(g2[j]);
-        float2 mf = __bfloat1622float2(m2[j]), vf = __bfloat1622float2(v2[j]);
+        float2 pf = C::to_f2(p2[j]), gf = C::to_f2(g2[j]);
+        float2 mf = C::to_f2(m2[j]), vf = C::to_f2(v2[j]);
         adam_update(pf.x, gf.x, mf.x, vf.x, h);
         adam_update(pf.y, gf.y, mf.y, vf.y, h);
-        p2[j] = __floats2bfloat162_rn(pf.x, pf.y);
-        m2[j] = __floats2bfloat162_rn(mf.x, mf.y);
-        v2[j] = __floats2bfloat162_rn(vf.x, vf.y);
+        p2[j] = C::from_f2(pf.x, pf.y);
+        m2[j] = C::from_f2(mf.x, mf.y);
+        v2[j] = C::from_f2(vf.x, vf.y);
       }
       reinterpret_cast<uint4*>(p)[i] = pp;
       reinterpret_cast<uint4*>(m)[i] = mm;
@@ -88,11 +114,11 @@ adam_multi_bf16_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0,
     done = nvec * 8;
   }
   for (int64_t i = done + threadIdx.x; i < c.n; i += blockDim.x) {
-    float pf = __bfloat162float(p[i]), mf = __bfloat162float(m[i]), vf = __bfloat162float(v[i]);
-    adam_update(pf, __bfloat162float(g[i]), mf, vf, h);
-    p[i] = __float2bfloat16(pf);
-    m[i] = __float2bfloat16(mf);
-    v[i] = __float2bfloat16(vf);
+    float pf = C::to_f(p[i]), mf = C::to_f(m[i]), vf = C::to_f(v[i]);
+    adam_update(pf, C::to_f(g[i]), mf, vf, h);
+    p[i] = C::from_f(pf);
+    m[i] = C::from_f(mf);
+    v[i] = C::from_f(vf);
   }
 }
 
@@ -189,9 +215,11 @@ static int adam_launch(const void* chunks_dev, int n_chunks, int64_t total_elems
   h.inv_sqrt_bc2 = float(1.0 / sqrt(bias_correction2));
   h.decoupled = decoupled;
   // algorithmic bytes: p, m, v read+written, g read = 7 accesses of the element size
-  ProfileScope prof(stream, PROF_ADAM, 7.0 * double(total_elems) * (dtype == SOWB_BF16 ? 2 : 4));
+  ProfileScope prof(stream, PROF_ADAM, 7.0 * double(total_elems) * (dtype == SOWB_F32 ? 4 : 2));
   if (dtype == SOWB_BF16)
-    adam_multi_bf16_kernel<<<n_chunks, 256, 0, stream>>>(static_cast<const AdamChunk*>(chunks_dev), h, step_dev);
+    adam_multi_16bit_kernel<__nv_bfloat16><<<n_chunks, 256, 0, stream>>>(static_cast<const AdamChunk*>(chunks_dev), h, step_dev);
+  else if (dtype == SOWB_F16)
+    adam_multi_16bit_kernel<__half><<<n_chunks, 256, 0, stream>>>(static_cast<const AdamChunk*>(chunks_dev), h, step_dev);
   else if (dtype == SOWB_F32)
     adam_multi_f32_kernel<<<n_chunks, 256, 0, stream>>>(static_cast<const AdamChunk*>(chunks_dev), h, step_dev);
   else

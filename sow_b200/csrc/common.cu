@@ -96,17 +96,17 @@ struct MapKey {
   const void* base;
   uint64_t inner, outer, pitch;
   uint32_t b0, b1;
-  int eb;
+  int dt;   // CUtensorMapDataType: a bf16 and an fp16 map of the same memory are different maps
   bool operator==(const MapKey& o) const {
     return base == o.base && inner == o.inner && outer == o.outer && pitch == o.pitch && b0 == o.b0 && b1 == o.b1 &&
-           eb == o.eb;
+           dt == o.dt;
   }
 };
 struct MapKeyHash {
   size_t operator()(const MapKey& k) const {
     uint64_t h = reinterpret_cast<uint64_t>(k.base) * 0x9E3779B97F4A7C15ull;
     h ^= (k.inner * 0xC2B2AE3D27D4EB4Full) ^ (k.outer << 17) ^ (k.pitch << 29) ^ (uint64_t(k.b0) << 7) ^
-         (uint64_t(k.b1) << 43) ^ uint64_t(k.eb);
+         (uint64_t(k.b1) << 43) ^ uint64_t(k.dt);
     return static_cast<size_t>(h ^ (h >> 31));
   }
 };
@@ -156,19 +156,22 @@ int ensure_context_for(const void* ptr) {
 }
 
 int make_tensor_map_2d(CUtensorMap* out, const void* base, uint64_t inner, uint64_t outer, uint64_t pitch_bytes,
-                       uint32_t box_inner, uint32_t box_outer, int elem_bytes) {
+                       uint32_t box_inner, uint32_t box_outer, CUtensorMapDataType dt) {
   if (base == nullptr) return set_error(SOWB_EINVAL, "tensor map: null base pointer");
   if ((reinterpret_cast<uintptr_t>(base) & 15) != 0)
     return set_error(SOWB_EINVAL, "tensor map: base pointer %p is not 16-byte aligned", base);
   if (pitch_bytes % 16 != 0)
     return set_error(SOWB_EINVAL, "tensor map: row pitch %llu B is not a multiple of 16 (features must be multiples of 8)",
                      (unsigned long long)pitch_bytes);
+  if (dt != CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 && dt != CU_TENSOR_MAP_DATA_TYPE_FLOAT16 && dt != CU_TENSOR_MAP_DATA_TYPE_FLOAT32)
+    return set_error(SOWB_EINVAL, "tensor map: unsupported data type %d", (int)dt);
+  const uint32_t elem_bytes = (dt == CU_TENSOR_MAP_DATA_TYPE_FLOAT32) ? 4 : 2;
   if (box_inner * elem_bytes != 128 || box_outer == 0 || box_outer > 256)
     return set_error(SOWB_EINVAL, "tensor map: unsupported box %u x %u", box_inner, box_outer);
 
   static std::mutex mu;
   static std::unordered_map<MapKey, CUtensorMap, MapKeyHash> cache;
-  MapKey key{base, inner, outer, pitch_bytes, box_inner, box_outer, elem_bytes};
+  MapKey key{base, inner, outer, pitch_bytes, box_inner, box_outer, static_cast<int>(dt)};
   {
     std::lock_guard<std::mutex> lk(mu);
     auto it = cache.find(key);
@@ -187,7 +190,6 @@ int make_tensor_map_2d(CUtensorMap* out, const void* base, uint64_t inner, uint6
   cuuint64_t strides[1] = {pitch_bytes};
   cuuint32_t box[2] = {box_inner, box_outer};
   cuuint32_t estr[2] = {1, 1};
-  CUtensorMapDataType dt = (elem_bytes == 2) ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
   static const CUtensorMapL2promotion promo = []() {
     const char* e = getenv("SOWB_TMA_PROMO");   // tuning knob: 0 none, 1 64 B, 2 128 B, 3 256 B (default)
     const int v = e ? atoi(e) : 3;

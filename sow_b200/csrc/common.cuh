@@ -70,9 +70,17 @@ int launch_sum_splits(const float* part, int splits, int64_t split_stride, int64
 int ensure_context_for(const void* ptr);
 
 // 2-D row-major tensor map with 128B swizzle.  `inner` is the contiguous dimension (elements), `outer` the row
-// count, `pitch_bytes` the row pitch; box = (box_inner x box_outer) elements.  elem_bytes: 2 (bf16) or 4 (fp32).
+// count, `pitch_bytes` the row pitch; box = (box_inner x box_outer) elements.  dt: BFLOAT16, FLOAT16 or FLOAT32.
 int make_tensor_map_2d(CUtensorMap* out, const void* base, uint64_t inner, uint64_t outer, uint64_t pitch_bytes,
-                       uint32_t box_inner, uint32_t box_outer, int elem_bytes);
+                       uint32_t box_inner, uint32_t box_outer, CUtensorMapDataType dt);
+// TMA element type of the 2-byte operands of a SOWB_BF16 / SOWB_F16 call
+inline CUtensorMapDataType map_type16(bool f16) {
+  return f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+}
+
+// The tensor-train entry points take bf16 and fp32 only: reject SOWB_F16 (and unknown codes) before any work is queued.
+#define SOWB_REQUIRE_TT_DTYPE(fn, dtype) \
+  SOWB_REQUIRE((dtype) == SOWB_BF16 || (dtype) == SOWB_F32, "%s: dtype %d unsupported (tensor-train path: bf16 / fp32)", fn, dtype)
 
 // ------------------------------------------------------------------------------------------------
 // Live per-kernel timing (bench.py roofline): when enabled, launches are bracketed by CUDA events recorded on the

@@ -6,7 +6,10 @@
 //   warp 0 / lane 0 : TMA producer  (global -> 128B-swizzled smem ring, mbarrier complete_tx)
 //   warp 1 / lane 0 : MMA issuer    (tcgen05.mma, M=128 x N=BN x K=16, fp32 accumulators in TMEM, 2 stages)
 //   warp 2          : TMEM allocator / deallocator
-//   warps 4..7      : epilogue      (tcgen05.ld -> registers -> {bf16 via swizzled smem + TMA store | fp32 split-K partial})
+//   warps 4..7      : epilogue      (tcgen05.ld -> registers -> {bf16 / fp16 via swizzled smem + TMA store | fp32 split-K partial})
+//
+// F16 selects the 16-bit operand type: bf16 (false) or IEEE fp16 (true) -- the instruction-descriptor format, the TMA
+// element type (host side) and the EPI_BF16_TMA conversion; everything else is shared.
 //
 // Operand "majorness" is a template parameter because the SoW hot path needs all four combinations without
 // re-laying-out any user-visible tensor (reference layout of W is (in,out), tn_gradient/layer/sow.py:28,74-79):
@@ -35,7 +38,7 @@ constexpr int kStoreBoxCols = 64;                                  // bf16 colum
 constexpr int kStageCBytes = kBM * kStoreBoxCols * 2;              // 16 KB per staging buffer
 
 enum EpiMode : int {
-  EPI_BF16_TMA = 0,    // D -> bf16, via smem staging + TMA store (clips M/N tails)
+  EPI_BF16_TMA = 0,    // D -> 16-bit (bf16, or fp16 with F16), via smem staging + TMA store (clips M/N tails)
   EPI_F32_PARTIAL = 1,  // D -> fp32 PARTIAL of split s stored at out_f32[s*split_stride + row*ldc + col]; the caller sums the
                        // splits in a fixed order (bit-reproducible, unlike red.global.add; no zero-fill needed)
   EPI_F32_TMA = 2,     // D -> fp32 (+ fp32 bias), via smem staging + TMA store: the output of the bf16x3 path of fp32 modules
@@ -58,7 +61,7 @@ struct GemmParams {
   int kb_per_split;
   int alpha_blocks;     // 0: alpha[0] for every column; else alpha[(col / 64)]
   float alpha[kMaxAlphaBlocks];
-  const __nv_bfloat16* bias;  // nullable, length N (EPI_BF16_TMA only)
+  const uint16_t* bias;       // nullable, length N, the operands' 16-bit type (EPI_BF16_TMA only)
   const float* bias_f32;      // nullable, length N (EPI_F32_TMA only)
   float* out_f32;             // EPI_F32_PARTIAL only
   int64_t split_stride;       // EPI_F32_PARTIAL only: elements between the partial outputs of consecutive splits
@@ -85,7 +88,7 @@ struct GemmSmem {
   static constexpr uint32_t kTmemCols = (2 * BN <= 32) ? 32 : (2 * BN <= 64 ? 64 : (2 * BN <= 128 ? 128 : (2 * BN <= 256 ? 256 : 512)));
 };
 
-template <int BN, bool A_MN, bool B_MN, int EPI, int MT = 1>
+template <int BN, bool A_MN, bool B_MN, int EPI, int MT = 1, bool F16 = false>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 sow_gemm_kernel(const __grid_constant__ GemmMaps maps, const GemmParams p) {
   using S = GemmSmem<BN, MT>;
@@ -185,7 +188,7 @@ sow_gemm_kernel(const __grid_constant__ GemmMaps maps, const GemmParams p) {
     }
   } else if (warp == 1 && lane == 0) {
     // ===================== MMA issuer =====================
-    constexpr uint32_t idesc = make_idesc(/*bf16*/ 1, kBM, BN, A_MN ? 1 : 0, B_MN ? 1 : 0);
+    constexpr uint32_t idesc = make_idesc(ab_format16<F16>(), kBM, BN, A_MN ? 1 : 0, B_MN ? 1 : 0);
     // K-major:  SBO = 1024 B between 8-row atoms; advance 32 B per UMMA_K inside the 128 B swizzle span.
     // MN-major: LBO = 8192 B between 64-wide MN blocks (one TMA box each), SBO = 1024 B between 8-deep K groups;
     //           advance 2 K-groups = 2048 B per UMMA_K.
@@ -272,14 +275,14 @@ sow_gemm_kernel(const __grid_constant__ GemmMaps maps, const GemmParams p) {
                 f[j] = alpha * __uint_as_float(v[c * 8 + j]);
                 if (p.bias != nullptr) {
                   const int col = colbase + c * 8 + j;
-                  if (col < p.N) f[j] += __bfloat162float(p.bias[col]);
+                  if (col < p.N) f[j] += lo16_to_f32<F16>(p.bias[col]);
                 }
               }
               uint4 pk;
-              pk.x = pack_bf16x2(f[0], f[1]);
-              pk.y = pack_bf16x2(f[2], f[3]);
-              pk.z = pack_bf16x2(f[4], f[5]);
-              pk.w = pack_bf16x2(f[6], f[7]);
+              pk.x = pack16x2<F16>(f[0], f[1]);
+              pk.y = pack16x2<F16>(f[2], f[3]);
+              pk.z = pack16x2<F16>(f[4], f[5]);
+              pk.w = pack16x2<F16>(f[6], f[7]);
               const int chunk = h * 4 + c;  // 16-byte chunk index inside the 128-byte row
               *reinterpret_cast<uint4*>(stg + row_in_tile * 128 + ((chunk ^ (row_in_tile & 7)) << 4)) = pk;
             }

@@ -20,11 +20,13 @@
 //   * dt of a chunk needs all G groups: a reduce-scatter over DISTRIBUTED SHARED MEMORY.  Row i of the chunk is
 //     finalised by CTA i % G: every other CTA stores its fp32 partial of that row into the owner's receive buffer
 //     (st.shared::cluster) and arrives on the owner's mbarrier; the owner adds the G partials in the fixed order
-//     0..G-1, scales, converts and writes the bf16 row.  No global partials, fences or atomics (the first version
+//     0..G-1, scales, converts and writes the 16-bit row.  No global partials, fences or atomics (the first version
 //     exchanged the partials through L2 with a last-arriver counter: 16 k cycles per chunk against a 6 k-cycle main
 //     loop, profiles/r02_k2_timeline.txt).
 //
 // Roles (256 threads): warp 0 lane 0 TMA producer, warp 1 lane 0 UMMA issuer, warp 2 TMEM allocator, warps 4-7 epilogue.
+// F16: dY, B, t and dt are IEEE fp16 instead of bf16 (instruction-descriptor format and the dt conversion; TMA maps on
+// the host side).  The dB^T partials are fp32 either way.
 #pragma once
 #include "ptx.cuh"
 
@@ -68,7 +70,7 @@ struct K2Member {
   int blk_first, blk_end;   // 128-col blocks [blk_first, blk_end) of dY covered by this launch
   int dt_accumulate;        // add onto the dt already in memory (second launch over a very wide `out`)
   float scale;
-  __nv_bfloat16* dt;        // [T, ldt] (this member's / rank chunk's 64 columns)
+  void* dt;                 // [T, ldt] 16-bit (this member's / rank chunk's 64 columns)
 };
 struct K2Params {
   int T, G, n_members;
@@ -79,6 +81,7 @@ struct K2Params {
   long long* dbg;           // debug timeline (tools/k2_timeline.py): CTA 0 records clock64 stamps [chunk][16], or NULL
 };
 
+template <bool F16>
 __global__ void __launch_bounds__(kK2Threads, 1)
 sow_k2_kernel(const __grid_constant__ K2Maps allmaps, const __grid_constant__ K2Params p) {
   extern __shared__ uint8_t smem_raw[];
@@ -195,8 +198,8 @@ sow_k2_kernel(const __grid_constant__ K2Maps allmaps, const __grid_constant__ K2
     }
   } else if (warp == 1 && lane == 0) {
     // ===================== UMMA issuer =====================
-    constexpr uint32_t idesc_dt = make_idesc(1, 128, 64, 0, 0);   // A K-major (dY), B K-major (B rows = r)
-    constexpr uint32_t idesc_db = make_idesc(1, 128, 64, 1, 1);   // A MN-major (dY^T), B MN-major (t)
+    constexpr uint32_t idesc_dt = make_idesc(ab_format16<F16>(), 128, 64, 0, 0);   // A K-major (dY), B K-major (B rows = r)
+    constexpr uint32_t idesc_db = make_idesc(ab_format16<F16>(), 128, 64, 1, 1);   // A MN-major (dY^T), B MN-major (t)
     int stage = 0, tb = 0, acc = 0;
     uint32_t phase = 0, tphase = 0, aphase = 0;
     bool first_chunk = true;
@@ -347,7 +350,7 @@ sow_k2_kernel(const __grid_constant__ K2Maps allmaps, const __grid_constant__ K2
         if (et == 0) stamp(cl, 10);
       }
       if (owner == g && row < p.T) {
-        uint4* dst = reinterpret_cast<uint4*>(M.dt + static_cast<int64_t>(row) * p.ldt);
+        uint4* dst = reinterpret_cast<uint4*>(static_cast<uint16_t*>(M.dt) + static_cast<int64_t>(row) * p.ldt);
 #pragma unroll
         for (int ch = 0; ch < 8; ++ch) {
           float f[8];
@@ -358,15 +361,15 @@ sow_k2_kernel(const __grid_constant__ K2Maps allmaps, const __grid_constant__ K2
             const uint32_t ow[4] = {old.x, old.y, old.z, old.w};
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
-              f[2 * i] += __uint_as_float(ow[i] << 16);
-              f[2 * i + 1] += __uint_as_float(ow[i] & 0xffff0000u);
+              f[2 * i] += lo16_to_f32<F16>(ow[i]);
+              f[2 * i + 1] += hi16_to_f32<F16>(ow[i]);
             }
           }
           uint4 pk;
-          pk.x = pack_bf16x2(f[0], f[1]);
-          pk.y = pack_bf16x2(f[2], f[3]);
-          pk.z = pack_bf16x2(f[4], f[5]);
-          pk.w = pack_bf16x2(f[6], f[7]);
+          pk.x = pack16x2<F16>(f[0], f[1]);
+          pk.y = pack16x2<F16>(f[2], f[3]);
+          pk.z = pack16x2<F16>(f[4], f[5]);
+          pk.w = pack16x2<F16>(f[6], f[7]);
           dst[ch] = pk;
         }
       }

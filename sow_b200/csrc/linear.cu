@@ -18,15 +18,16 @@ constexpr int kMaxGroup = 4;   // members per group (dX fuses at most kMaxSeg - 
 // small helper kernels
 // ------------------------------------------------------------------------------------------------
 // A_i (in, r_i) for i < n  ->  A_cat (in, R) = [A_0 | 0 | A_1 | 0 | ...], every member zero-padded to a multiple of 64
-// columns: gives the factors a TMA-legal row pitch and one operand for the shared down-projection.
+// columns: gives the factors a TMA-legal row pitch and one operand for the shared down-projection.  A bit copy of 16-bit
+// elements (0x0000 is +0 in bf16 and fp16): serves both 16-bit types.
 struct PackArgs {
-  const __nv_bfloat16* A[kMaxGroup];
+  const uint16_t* A[kMaxGroup];
   int r[kMaxGroup];
   int off[kMaxGroup + 1];   // first column of member i in A_cat; off[n] = R
   int n;
 };
-__global__ void pack_factors_kernel(const PackArgs a, __nv_bfloat16* __restrict__ A_cat, int in, int R) {
-  const int64_t total = static_cast<int64_t>(in) * (R >> 1);      // one bf16 pair per thread
+__global__ void pack_factors_kernel(const PackArgs a, uint16_t* __restrict__ A_cat, int in, int R) {
+  const int64_t total = static_cast<int64_t>(in) * (R >> 1);      // one 16-bit pair per thread
   for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < total;
        i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int row = static_cast<int>(i / (R >> 1));
@@ -34,22 +35,20 @@ __global__ void pack_factors_kernel(const PackArgs a, __nv_bfloat16* __restrict_
     int m = 0;
     while (m + 1 < a.n && col >= a.off[m + 1]) ++m;
     const int c = col - a.off[m];
-    const __nv_bfloat16 z = __float2bfloat16(0.f);
-    const __nv_bfloat16* src = a.A[m] + static_cast<int64_t>(row) * a.r[m];
-    __nv_bfloat162 v;
-    v.x = (c < a.r[m]) ? src[c] : z;
-    v.y = (c + 1 < a.r[m]) ? src[c + 1] : z;
-    *reinterpret_cast<__nv_bfloat162*>(A_cat + static_cast<int64_t>(row) * R + col) = v;
+    const uint16_t* src = a.A[m] + static_cast<int64_t>(row) * a.r[m];
+    const uint32_t lo = (c < a.r[m]) ? src[c] : 0u;
+    const uint32_t hi = (c + 1 < a.r[m]) ? src[c + 1] : 0u;
+    *reinterpret_cast<uint32_t*>(A_cat + static_cast<int64_t>(row) * R + col) = lo | (hi << 16);
   }
 }
 
-// fp32 split PARTIALS -> bf16 gradients in the reference layouts, summed over the splits in a fixed order (so the
+// fp32 split PARTIALS -> 16-bit (bf16 / fp16) gradients in the reference layouts, summed over the splits in a fixed order (so the
 // factor gradients are bit-reproducible run to run).  A job sums `splits` partial matrices [rows x ld_src] and writes
 // the first `cols` columns either as they are (dA: dst[row, col]) or transposed (dB: partial is dB^T, dst[col, row]).
 struct FinJob {
   const float* src;
   int64_t split_stride;
-  __nv_bfloat16* dst;
+  uint16_t* dst;
   int splits, rows, cols, ld_src, ld_dst, transpose, blk_begin, col_tiles;
 };
 constexpr int kMaxFinJobs = 8;
@@ -57,6 +56,12 @@ struct FinJobs {
   FinJob j[kMaxFinJobs];
   int n;
 };
+template <bool F16>
+__device__ __forceinline__ uint16_t to16(float f) {
+  return static_cast<uint16_t>(pack16x2<F16>(f, 0.f) & 0xffffu);
+}
+
+template <bool F16>
 __global__ void finalize_jobs_kernel(const FinJobs jobs) {
   __shared__ float tile[32][33];
   int ji = 0;
@@ -81,14 +86,14 @@ __global__ void finalize_jobs_kernel(const FinJobs jobs) {
     for (; k < J.splits; ++k) s += __ldcs(p + k * J.split_stride);
   }
   if (!J.transpose) {
-    if (row < J.rows && col < J.cols) J.dst[static_cast<int64_t>(row) * J.ld_dst + col] = __float2bfloat16(s);
+    if (row < J.rows && col < J.cols) J.dst[static_cast<int64_t>(row) * J.ld_dst + col] = to16<F16>(s);
     return;
   }
   tile[threadIdx.y][threadIdx.x] = s;
   __syncthreads();
   const int orow = r0 + threadIdx.x, ocol = c0 + threadIdx.y;   // orow: partial row (out index), ocol: rank index
   if (orow < J.rows && ocol < J.cols)
-    J.dst[static_cast<int64_t>(ocol) * J.ld_dst + orow] = __float2bfloat16(tile[threadIdx.x][threadIdx.y]);
+    J.dst[static_cast<int64_t>(ocol) * J.ld_dst + orow] = to16<F16>(tile[threadIdx.x][threadIdx.y]);
 }
 
 // v -> hi = bf16(v), lo = bf16(v - hi): operand pieces of the bf16x3 products (fp32 modules)
@@ -122,25 +127,27 @@ __global__ void split_bf16x2_tail_kernel(const float* __restrict__ src, __nv_bfl
 
 // dbias[o] = sum_t dY[t, o]: block = 64 columns x 4 row-lanes, grid.y splits T; every block writes its partial row,
 // the conversion kernel sums the partial rows in a fixed order (bit-reproducible).
-__global__ void colsum_kernel(const __nv_bfloat16* __restrict__ dy, float* __restrict__ part, int64_t T, int out) {
+template <bool F16>
+__global__ void colsum_kernel(const uint16_t* __restrict__ dy, float* __restrict__ part, int64_t T, int out) {
   __shared__ float red[4][64];
   const int col = blockIdx.x * 64 + threadIdx.x;
   const int64_t rows_per = (T + gridDim.y - 1) / gridDim.y;
   const int64_t t0 = blockIdx.y * rows_per, t1 = min(T, t0 + rows_per);
   float s = 0.f;
   if (col < out)
-    for (int64_t t = t0 + threadIdx.y; t < t1; t += blockDim.y) s += __bfloat162float(dy[t * out + col]);
+    for (int64_t t = t0 + threadIdx.y; t < t1; t += blockDim.y) s += lo16_to_f32<F16>(dy[t * out + col]);
   red[threadIdx.y][threadIdx.x] = s;
   __syncthreads();
   if (threadIdx.y == 0 && col < out)
     part[static_cast<int64_t>(blockIdx.y) * out + col] = (red[0][threadIdx.x] + red[1][threadIdx.x]) + (red[2][threadIdx.x] + red[3][threadIdx.x]);
 }
-__global__ void sum_partials_to_bf16_kernel(const float* __restrict__ part, __nv_bfloat16* __restrict__ dst, int n, int parts) {
+template <bool F16>
+__global__ void sum_partials_to_16_kernel(const float* __restrict__ part, uint16_t* __restrict__ dst, int n, int parts) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) {
     float s = 0.f;
     for (int k = 0; k < parts; ++k) s += part[static_cast<int64_t>(k) * n + i];
-    dst[i] = __float2bfloat16(s);
+    dst[i] = to16<F16>(s);
   }
 }
 
@@ -159,9 +166,10 @@ struct Segment {
 
 // Operand A of D = A.B: logical [M, K].  K-major  <=> stored [M rows, K cols];  MN-major <=> stored [K rows, M cols].
 // Operand B of D = A.B: logical [K, N].  K-major  <=> stored [N rows, K cols];  MN-major <=> stored [K rows, N cols].
+// f16: the 16-bit operands (and a 16-bit C / bias) are fp16, else bf16.
 template <int BN, bool A_MN, bool B_MN, int EPI, int MT = 1>
 static int launch_gemm(const Segment* segs, int nseg, void* C_bf16, float* C_f32, int ldc, int M, int N,
-                       const float* alpha_blocks, int n_alpha, const void* bias, bool split_k, cudaStream_t stream,
+                       const float* alpha_blocks, int n_alpha, const void* bias, bool split_k, bool f16, cudaStream_t stream,
                        int prof_class, double alg_flops, int* splits_out = nullptr) {
   using S = GemmSmem<BN, MT>;
   if (nseg < 1 || nseg > kMaxSeg) return set_error(SOWB_EINVAL, "launch_gemm: %d segments (max %d)", nseg, kMaxSeg);
@@ -169,21 +177,22 @@ static int launch_gemm(const Segment* segs, int nseg, void* C_bf16, float* C_f32
   GemmParams p;
   int rc;
   int kb = 0;
+  const CUtensorMapDataType t16 = map_type16(f16);
   for (int s = 0; s < kMaxSeg; ++s) {
     const Segment& sg = segs[s < nseg ? s : 0];
-    rc = make_tensor_map_2d(&maps.a[s], sg.A.ptr, sg.A.cols, sg.A.rows, sg.A.pitch_elems * 2, 64, A_MN ? 64 : kBM, 2);
+    rc = make_tensor_map_2d(&maps.a[s], sg.A.ptr, sg.A.cols, sg.A.rows, sg.A.pitch_elems * 2, 64, A_MN ? 64 : kBM, t16);
     if (rc) return rc;
-    rc = make_tensor_map_2d(&maps.b[s], sg.B.ptr, sg.B.cols, sg.B.rows, sg.B.pitch_elems * 2, 64, B_MN ? 64 : BN, 2);
+    rc = make_tensor_map_2d(&maps.b[s], sg.B.ptr, sg.B.cols, sg.B.rows, sg.B.pitch_elems * 2, 64, B_MN ? 64 : BN, t16);
     if (rc) return rc;
     if (s < nseg) kb += ceil_div(sg.K, kBK);
     p.kb_end[s] = kb;
   }
   maps.c = maps.a[0];
   if (EPI == EPI_BF16_TMA) {
-    rc = make_tensor_map_2d(&maps.c, C_bf16, N, M, static_cast<uint64_t>(ldc) * 2, kStoreBoxCols, kBM, 2);
+    rc = make_tensor_map_2d(&maps.c, C_bf16, N, M, static_cast<uint64_t>(ldc) * 2, kStoreBoxCols, kBM, t16);
     if (rc) return rc;
   } else if (EPI == EPI_F32_TMA) {
-    rc = make_tensor_map_2d(&maps.c, C_f32, N, M, static_cast<uint64_t>(ldc) * 4, 32, kBM, 4);
+    rc = make_tensor_map_2d(&maps.c, C_f32, N, M, static_cast<uint64_t>(ldc) * 4, 32, kBM, CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
     if (rc) return rc;
   }
   p.M = M;
@@ -203,7 +212,7 @@ static int launch_gemm(const Segment* segs, int nseg, void* C_bf16, float* C_f32
   p.splits = ceil_div(kb_total, std::max(1, p.kb_per_split));
   p.alpha_blocks = (n_alpha > 1) ? std::min(n_alpha, kMaxAlphaBlocks) : 0;
   for (int i = 0; i < kMaxAlphaBlocks; ++i) p.alpha[i] = (i < n_alpha) ? alpha_blocks[i] : alpha_blocks[std::max(0, n_alpha - 1)];
-  p.bias = (EPI == EPI_BF16_TMA) ? static_cast<const __nv_bfloat16*>(bias) : nullptr;
+  p.bias = (EPI == EPI_BF16_TMA) ? static_cast<const uint16_t*>(bias) : nullptr;
   p.bias_f32 = (EPI == EPI_F32_TMA) ? static_cast<const float*>(bias) : nullptr;
   p.out_f32 = C_f32;
   p.split_stride = static_cast<int64_t>(M) * ldc;
@@ -211,7 +220,10 @@ static int launch_gemm(const Segment* segs, int nseg, void* C_bf16, float* C_f32
   if (splits_out) *splits_out = p.splits;
   const int total = p.m_tiles * p.n_tiles * p.splits;
   if (total <= 0 || kb_total <= 0) return SOWB_OK;
-  auto kern = sow_gemm_kernel<BN, A_MN, B_MN, EPI, MT>;
+  auto kern = sow_gemm_kernel<BN, A_MN, B_MN, EPI, MT, false>;
+  if constexpr (EPI != EPI_F32_TMA) {   // the bf16x3 path of fp32 modules has bf16 operands only
+    if (f16) kern = sow_gemm_kernel<BN, A_MN, B_MN, EPI, MT, true>;
+  }
   SOWB_CHECK_CUDA(set_max_smem_once(kern, size_t(S::kTotal)));
   const int grid = total < sms ? total : sms;
   ProfileScope prof(stream, prof_class, alg_flops);   // algorithmic flops: un-padded ranks (SURVEY.md 8d)
@@ -255,17 +267,17 @@ static int skinny_bn(int R) { return R >= 256 ? 256 : R; }
 
 template <bool A_MN, bool B_MN, int EPI>
 static int launch_skinny(int R, const Segment* seg, int nseg, void* C_bf16, float* C_f32, int ldc, int M,
-                         const float* alpha, int n_alpha, bool split_k, cudaStream_t stream, int prof_class,
+                         const float* alpha, int n_alpha, bool split_k, bool f16, cudaStream_t stream, int prof_class,
                          double alg_flops, int* splits_out = nullptr) {
   switch (skinny_bn(R)) {
     case 64:
-      return launch_gemm<64, A_MN, B_MN, EPI>(seg, nseg, C_bf16, C_f32, ldc, M, R, alpha, n_alpha, nullptr, split_k, stream, prof_class, alg_flops, splits_out);
+      return launch_gemm<64, A_MN, B_MN, EPI>(seg, nseg, C_bf16, C_f32, ldc, M, R, alpha, n_alpha, nullptr, split_k, f16, stream, prof_class, alg_flops, splits_out);
     case 128:
-      return launch_gemm<128, A_MN, B_MN, EPI>(seg, nseg, C_bf16, C_f32, ldc, M, R, alpha, n_alpha, nullptr, split_k, stream, prof_class, alg_flops, splits_out);
+      return launch_gemm<128, A_MN, B_MN, EPI>(seg, nseg, C_bf16, C_f32, ldc, M, R, alpha, n_alpha, nullptr, split_k, f16, stream, prof_class, alg_flops, splits_out);
     case 192:
-      return launch_gemm<192, A_MN, B_MN, EPI>(seg, nseg, C_bf16, C_f32, ldc, M, R, alpha, n_alpha, nullptr, split_k, stream, prof_class, alg_flops, splits_out);
+      return launch_gemm<192, A_MN, B_MN, EPI>(seg, nseg, C_bf16, C_f32, ldc, M, R, alpha, n_alpha, nullptr, split_k, f16, stream, prof_class, alg_flops, splits_out);
     default:
-      return launch_gemm<256, A_MN, B_MN, EPI>(seg, nseg, C_bf16, C_f32, ldc, M, R, alpha, n_alpha, nullptr, split_k, stream, prof_class, alg_flops, splits_out);
+      return launch_gemm<256, A_MN, B_MN, EPI>(seg, nseg, C_bf16, C_f32, ldc, M, R, alpha, n_alpha, nullptr, split_k, f16, stream, prof_class, alg_flops, splits_out);
   }
 }
 
@@ -281,8 +293,9 @@ static int k2_max_clusters(int G) {
   std::lock_guard<std::mutex> lk(mu);
   if (cache[dev][G] == 0) {
     int n = 0;
-    set_max_smem_once(sow_k2_kernel, size_t(kK2SmemTotal));
-    if (G > 8) cudaFuncSetAttribute(sow_k2_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    // the fp16 instantiation has the same resources: one query serves both
+    set_max_smem_once(sow_k2_kernel<false>, size_t(kK2SmemTotal));
+    if (G > 8) cudaFuncSetAttribute(sow_k2_kernel<false>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(G * 64);
     cfg.blockDim = dim3(kK2Threads);
@@ -294,7 +307,7 @@ static int k2_max_clusters(int G) {
     at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    if (cudaOccupancyMaxActiveClusters(&n, sow_k2_kernel, &cfg) != cudaSuccess || n <= 0) {
+    if (cudaOccupancyMaxActiveClusters(&n, sow_k2_kernel<false>, &cfg) != cudaSuccess || n <= 0) {
       cudaGetLastError();
       n = std::max(1, (num_sms() / G) * 3 / 4);      // conservative guess if the query is unavailable
     }
@@ -329,7 +342,7 @@ static int group_layout(const char* fn, const sowb_group_member* m, int n, int64
     const int rc0 = ensure_context_for(any);   // backward runs on autograd's worker thread
     if (rc0) return rc0;
   }
-  if (dtype != SOWB_BF16 && dtype != SOWB_F32) return set_error(SOWB_EINVAL, "%s: unknown dtype %d", fn, dtype);
+  if (dtype != SOWB_BF16 && dtype != SOWB_F32 && dtype != SOWB_F16) return set_error(SOWB_EINVAL, "%s: unknown dtype %d", fn, dtype);
   if (m == nullptr || n < 1 || n > kMaxGroup) return set_error(SOWB_EINVAL, "%s: group size %d (1..%d)", fn, n, kMaxGroup);
   if (T <= 0 || in <= 0) return set_error(SOWB_EINVAL, "%s: non-positive dimension", fn);
   if (T >= (int64_t(1) << 31)) return set_error(SOWB_EINVAL, "%s: T too large", fn);
@@ -428,15 +441,17 @@ int sow_group_fwd(const void* x, const void* x_lo, const sowb_group_member* m, i
   int rc = group_layout("sow_group_fwd", m, n, T, in, dtype, x, &L);
   if (rc) return rc;
   SOWB_REQUIRE(x && A_cat && t_cat, "sow_group_fwd: null pointer argument");
-  const bool f32 = dtype == SOWB_F32;
+  const bool f32 = dtype == SOWB_F32, f16 = dtype == SOWB_F16;
   SOWB_REQUIRE(!f32 || x_lo != nullptr, "sow_group_fwd: SOWB_F32 needs the low piece of x");
+  SOWB_REQUIRE(!f16 || x_lo == nullptr, "sow_group_fwd: SOWB_F16 takes no x_lo");
+  for (int i = 0; i < n; ++i) SOWB_REQUIRE(!f16 || m[i].W_lo == nullptr, "sow_group_fwd: SOWB_F16 takes no W_lo (member %d)", i);
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   const int R = L.R;
   {
     PackArgs pa;
     pa.n = n;
     for (int i = 0; i < kMaxGroup; ++i) {
-      pa.A[i] = static_cast<const __nv_bfloat16*>(m[i < n ? i : 0].A);
+      pa.A[i] = static_cast<const uint16_t*>(m[i < n ? i : 0].A);
       pa.r[i] = m[i < n ? i : 0].r;
       pa.off[i] = L.off[i < n ? i : n];
     }
@@ -444,7 +459,7 @@ int sow_group_fwd(const void* x, const void* x_lo, const sowb_group_member* m, i
     for (int i = n; i <= kMaxGroup; ++i) pa.off[i] = R;
     const int64_t total = int64_t(in) * (R / 2);
     const int blocks = static_cast<int>(std::min<int64_t>((total + 255) / 256, 2048));
-    pack_factors_kernel<<<blocks, 256, 0, stream>>>(pa, static_cast<__nv_bfloat16*>(A_cat), in, R);
+    pack_factors_kernel<<<blocks, 256, 0, stream>>>(pa, static_cast<uint16_t*>(A_cat), in, R);
     SOWB_CHECK_CUDA(cudaGetLastError());
   }
   // t_cat [T, R] = scale_i * x . A_cat      (one pass over x for every member of the group)
@@ -460,14 +475,14 @@ int sow_group_fwd(const void* x, const void* x_lo, const sowb_group_member* m, i
     int rsum = 0;
     for (int i = 0; i < n; ++i) rsum += m[i].r;
     rc = launch_skinny<false, true, EPI_BF16_TMA>(R, sg, f32 ? 2 : 1, t_cat, nullptr, R, static_cast<int>(T), alpha, nb, false,
-                                                  stream, PROF_GEMM_SKINNY, 2.0 * double(T) * double(in) * double(rsum));
+                                                  f16, stream, PROF_GEMM_SKINNY, 2.0 * double(T) * double(in) * double(rsum));
     if (rc) return rc;
   }
   // y_i = x . W_i + t_i . B_i (+ bias_i)
   const float one = 1.0f;
   for (int i = 0; i < n; ++i) {
     SOWB_REQUIRE(m[i].y != nullptr, "sow_group_fwd: member %d has no output buffer", i);
-    const __nv_bfloat16* t_i = static_cast<const __nv_bfloat16*>(t_cat) + L.off[i];
+    const uint16_t* t_i = static_cast<const uint16_t*>(t_cat) + L.off[i];
     Segment segs[4];
     int ns = 0;
     if (m[i].W != nullptr) {
@@ -488,14 +503,14 @@ int sow_group_fwd(const void* x, const void* x_lo, const sowb_group_member* m, i
     const double fl = 2.0 * double(T) * double(m[i].out) * (double(m[i].W != nullptr ? in : 0) + double(m[i].r));
     if (f32)
       rc = launch_gemm<256, false, true, EPI_F32_TMA>(segs, ns, nullptr, static_cast<float*>(m[i].y), m[i].out,
-                                                      static_cast<int>(T), m[i].out, &one, 1, m[i].bias, false, stream,
-                                                      PROF_GEMM_FWD, fl);
+                                                      static_cast<int>(T), m[i].out, &one, 1, m[i].bias, false, false,
+                                                      stream, PROF_GEMM_FWD, fl);
     else if (use_big_tiles(static_cast<int>(T), m[i].out, ceil_div(in, kBK) * (m[i].W != nullptr) + L.rpad[i] / kBK))
       rc = launch_gemm<256, false, true, EPI_BF16_TMA, 2>(segs, ns, m[i].y, nullptr, m[i].out, static_cast<int>(T), m[i].out,
-                                                          &one, 1, m[i].bias, false, stream, PROF_GEMM_FWD, fl);
+                                                          &one, 1, m[i].bias, false, f16, stream, PROF_GEMM_FWD, fl);
     else
       rc = launch_gemm<256, false, true, EPI_BF16_TMA>(segs, ns, m[i].y, nullptr, m[i].out, static_cast<int>(T), m[i].out,
-                                                       &one, 1, m[i].bias, false, stream, PROF_GEMM_FWD, fl);
+                                                       &one, 1, m[i].bias, false, f16, stream, PROF_GEMM_FWD, fl);
     if (rc) return rc;
   }
   return SOWB_OK;
@@ -515,16 +530,21 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
   uint8_t* wsp = static_cast<uint8_t*>(ws);
   const int R = L.R;
   const int Ti = static_cast<int>(T);
+  const bool f16 = dtype == SOWB_F16;
+  const CUtensorMapDataType t16 = map_type16(f16);
+  for (int i = 0; i < n; ++i)
+    SOWB_REQUIRE(!f16 || (m[i].W_lo == nullptr && m[i].dy_lo == nullptr), "sow_group_bwd: SOWB_F16 takes no W_lo / dy_lo (member %d)", i);
 
   // ---- K2: one pass over every dY_i -> dt_i (into dt_cat) and the split partials of dB_i^T -------------
-  SOWB_CHECK_CUDA(set_max_smem_once(sow_k2_kernel, size_t(kK2SmemTotal)));
+  auto k2_kernel = f16 ? sow_k2_kernel<true> : sow_k2_kernel<false>;
+  SOWB_CHECK_CUDA(set_max_smem_once(k2_kernel, size_t(kK2SmemTotal)));
   K2Plan plans[kMaxGroup];
   bool uniform = true;
   for (int i = 0; i < n; ++i) {
     SOWB_REQUIRE(m[i].dy != nullptr, "sow_group_bwd: member %d has no upstream gradient", i);
     plans[i] = k2_plan(T, m[i].out);
     if (plans[i].G > 8)
-      SOWB_CHECK_CUDA(cudaFuncSetAttribute(sow_k2_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+      SOWB_CHECK_CUDA(cudaFuncSetAttribute(k2_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     uniform = uniform && plans[i].G == plans[0].G && plans[i].n_launch == plans[0].n_launch && L.rpad[i] == L.rpad[0];
   }
   // members that share the cluster size go into ONE launch with the clusters partitioned among them
@@ -560,17 +580,17 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
           const int i = i0 + std::min(j, cnt - 1);
           const K2Plan& pl = plans[i];
           K2MemberMaps& mm = maps.m[j];
-          rc = make_tensor_map_2d(&mm.dy, m[i].dy, m[i].out, T, uint64_t(m[i].out) * 2, 64, 128, 2);
+          rc = make_tensor_map_2d(&mm.dy, m[i].dy, m[i].out, T, uint64_t(m[i].out) * 2, 64, 128, t16);
           if (rc) return rc;
           const int rows_b = std::min(64, m[i].r - ch * 64);
-          rc = make_tensor_map_2d(&mm.b, static_cast<const __nv_bfloat16*>(m[i].B) + size_t(ch) * 64 * m[i].out, m[i].out,
-                                  rows_b, uint64_t(m[i].out) * 2, 64, 64, 2);
+          rc = make_tensor_map_2d(&mm.b, static_cast<const uint16_t*>(m[i].B) + size_t(ch) * 64 * m[i].out, m[i].out,
+                                  rows_b, uint64_t(m[i].out) * 2, 64, 64, t16);
           if (rc) return rc;
-          rc = make_tensor_map_2d(&mm.t, static_cast<const __nv_bfloat16*>(t_cat) + L.off[i] + ch * 64, 64, T,
-                                  uint64_t(R) * 2, 64, 128, 2);
+          rc = make_tensor_map_2d(&mm.t, static_cast<const uint16_t*>(t_cat) + L.off[i] + ch * 64, 64, T,
+                                  uint64_t(R) * 2, 64, 128, t16);
           if (rc) return rc;
           float* dB_part = reinterpret_cast<float*>(wsp + oB[i]) + size_t(ch) * pl.n_clusters * pl.out_pad * 64;
-          rc = make_tensor_map_2d(&mm.dbp, dB_part, 64, uint64_t(pl.n_clusters) * pl.out_pad, 64 * 4, 32, 32, 4);
+          rc = make_tensor_map_2d(&mm.dbp, dB_part, 64, uint64_t(pl.n_clusters) * pl.out_pad, 64 * 4, 32, 32, CU_TENSOR_MAP_DATA_TYPE_FLOAT32);
           if (rc) return rc;
           K2Member& km = p.m[j];
           const int nblk = ceil_div(m[i].out, 128);
@@ -581,7 +601,7 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
           km.blk_end = std::min(nblk, km.blk_first + pl.blk_per_launch);
           km.dt_accumulate = ln > 0;
           km.scale = m[i].scale;
-          km.dt = static_cast<__nv_bfloat16*>(dt_cat) + L.off[i] + ch * 64;
+          km.dt = static_cast<uint16_t*>(dt_cat) + L.off[i] + ch * 64;
           // algorithmic flops: dt and dB, un-padded r (SURVEY.md 8d)
           if (j < cnt && ln == 0) flops += 4.0 * double(T) * double(m[i].out) * double(rows_b);
         }
@@ -598,7 +618,7 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
         at[0].val.clusterDim.z = 1;
         cfg.attrs = at;
         cfg.numAttrs = pl0.G > 1 ? 1 : 0;
-        SOWB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, sow_k2_kernel, maps, p));
+        SOWB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, k2_kernel, maps, p));
       }
     }
   }
@@ -614,27 +634,28 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
                Operand{dt_cat, uint64_t(T), uint64_t(R), uint64_t(R)}, Ti};  // B operand MN-major: [K=T rows, N=R cols]
     int rsum = 0;
     for (int i = 0; i < n; ++i) rsum += m[i].r;
-    rc = launch_skinny<true, true, EPI_F32_PARTIAL>(R, &sg, 1, nullptr, partA, R, in, &one, 1, true, stream, PROF_GEMM_SPLITK,
+    rc = launch_skinny<true, true, EPI_F32_PARTIAL>(R, &sg, 1, nullptr, partA, R, in, &one, 1, true, f16, stream, PROF_GEMM_SPLITK,
                                                     2.0 * double(T) * double(in) * double(rsum), &splitsA);
     if (rc) return rc;
     if (splitsA > splitk_count(in, R, skinny_bn(R), Ti))
       return set_error(SOWB_EWORKSPACE, "sow_group_bwd: split-K count exceeds the workspace plan");
   }
 
-  // ---- partials -> bf16 dA_i (in, r_i), dB_i (r_i, out_i) ------------------------------------------------------
+  // ---- partials -> 16-bit dA_i (in, r_i), dB_i (r_i, out_i) ------------------------------------------------------
   {
     FinJobs jobs;
     jobs.n = 0;
     int blocks = 0;
     auto flush = [&]() -> int {
       if (jobs.n == 0) return SOWB_OK;
-      finalize_jobs_kernel<<<blocks, dim3(32, 32), 0, stream>>>(jobs);
+      if (f16) finalize_jobs_kernel<true><<<blocks, dim3(32, 32), 0, stream>>>(jobs);
+      else finalize_jobs_kernel<false><<<blocks, dim3(32, 32), 0, stream>>>(jobs);
       SOWB_CHECK_CUDA(cudaGetLastError());
       jobs.n = 0;
       blocks = 0;
       return SOWB_OK;
     };
-    auto add = [&](const float* src, int64_t stride, int splits, int rows, int cols, int ld_src, __nv_bfloat16* dst,
+    auto add = [&](const float* src, int64_t stride, int splits, int rows, int cols, int ld_src, uint16_t* dst,
                    int ld_dst, int transpose) -> int {
       if (jobs.n == kMaxFinJobs) {
         const int rcf = flush();
@@ -657,7 +678,7 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
     };
     for (int i = 0; i < n; ++i) {
       if (m[i].dA != nullptr) {
-        rc = add(partA + L.off[i], int64_t(in) * R, splitsA, in, m[i].r, R, static_cast<__nv_bfloat16*>(m[i].dA), m[i].r, 0);
+        rc = add(partA + L.off[i], int64_t(in) * R, splitsA, in, m[i].r, R, static_cast<uint16_t*>(m[i].dA), m[i].r, 0);
         if (rc) return rc;
       }
       if (m[i].dB != nullptr) {
@@ -665,7 +686,7 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
           const int rows_b = std::min(64, m[i].r - ch * 64);
           const float* src = reinterpret_cast<float*>(wsp + oB[i]) + size_t(ch) * plans[i].n_clusters * plans[i].out_pad * 64;
           rc = add(src, int64_t(plans[i].out_pad) * 64, plans[i].n_clusters, m[i].out, rows_b, 64,
-                   static_cast<__nv_bfloat16*>(m[i].dB) + size_t(ch) * 64 * m[i].out, m[i].out, 1);
+                   static_cast<uint16_t*>(m[i].dB) + size_t(ch) * 64 * m[i].out, m[i].out, 1);
           if (rc) return rc;
         }
       }
@@ -679,10 +700,13 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
     if (m[i].dbias == nullptr) continue;
     float* partBias = reinterpret_cast<float*>(wsp + oBias);
     dim3 grid(ceil_div(m[i].out, 64), static_cast<unsigned>(std::min<int64_t>(kBiasParts, (T + 255) / 256)));
-    colsum_kernel<<<grid, dim3(64, 4), 0, stream>>>(static_cast<const __nv_bfloat16*>(m[i].dy), partBias, T, m[i].out);
+    const uint16_t* dy = static_cast<const uint16_t*>(m[i].dy);
+    uint16_t* db = static_cast<uint16_t*>(m[i].dbias);
+    if (f16) colsum_kernel<true><<<grid, dim3(64, 4), 0, stream>>>(dy, partBias, T, m[i].out);
+    else colsum_kernel<false><<<grid, dim3(64, 4), 0, stream>>>(dy, partBias, T, m[i].out);
     SOWB_CHECK_CUDA(cudaGetLastError());
-    sum_partials_to_bf16_kernel<<<ceil_div(m[i].out, 256), 256, 0, stream>>>(partBias, static_cast<__nv_bfloat16*>(m[i].dbias),
-                                                                            m[i].out, static_cast<int>(grid.y));
+    if (f16) sum_partials_to_16_kernel<true><<<ceil_div(m[i].out, 256), 256, 0, stream>>>(partBias, db, m[i].out, int(grid.y));
+    else sum_partials_to_16_kernel<false><<<ceil_div(m[i].out, 256), 256, 0, stream>>>(partBias, db, m[i].out, int(grid.y));
     SOWB_CHECK_CUDA(cudaGetLastError());
   }
 
@@ -715,12 +739,12 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
     for (int i = 0; i < n; ++i) kalg += double(m[i].W != nullptr ? m[i].out : 0) + double(m[i].r);
     if (f32)
       rc = launch_gemm<256, false, false, EPI_F32_TMA>(segs, ns, nullptr, static_cast<float*>(dx), in, Ti, in, &one, 1, nullptr,
-                                                       false, stream, PROF_GEMM_DX, 2.0 * double(T) * double(in) * kalg);
+                                                       false, false, stream, PROF_GEMM_DX, 2.0 * double(T) * double(in) * kalg);
     else if (use_big_tiles(Ti, in, static_cast<int>(kalg) / kBK))
-      rc = launch_gemm<256, false, false, EPI_BF16_TMA, 2>(segs, ns, dx, nullptr, in, Ti, in, &one, 1, nullptr, false, stream,
+      rc = launch_gemm<256, false, false, EPI_BF16_TMA, 2>(segs, ns, dx, nullptr, in, Ti, in, &one, 1, nullptr, false, f16, stream,
                                                            PROF_GEMM_DX, 2.0 * double(T) * double(in) * kalg);
     else
-      rc = launch_gemm<256, false, false, EPI_BF16_TMA>(segs, ns, dx, nullptr, in, Ti, in, &one, 1, nullptr, false, stream,
+      rc = launch_gemm<256, false, false, EPI_BF16_TMA>(segs, ns, dx, nullptr, in, Ti, in, &one, 1, nullptr, false, f16, stream,
                                                         PROF_GEMM_DX, 2.0 * double(T) * double(in) * kalg);
     if (rc) return rc;
   }

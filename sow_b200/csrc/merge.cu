@@ -29,6 +29,9 @@
 // (4 slots measured no faster: the memory system, not the slot count, binds).  The scalar fields of every table
 // entry are staged in shared memory at kernel start and the next matrix's tensor maps are prefetched one matrix
 // ahead, because under HBM saturation a dependent global load costs microseconds.
+// F16 (template flag): W, A and B are IEEE fp16 instead of bf16 -- the instruction-descriptor format, the widening of
+// W_prev and the one rounding of the new W in the epilogue (TMA element types on the host side).  The A repack and the
+// store group move 16-bit words without interpreting them.
 // Debug aid: sow_merge_debug_timeline() makes CTA 0 record clock64 stamps per tile (tools/merge_timeline.py).
 #include "common.cuh"
 #include "ptx.cuh"
@@ -203,6 +206,7 @@ struct MergeCursor {
   }
 };
 
+template <bool F16>
 __global__ void __launch_bounds__(kMgThreads, 1)
 sow_merge_kernel(const MergeDevEntry* __restrict__ tab, int n_entries, int total_tiles, int prefetch,
                  long long* __restrict__ dbg_ts) {
@@ -382,7 +386,7 @@ sow_merge_kernel(const MergeDevEntry* __restrict__ tab, int n_entries, int total
         const MergeInfo* e = c.e;
         const int r = e->r, lda = e->lda;
         const bool live = row < min(kMgBM, e->in - c.m0);
-        uint32_t w[32];  // the row as 32 packed bf16 pairs, zero beyond r
+        uint32_t w[32];  // the row as 32 packed 16-bit pairs, zero beyond r
         if (e->a_bulk) {
           mbar_wait(astage_full, st_phase);
           st_phase ^= 1;
@@ -425,7 +429,7 @@ sow_merge_kernel(const MergeDevEntry* __restrict__ tab, int n_entries, int total
   } else if (warp == 9) {
     if (lane == 0 && lo < hi) {
       // ===================== MMA issuer =====================
-      constexpr uint32_t idesc = make_idesc(1, kMgBM, kMgBN, 0, 1);
+      constexpr uint32_t idesc = make_idesc(ab_format16<F16>(), kMgBM, kMgBN, 0, 1);
       MergeCursor c;
       c.init(tab, info, n_entries, lo);
       int acc = 0;
@@ -552,15 +556,15 @@ sow_merge_kernel(const MergeDevEntry* __restrict__ tab, int n_entries, int total
             const uint32_t ow[4] = {old.x, old.y, old.z, old.w};
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
-              f[2 * j] += __uint_as_float(ow[j] << 16);
-              f[2 * j + 1] += __uint_as_float(ow[j] & 0xffff0000u);
+              f[2 * j] += lo16_to_f32<F16>(ow[j]);
+              f[2 * j + 1] += hi16_to_f32<F16>(ow[j]);
             }
           }
           uint4 pk;
-          pk.x = pack_bf16x2(f[0], f[1]);
-          pk.y = pack_bf16x2(f[2], f[3]);
-          pk.z = pack_bf16x2(f[4], f[5]);
-          pk.w = pack_bf16x2(f[6], f[7]);
+          pk.x = pack16x2<F16>(f[0], f[1]);
+          pk.y = pack16x2<F16>(f[2], f[3]);
+          pk.z = pack16x2<F16>(f[4], f[5]);
+          pk.w = pack16x2<F16>(f[6], f[7]);
           *p = pk;
         }
         fence_proxy_async_smem();
@@ -767,7 +771,7 @@ static int merge_grouped_f32(const sowb_merge_entry* entries, int n, void* table
 int sow_merge_grouped(const sowb_merge_entry* entries, int n, int dtype, void* table_dev, size_t table_bytes,
                       void* stream_) {
   if (n <= 0) return SOWB_OK;
-  if (dtype != SOWB_BF16 && dtype != SOWB_F32) return set_error(SOWB_EINVAL, "sow_merge_grouped: unknown dtype %d", dtype);
+  if (dtype != SOWB_BF16 && dtype != SOWB_F32 && dtype != SOWB_F16) return set_error(SOWB_EINVAL, "sow_merge_grouped: unknown dtype %d", dtype);
   SOWB_REQUIRE(entries != nullptr && table_dev != nullptr, "sow_merge_grouped: null pointer argument");
   if (int rc0 = ensure_context_for(table_dev)) return rc0;
   if (dtype == SOWB_F32) {
@@ -779,6 +783,9 @@ int sow_merge_grouped(const sowb_merge_entry* entries, int n, int dtype, void* t
   int rc = require_sm100();
   if (rc) return rc;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const bool f16 = dtype == SOWB_F16;
+  const CUtensorMapDataType t16 = map_type16(f16);
+  auto kernel = f16 ? sow_merge_kernel<true> : sow_merge_kernel<false>;
   int max_chunks = 1;
   for (int i = 0; i < n; ++i) {
     const sowb_merge_entry& e = entries[i];
@@ -790,7 +797,7 @@ int sow_merge_grouped(const sowb_merge_entry* entries, int n, int dtype, void* t
   if (table_bytes < size_t(n) * sizeof(MergeDevEntry))
     return set_error(SOWB_EWORKSPACE, "sow_merge_grouped: table %zu B < required %zu B", table_bytes,
                      size_t(n) * sizeof(MergeDevEntry));
-  SOWB_CHECK_CUDA(set_max_smem_once(sow_merge_kernel, size_t(kMgSmemTotal)));
+  SOWB_CHECK_CUDA(set_max_smem_once(kernel, size_t(kMgSmemTotal)));
   const int sms = num_sms();
   // ranks above 64 are applied as successive 64-wide chunks (W_prev = W after the first chunk)
   for (int chunk = 0; chunk < max_chunks; ++chunk) {
@@ -804,16 +811,16 @@ int sow_merge_grouped(const sowb_merge_entry* entries, int n, int dtype, void* t
       memset(&d, 0, sizeof(d));
       const void* prev = (chunk == 0) ? e.W_prev : e.W;
       d.has_prev = prev != nullptr;
-      rc = make_tensor_map_2d(&d.tmWout, e.W, e.out, e.in, uint64_t(e.out) * 2, 64, kMgBM, 2);
+      rc = make_tensor_map_2d(&d.tmWout, e.W, e.out, e.in, uint64_t(e.out) * 2, 64, kMgBM, t16);
       if (rc) return rc;
       d.tmWin = d.tmWout;
       if (prev != nullptr && prev != e.W) {
-        rc = make_tensor_map_2d(&d.tmWin, prev, e.out, e.in, uint64_t(e.out) * 2, 64, kMgBM, 2);
+        rc = make_tensor_map_2d(&d.tmWin, prev, e.out, e.in, uint64_t(e.out) * 2, 64, kMgBM, t16);
         if (rc) return rc;
       }
       const int rc_rows = std::min(64, e.r - r0);
       const __nv_bfloat16* Bp = static_cast<const __nv_bfloat16*>(e.B) + size_t(r0) * e.out;
-      rc = make_tensor_map_2d(&d.tmB, Bp, e.out, rc_rows, uint64_t(e.out) * 2, 64, 64, 2);
+      rc = make_tensor_map_2d(&d.tmB, Bp, e.out, rc_rows, uint64_t(e.out) * 2, 64, 64, t16);
       if (rc) return rc;
       d.A = static_cast<const __nv_bfloat16*>(e.A) + r0;
       d.W = static_cast<__nv_bfloat16*>(e.W);
@@ -850,8 +857,8 @@ int sow_merge_grouped(const sowb_merge_entry* entries, int n, int dtype, void* t
         const char* e = getenv("SOWB_MERGE_PREFETCH");   // tuning knob: tiles of L2 prefetch distance (0 = off)
         return e ? atoi(e) : kMgPrefetchDefault;
       }();
-      sow_merge_kernel<<<grid, kMgThreads, kMgSmemTotal, stream>>>(static_cast<const MergeDevEntry*>(table_dev),
-                                                                   static_cast<int>(cnt), tiles, prefetch, g_merge_ts);
+      kernel<<<grid, kMgThreads, kMgSmemTotal, stream>>>(static_cast<const MergeDevEntry*>(table_dev), static_cast<int>(cnt),
+                                                         tiles, prefetch, g_merge_ts);
       SOWB_CHECK_CUDA(cudaGetLastError());
     }
   }

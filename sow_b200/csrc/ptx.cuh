@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda.h>
 #include <stdint.h>
 
@@ -244,6 +245,29 @@ __host__ __device__ constexpr uint32_t make_idesc(uint32_t ab_format, uint32_t M
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
   return *reinterpret_cast<uint32_t*>(&v);
+}
+
+// The 16-bit operand type of the tcgen05 paths as a template flag: F16 = false -> bf16, true -> IEEE fp16.
+//   kind::f16 instruction-descriptor format: 1 = bf16, 0 = fp16 (same rate).
+//   pack: round to nearest even (cvt.rn.f16x2.f32 / cvt.rn.bf16x2.f32, no .satfinite: fp16 overflow gives +-inf).
+template <bool F16>
+__host__ __device__ constexpr uint32_t ab_format16() { return F16 ? 0u : 1u; }
+template <bool F16>
+__device__ __forceinline__ uint32_t pack16x2(float lo, float hi) {
+  if (F16) {
+    __half2 v = __floats2half2_rn(lo, hi);
+    return *reinterpret_cast<uint32_t*>(&v);
+  }
+  return pack_bf16x2(lo, hi);
+}
+// the low / high 16-bit element of a packed pair, widened exactly to fp32
+template <bool F16>
+__device__ __forceinline__ float lo16_to_f32(uint32_t w) {
+  return F16 ? __half2float(__ushort_as_half(static_cast<unsigned short>(w & 0xffffu))) : __uint_as_float(w << 16);
+}
+template <bool F16>
+__device__ __forceinline__ float hi16_to_f32(uint32_t w) {
+  return F16 ? __half2float(__ushort_as_half(static_cast<unsigned short>(w >> 16))) : __uint_as_float(w & 0xffff0000u);
 }
 
 // ----------------------------------------------------------------------------------------------

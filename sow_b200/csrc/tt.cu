@@ -2275,6 +2275,7 @@ static int adam2_common(bool head, void* p, const void* g, const float* G1m, con
   float* part = static_cast<float*>(ws);
   const float beta1 = float(beta1_d), beta2 = float(beta2_d), omb1 = float(1.0 - beta1_d), omb2 = float(1.0 - beta2_d);
   SOWB_REQUIRE(g != nullptr, "tt_adam2: null gradient pointer");
+  SOWB_REQUIRE_TT_DTYPE("tt_adam2", dtype);
   if (int rc0 = ensure_context_for(g)) return rc0;
   SOWB_REQUIRE(first_step || (G1m && G2m && G1v && G2v), "tt_adam2: null core pointer");
   SOWB_REQUIRE(r > 0 && r <= 64, "tt_adam2: rank %d unsupported (1..64)", r);
@@ -2523,6 +2524,7 @@ int tt_project(const float* L, int64_t l_batch_stride, const float* Q, int64_t q
 
 int tt_gather2(const void* src, int M, int N, int mm, int nn, float* X, int ncols, int dtype, void* stream_) {
   SOWB_REQUIRE(src && X, "tt_gather2: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_gather2", dtype);
   SOWB_REQUIRE(mm > 0 && nn > 0 && ncols > 0 && int64_t(mm) * mm >= M && int64_t(nn) * nn >= N, "tt_gather2: bad shape");
   if (int rc0 = ensure_context_for(src)) return rc0;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
@@ -2548,6 +2550,7 @@ size_t tt_project2_workspace_bytes(int mm, int nn, int r) {
 int tt_project2(const void* src, int M, int N, int mm, int nn, const float* Q, float* R, int r, int dtype, void* ws,
                 size_t ws_bytes, void* stream_) {
   SOWB_REQUIRE(src && Q && R, "tt_project2: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_project2", dtype);
   SOWB_REQUIRE(mm > 0 && nn > 0 && r > 0 && int64_t(mm) * mm >= M && int64_t(nn) * nn >= N, "tt_project2: bad shape");
   SOWB_REQUIRE(dtype == SOWB_BF16 || dtype == SOWB_F32, "tt_project2: unknown dtype %d", dtype);
   if (int rc0 = ensure_context_for(src)) return rc0;
@@ -2583,6 +2586,7 @@ int tt_project2(const void* src, int M, int N, int mm, int nn, const float* Q, f
 
 int tt_reconstruct2(const float* G1, const float* G2, int r, void* dst, int M, int N, int mm, int nn, int dtype, void* stream_) {
   SOWB_REQUIRE(G1 && G2 && dst, "tt_reconstruct2: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_reconstruct2", dtype);
   SOWB_REQUIRE(mm > 0 && nn > 0 && r > 0 && int64_t(mm) * mm >= M && int64_t(nn) * nn >= N, "tt_reconstruct2: bad shape");
   if (int rc0 = ensure_context_for(G1)) return rc0;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
@@ -2630,6 +2634,7 @@ int tt_reconstruct2(const float* G1, const float* G2, int r, void* dst, int M, i
 
 int tt_interleave(const void* src, int M, int N, int mm, int nn, int order, float* out, int dtype, void* stream_) {
   SOWB_REQUIRE(src && out, "tt_interleave: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_interleave", dtype);
   if (int rc0 = ensure_context_for(src)) return rc0;
   SOWB_REQUIRE(order >= 1 && order <= 8 && mm > 0 && nn > 0, "tt_interleave: bad order/shape");
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
@@ -2661,6 +2666,7 @@ int tt_interleave(const void* src, int M, int N, int mm, int nn, int order, floa
 
 int tt_deinterleave(const float* src, int M, int N, int mm, int nn, int order, void* out, int dtype, void* stream_) {
   SOWB_REQUIRE(src && out, "tt_deinterleave: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_deinterleave", dtype);
   if (int rc0 = ensure_context_for(src)) return rc0;
   SOWB_REQUIRE(order >= 1 && order <= 8 && mm > 0 && nn > 0, "tt_deinterleave: bad order/shape");
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
@@ -2732,6 +2738,7 @@ int tt_adam_fused2(void* p, const void* g, const float* G1m, const float* G2m, c
   const float beta1 = float(beta1_d), beta2 = float(beta2_d), omb1 = float(1.0 - beta1_d), omb2 = float(1.0 - beta2_d);
   const float eps = float(eps_d), step_size = float(step_size_d), lr_wd = float(lr_wd_d);
   SOWB_REQUIRE(p && g && m_out && v_out, "tt_adam_fused2: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_adam_fused2", dtype);
   if (int rc0 = ensure_context_for(g)) return rc0;
   SOWB_REQUIRE(first_step || (G1m && G2m && G1v && G2v), "tt_adam_fused2: null core pointer");
   SOWB_REQUIRE(r > 0 && r <= 128, "tt_adam_fused2: rank %d unsupported (1..128)", r);
@@ -2762,6 +2769,7 @@ int tt_adam_interleaved(void* p, const void* g, float* m, float* v, int M, int N
   const float beta1 = float(beta1_d), beta2 = float(beta2_d), omb1 = float(1.0 - beta1_d), omb2 = float(1.0 - beta2_d);
   const float eps = float(eps_d), step_size = float(step_size_d), lr_wd = float(lr_wd_d);
   SOWB_REQUIRE(p && g && m && v, "tt_adam_interleaved: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_adam_interleaved", dtype);
   SOWB_REQUIRE(order >= 1 && order <= 8 && mm > 0 && nn > 0, "tt_adam_interleaved: bad order/shape");
   if (int rc0 = ensure_context_for(g)) return rc0;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
@@ -2847,6 +2855,7 @@ int tt_adam_nd_step(void* p, const void* g, const float* const* cores_in, float*
                   int mm, int nn, int order, double beta1, double beta2, double eps, double step_size, double lr_wd,
                   int first_step, int dtype, void* ws, size_t ws_bytes, void* stream_) {
   SOWB_REQUIRE(p && g && cores_out && ranks && ws, "tt_adam_nd_step: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_adam_nd_step", dtype);
   SOWB_REQUIRE(first_step || cores_in, "tt_adam_nd_step: null core table");
   const AdamNPlan pl = adamN_plan(mm, nn, order, ranks);
   SOWB_REQUIRE(pl.ok, "tt_adam_nd_step: unsupported order / ranks (order 3..8, boundary ranks 1, inner ranks <= 64 and <= the unfolding sizes)");
@@ -2911,6 +2920,7 @@ size_t tt_nd_workspace_bytes(int mm, int nn, int order, const int* ranks) {
 int tt_decompose_nd(const void* src, float* const* cores_out, const int* ranks, int M, int N, int mm, int nn, int order, int dtype,
                     void* ws, size_t ws_bytes, void* stream_) {
   SOWB_REQUIRE(src && cores_out && ranks && ws, "tt_decompose_nd: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_decompose_nd", dtype);
   const AdamNPlan pl = adamN_plan(mm, nn, order, ranks, 1);
   SOWB_REQUIRE(pl.ok, "tt_decompose_nd: unsupported order / ranks");
   SOWB_REQUIRE((reinterpret_cast<uintptr_t>(ws) & 255) == 0, "tt_decompose_nd: workspace must be 256-byte aligned");
@@ -2940,6 +2950,7 @@ int tt_decompose_nd(const void* src, float* const* cores_out, const int* ranks, 
 int tt_reconstruct_nd(const float* const* cores, const int* ranks, void* dst, int M, int N, int mm, int nn, int order, int dtype,
                       void* ws, size_t ws_bytes, void* stream_) {
   SOWB_REQUIRE(cores && ranks && dst && ws, "tt_reconstruct_nd: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_reconstruct_nd", dtype);
   const AdamNPlan pl = adamN_plan(mm, nn, order, ranks, 1);
   SOWB_REQUIRE(pl.ok, "tt_reconstruct_nd: unsupported order / ranks");
   SOWB_REQUIRE((reinterpret_cast<uintptr_t>(ws) & 255) == 0, "tt_reconstruct_nd: workspace must be 256-byte aligned");
@@ -2967,6 +2978,7 @@ int tt_adam_dense(void* p, const void* g, float* m, float* v, int64_t numel, dou
   const float beta1 = float(beta1_d), beta2 = float(beta2_d), omb1 = float(1.0 - beta1_d), omb2 = float(1.0 - beta2_d);
   const float eps = float(eps_d), step_size = float(step_size_d), lr_wd = float(lr_wd_d);
   SOWB_REQUIRE(p && g && m && v && numel > 0, "tt_adam_dense: bad argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_adam_dense", dtype);
   if (int rc0 = ensure_context_for(g)) return rc0;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   if (dtype == SOWB_BF16)

@@ -566,6 +566,7 @@ int tt_adam2_step(void* p, const void* g, const float* G1m, const float* G2m, co
                   double eps, double step_size, double lr_wd, int first_step, int dtype, void* ws, size_t ws_bytes,
                   void* stream_) {
   SOWB_REQUIRE(p && g && Qm && Qv && Rm && Rv && ws, "tt_adam2_step: null pointer argument");
+  SOWB_REQUIRE_TT_DTYPE("tt_adam2_step", dtype);
   if (int rc0 = ensure_context_for(g)) return rc0;
   SOWB_REQUIRE(first_step || (G1m && G2m && G1v && G2v), "tt_adam2_step: null core pointer");
   SOWB_REQUIRE(r > 0 && r <= 64, "tt_adam2_step: rank %d unsupported (1..64)", r);
@@ -631,17 +632,17 @@ int tt_adam2_step(void* p, const void* g, const float* G1m, const float* G2m, co
   CUtensorMap tmG1m, tmG1v, tmG2m, tmG2v, tmQm, tmQv;
   const __nv_bfloat16* g1m_src = first_step ? pcs[4] : pcs[0];   // unused maps still need a valid base address
   const __nv_bfloat16* g1v_src = first_step ? pcs[5] : pcs[1];
-  rc = make_tensor_map_2d(&tmG1m, g1m_src, 64, uint64_t(3) * P_pad, 128, 64, 128, 2);
+  rc = make_tensor_map_2d(&tmG1m, g1m_src, 64, uint64_t(3) * P_pad, 128, 64, 128, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
   if (rc) return rc;
-  rc = make_tensor_map_2d(&tmG1v, g1v_src, 64, uint64_t(3) * P_pad, 128, 64, 128, 2);
+  rc = make_tensor_map_2d(&tmG1v, g1v_src, 64, uint64_t(3) * P_pad, 128, 64, 128, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
   if (rc) return rc;
-  rc = make_tensor_map_2d(&tmG2m, pcs[2], P_pad, 3 * 64, uint64_t(P_pad) * 2, 64, 64, 2);
+  rc = make_tensor_map_2d(&tmG2m, pcs[2], P_pad, 3 * 64, uint64_t(P_pad) * 2, 64, 64, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
   if (rc) return rc;
-  rc = make_tensor_map_2d(&tmG2v, pcs[3], P_pad, 3 * 64, uint64_t(P_pad) * 2, 64, 64, 2);
+  rc = make_tensor_map_2d(&tmG2v, pcs[3], P_pad, 3 * 64, uint64_t(P_pad) * 2, 64, 64, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
   if (rc) return rc;
-  rc = make_tensor_map_2d(&tmQm, pcs[4], 64, uint64_t(3) * P_pad, 128, 64, 128, 2);
+  rc = make_tensor_map_2d(&tmQm, pcs[4], 64, uint64_t(3) * P_pad, 128, 64, 128, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
   if (rc) return rc;
-  rc = make_tensor_map_2d(&tmQv, pcs[5], 64, uint64_t(3) * P_pad, 128, 64, 128, 2);
+  rc = make_tensor_map_2d(&tmQv, pcs[5], 64, uint64_t(3) * P_pad, 128, 64, 128, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
   if (rc) return rc;
 
   TcParams prm;

@@ -16,12 +16,19 @@ from torch import Tensor
 from . import ops
 
 
-def _bf16c(t: Optional[Tensor]) -> Optional[Tensor]:
+def _bf16c(t: Optional[Tensor], dt: torch.dtype = torch.bfloat16) -> Optional[Tensor]:
+    """``t`` as a contiguous tensor of the 16-bit compute dtype ``dt`` (bf16, or fp16 on the fp16 path)."""
     if t is None:
         return None
-    if t.dtype != torch.bfloat16:
-        t = t.to(torch.bfloat16)
+    if t.dtype != dt:
+        t = t.to(dt)
     return t if t.is_contiguous() else t.contiguous()
+
+
+def _half_dtype(x: Tensor, Ws, f32: bool) -> torch.dtype:
+    """16-bit compute dtype of a call: fp16 when x and every dense W are fp16 (layer._native_f16), else bf16."""
+    f16 = not f32 and x.dtype == torch.float16 and all(w is None or w.dtype == torch.float16 for w in Ws)
+    return torch.float16 if f16 else torch.bfloat16
 
 
 # bf16 pieces of fp32 accumulation weights, keyed by storage address.  The ops take the user-visible W (any dtype) so
@@ -34,11 +41,12 @@ def invalidate_weight_cache() -> None:
     _w_pieces.clear()
 
 
-def _weight_pieces(W: Optional[Tensor], want_f32: bool):
-    """(W_c, W_lo): bf16 W -> (W, None); fp32 W with an fp32 caller -> its two bf16 pieces (cached); else one bf16 copy."""
+def _weight_pieces(W: Optional[Tensor], want_f32: bool, hdt: torch.dtype = torch.bfloat16):
+    """(W_c, W_lo): W of the compute dtype ``hdt`` (bf16, or fp16 on the fp16 path) -> (W, None); fp32 W with an fp32
+    caller -> its two bf16 pieces (cached); else one bf16 copy."""
     if W is None or W.numel() == 0:
         return None, None
-    if W.dtype == torch.bfloat16 and W.is_contiguous():
+    if W.dtype == hdt and W.is_contiguous():
         return W, None
     key = (W.data_ptr(), W._version, W.dtype, want_f32)
     hit = _w_pieces.get(W.data_ptr())
@@ -55,22 +63,24 @@ def _weight_pieces(W: Optional[Tensor], want_f32: bool):
 
 @torch.library.custom_op("sow_b200::linear_fwd", mutates_args=())
 def linear_fwd(x: Tensor, W: Optional[Tensor], A: Tensor, B: Tensor, bias: Optional[Tensor], scale: float) -> List[Tensor]:
-    """[y (..., out) in x.dtype, A_pad (in, r_pad) bf16, t (T, r_pad) bf16].  W: acc_downweight (any dtype) or None."""
+    """[y (..., out) in x.dtype, A_pad (in, r_pad), t (T, r_pad)] with A_pad / t fp16 on the fp16 path, else bf16.
+    W: acc_downweight (any dtype) or None."""
     fin = A.shape[0]
     lead = x.shape[:-1]
+    f32 = x.dtype == torch.float32 and W is not None and W.dtype == torch.float32 and (bias is None or bias.dtype == torch.float32)
+    hdt = _half_dtype(x, [W], f32)
     if x.numel() == 0:
         rp = ops.rank_pad(A.shape[1])
-        return [x.new_zeros(*lead, B.shape[1]), x.new_zeros((fin, rp), dtype=torch.bfloat16),
-                x.new_zeros((0, rp), dtype=torch.bfloat16)]
-    f32 = x.dtype == torch.float32 and W is not None and W.dtype == torch.float32 and (bias is None or bias.dtype == torch.float32)
-    W, W_lo = _weight_pieces(W, f32)
+        return [x.new_zeros(*lead, B.shape[1]), x.new_zeros((fin, rp), dtype=hdt), x.new_zeros((0, rp), dtype=hdt)]
+    W, W_lo = _weight_pieces(W, f32, hdt)
     if f32:
         xf = x.reshape(-1, fin)
         x_hi, x_lo = ops.split_f32(xf if xf.is_contiguous() else xf.contiguous())
         ys, A_cat, t_cat = ops.group_fwd(x_hi, [(W, _bf16c(A), _bf16c(B), None if bias is None else bias.contiguous(),
                                                  scale, W_lo)], x_lo=x_lo)
     else:
-        ys, A_cat, t_cat = ops.group_fwd(_bf16c(x.reshape(-1, fin)), [(_bf16c(W), _bf16c(A), _bf16c(B), _bf16c(bias), scale)])
+        ys, A_cat, t_cat = ops.group_fwd(_bf16c(x.reshape(-1, fin), hdt),
+                                         [(_bf16c(W, hdt), _bf16c(A, hdt), _bf16c(B, hdt), _bf16c(bias, hdt), scale)])
     y = ys[0].reshape(*lead, B.shape[1])
     return [y if y.dtype == x.dtype else y.to(x.dtype), A_cat, t_cat]
 
@@ -80,22 +90,24 @@ def _(x, W, A, B, bias, scale):
     fin = A.shape[0]
     rp = (A.shape[1] + 63) // 64 * 64
     T = x.numel() // fin
-    return [x.new_empty((*x.shape[:-1], B.shape[1])), x.new_empty((fin, rp), dtype=torch.bfloat16),
-            x.new_empty((T, rp), dtype=torch.bfloat16)]
+    f32 = x.dtype == torch.float32 and W is not None and W.dtype == torch.float32 and (bias is None or bias.dtype == torch.float32)
+    hdt = _half_dtype(x, [W], f32)
+    return [x.new_empty((*x.shape[:-1], B.shape[1])), x.new_empty((fin, rp), dtype=hdt), x.new_empty((T, rp), dtype=hdt)]
 
 
 @torch.library.custom_op("sow_b200::linear_bwd", mutates_args=())
 def linear_bwd(dy: Tensor, x: Tensor, W: Optional[Tensor], A_pad: Tensor, t: Tensor, B: Tensor, scale: float, r: int,
                need_dx: bool, need_dbias: bool, f32: bool) -> List[Tensor]:
-    """[dx (x.shape, x.dtype; empty if not needed), dA (in, r) bf16, dB (r, out) bf16, dbias (out) bf16 or empty]."""
+    """[dx (x.shape, x.dtype; empty if not needed), dA (in, r), dB (r, out), dbias (out) or empty]; the gradients have t's
+    dtype (fp16 on the fp16 path, else bf16)."""
     fin = A_pad.shape[0]
     fout = B.shape[1]
     dev = x.device
+    hdt = t.dtype
     if x.numel() == 0:
-        return [x.new_zeros(x.shape if need_dx else (0,)), torch.zeros((fin, r), dtype=torch.bfloat16, device=dev),
-                torch.zeros((r, fout), dtype=torch.bfloat16, device=dev),
-                torch.zeros((fout if need_dbias else 0,), dtype=torch.bfloat16, device=dev)]
-    W, W_lo = _weight_pieces(W, f32)
+        return [x.new_zeros(x.shape if need_dx else (0,)), torch.zeros((fin, r), dtype=hdt, device=dev),
+                torch.zeros((r, fout), dtype=hdt, device=dev), torch.zeros((fout if need_dbias else 0,), dtype=hdt, device=dev)]
+    W, W_lo = _weight_pieces(W, f32, hdt)
     dy2 = dy.reshape(-1, fout)
     if f32:
         xf = x.reshape(-1, fin)
@@ -105,22 +117,22 @@ def linear_bwd(dy: Tensor, x: Tensor, W: Optional[Tensor], A_pad: Tensor, t: Ten
         member = (W, _bf16c(B), dy_hi, scale, True, True, need_dbias, W_lo, dy_lo)
         dx, dAs, dBs, dbs = ops.group_bwd(x_hi, A_pad, t, [member], need_dx, f32=True)
     else:
-        member = (_bf16c(W), _bf16c(B), _bf16c(dy2), scale, True, True, need_dbias)
-        dx, dAs, dBs, dbs = ops.group_bwd(_bf16c(x.reshape(-1, fin)), A_pad, t, [member], need_dx)
+        member = (_bf16c(W, hdt), _bf16c(B, hdt), _bf16c(dy2, hdt), scale, True, True, need_dbias)
+        dx, dAs, dBs, dbs = ops.group_bwd(_bf16c(x.reshape(-1, fin), hdt), A_pad, t, [member], need_dx)
     if dx is None:
         dx = x.new_zeros((0,))
     else:
         dx = dx.reshape(x.shape)
         dx = dx if dx.dtype == x.dtype else dx.to(x.dtype)
-    db = dbs[0] if dbs[0] is not None else torch.zeros((0,), dtype=torch.bfloat16, device=dev)
+    db = dbs[0] if dbs[0] is not None else torch.zeros((0,), dtype=hdt, device=dev)
     return [dx, dAs[0], dBs[0], db]
 
 
 @linear_bwd.register_fake
 def _(dy, x, W, A_pad, t, B, scale, r, need_dx, need_dbias, f32):
     fin, fout = A_pad.shape[0], B.shape[1]
-    return [x.new_empty(x.shape if need_dx else (0,)), x.new_empty((fin, r), dtype=torch.bfloat16),
-            x.new_empty((r, fout), dtype=torch.bfloat16), x.new_empty((fout if need_dbias else 0,), dtype=torch.bfloat16)]
+    return [x.new_empty(x.shape if need_dx else (0,)), x.new_empty((fin, r), dtype=t.dtype),
+            x.new_empty((r, fout), dtype=t.dtype), x.new_empty((fout if need_dbias else 0,), dtype=t.dtype)]
 
 
 def _setup_context(ctx, inputs, output):
@@ -162,21 +174,27 @@ def sow_linear_traceable(x: Tensor, W: Optional[Tensor], A: Tensor, B: Tensor, b
 from typing import Sequence  # noqa: E402
 
 
+def _group_f32(x: Tensor, Ws, biases) -> bool:
+    """The fp32-faithful (bf16x3) path of a group: fp32 x, at least one dense W, and every W and bias fp32."""
+    return bool(x.dtype == torch.float32 and any(w is not None for w in Ws)
+                and all(w is None or w.dtype == torch.float32 for w in Ws)
+                and all(b is None or b.dtype == torch.float32 for b in biases))
+
+
 @torch.library.custom_op("sow_b200::group_fwd", mutates_args=())
 def group_fwd(x: Tensor, Ws: Sequence[Optional[Tensor]], As: Sequence[Tensor], Bs: Sequence[Tensor],
               biases: Sequence[Optional[Tensor]], scales: Sequence[float]) -> List[Tensor]:
-    """[y_0 .. y_{n-1} (x.dtype), A_cat (in, R) bf16, t_cat (T, R) bf16] for n projections that read the same x."""
+    """[y_0 .. y_{n-1} (x.dtype), A_cat (in, R), t_cat (T, R)] for n projections that read the same x; A_cat / t_cat
+    fp16 on the fp16 path, else bf16."""
     n = len(As)
     fin = As[0].shape[0]
     lead = x.shape[:-1]
     R = sum(ops.rank_pad(a.shape[1]) for a in As)
+    f32 = _group_f32(x, Ws, biases)
+    hdt = _half_dtype(x, Ws, f32)
     if x.numel() == 0:
-        return [x.new_zeros(*lead, b.shape[1]) for b in Bs] + [x.new_zeros((fin, R), dtype=torch.bfloat16),
-                                                              x.new_zeros((0, R), dtype=torch.bfloat16)]
-    f32 = (x.dtype == torch.float32 and any(w is not None for w in Ws)
-           and all(w is None or w.dtype == torch.float32 for w in Ws)
-           and all(b is None or b.dtype == torch.float32 for b in biases))
-    pieces = [_weight_pieces(w, f32) for w in Ws]
+        return [x.new_zeros(*lead, b.shape[1]) for b in Bs] + [x.new_zeros((fin, R), dtype=hdt), x.new_zeros((0, R), dtype=hdt)]
+    pieces = [_weight_pieces(w, f32, hdt) for w in Ws]
     if f32:
         xf = x.reshape(-1, fin)
         x_hi, x_lo = ops.split_f32(xf if xf.is_contiguous() else xf.contiguous())
@@ -185,8 +203,8 @@ def group_fwd(x: Tensor, Ws: Sequence[Optional[Tensor]], As: Sequence[Tensor], B
                     scales[i], pieces[i][1]) for i in range(n)], x_lo=x_lo)
     else:
         ys, A_cat, t_cat = ops.group_fwd(
-            _bf16c(x.reshape(-1, fin)),
-            [(pieces[i][0], _bf16c(As[i]), _bf16c(Bs[i]), _bf16c(biases[i]), scales[i]) for i in range(n)])
+            _bf16c(x.reshape(-1, fin), hdt),
+            [(pieces[i][0], _bf16c(As[i], hdt), _bf16c(Bs[i], hdt), _bf16c(biases[i], hdt), scales[i]) for i in range(n)])
     outs = []
     for y, b in zip(ys, Bs):
         y = y.reshape(*lead, b.shape[1])
@@ -199,30 +217,33 @@ def _(x, Ws, As, Bs, biases, scales):
     fin = As[0].shape[0]
     R = sum((a.shape[1] + 63) // 64 * 64 for a in As)
     T = x.numel() // fin
-    return [x.new_empty((*x.shape[:-1], b.shape[1])) for b in Bs] + [x.new_empty((fin, R), dtype=torch.bfloat16),
-                                                                    x.new_empty((T, R), dtype=torch.bfloat16)]
+    hdt = _half_dtype(x, Ws, _group_f32(x, Ws, biases))
+    return [x.new_empty((*x.shape[:-1], b.shape[1])) for b in Bs] + [x.new_empty((fin, R), dtype=hdt),
+                                                                    x.new_empty((T, R), dtype=hdt)]
 
 
 @torch.library.custom_op("sow_b200::group_bwd", mutates_args=())
 def group_bwd(dys: Sequence[Tensor], x: Tensor, Ws: Sequence[Optional[Tensor]], A_cat: Tensor, t_cat: Tensor,
               Bs: Sequence[Tensor], scales: Sequence[float], ranks: Sequence[int], need_dx: bool,
               need_dbias: Sequence[bool], f32: bool) -> List[Tensor]:
-    """[dx (empty if not needed)] + [dA_i (in, r_i) bf16] + [dB_i (r_i, out_i) bf16] + [dbias_i (out_i) bf16 or empty]."""
+    """[dx (empty if not needed)] + [dA_i (in, r_i)] + [dB_i (r_i, out_i)] + [dbias_i (out_i) or empty]; the gradients
+    have t_cat's dtype (fp16 on the fp16 path, else bf16)."""
     n = len(Bs)
     fin = A_cat.shape[0]
     dev = x.device
+    hdt = t_cat.dtype
     if x.numel() == 0:
         return ([x.new_zeros(x.shape if need_dx else (0,))]
-                + [torch.zeros((fin, ranks[i]), dtype=torch.bfloat16, device=dev) for i in range(n)]
-                + [torch.zeros((ranks[i], Bs[i].shape[1]), dtype=torch.bfloat16, device=dev) for i in range(n)]
-                + [torch.zeros((Bs[i].shape[1] if need_dbias[i] else 0,), dtype=torch.bfloat16, device=dev) for i in range(n)])
-    pieces = [_weight_pieces(w, f32) for w in Ws]
+                + [torch.zeros((fin, ranks[i]), dtype=hdt, device=dev) for i in range(n)]
+                + [torch.zeros((ranks[i], Bs[i].shape[1]), dtype=hdt, device=dev) for i in range(n)]
+                + [torch.zeros((Bs[i].shape[1] if need_dbias[i] else 0,), dtype=hdt, device=dev) for i in range(n)])
+    pieces = [_weight_pieces(w, f32, hdt) for w in Ws]
     members = []
     if f32:
         xf = x.reshape(-1, fin)
         x2, _ = ops.split_f32(xf if xf.is_contiguous() else xf.contiguous())
     else:
-        x2 = _bf16c(x.reshape(-1, fin))
+        x2 = _bf16c(x.reshape(-1, fin), hdt)
     for i in range(n):
         dy2 = dys[i].reshape(-1, Bs[i].shape[1])
         if f32:
@@ -231,14 +252,14 @@ def group_bwd(dys: Sequence[Tensor], x: Tensor, Ws: Sequence[Optional[Tensor]], 
             members.append((pieces[i][0], _bf16c(Bs[i]), dy_hi, scales[i], True, True, need_dbias[i], pieces[i][1],
                             dy_lo if pieces[i][0] is not None else None))
         else:
-            members.append((pieces[i][0], _bf16c(Bs[i]), _bf16c(dy2), scales[i], True, True, need_dbias[i]))
+            members.append((pieces[i][0], _bf16c(Bs[i], hdt), _bf16c(dy2, hdt), scales[i], True, True, need_dbias[i]))
     dx, dAs, dBs, dbs = ops.group_bwd(x2, A_cat, t_cat, members, need_dx, f32=f32)
     if dx is None:
         dx = x.new_zeros((0,))
     else:
         dx = dx.reshape(x.shape)
         dx = dx if dx.dtype == x.dtype else dx.to(x.dtype)
-    dbs = [d if d is not None else torch.zeros((0,), dtype=torch.bfloat16, device=dev) for d in dbs]
+    dbs = [d if d is not None else torch.zeros((0,), dtype=hdt, device=dev) for d in dbs]
     return [dx] + list(dAs) + list(dBs) + dbs
 
 
@@ -246,10 +267,11 @@ def group_bwd(dys: Sequence[Tensor], x: Tensor, Ws: Sequence[Optional[Tensor]], 
 def _(dys, x, Ws, A_cat, t_cat, Bs, scales, ranks, need_dx, need_dbias, f32):
     n = len(Bs)
     fin = A_cat.shape[0]
+    hdt = t_cat.dtype
     return ([x.new_empty(x.shape if need_dx else (0,))]
-            + [x.new_empty((fin, ranks[i]), dtype=torch.bfloat16) for i in range(n)]
-            + [x.new_empty((ranks[i], Bs[i].shape[1]), dtype=torch.bfloat16) for i in range(n)]
-            + [x.new_empty((Bs[i].shape[1] if need_dbias[i] else 0,), dtype=torch.bfloat16) for i in range(n)])
+            + [x.new_empty((fin, ranks[i]), dtype=hdt) for i in range(n)]
+            + [x.new_empty((ranks[i], Bs[i].shape[1]), dtype=hdt) for i in range(n)]
+            + [x.new_empty((Bs[i].shape[1] if need_dbias[i] else 0,), dtype=hdt) for i in range(n)])
 
 
 def _group_setup_context(ctx, inputs, output):
@@ -261,9 +283,7 @@ def _group_setup_context(ctx, inputs, output):
     ctx.scales = [float(s) for s in scales]
     ctx.ranks = [int(a.shape[1]) for a in As]
     ctx.dtypes = ([a.dtype for a in As], [b.dtype for b in Bs], [None if b is None else b.dtype for b in biases])
-    ctx.f32 = bool(x.dtype == torch.float32 and any(w is not None for w in Ws)
-                   and all(w is None or w.dtype == torch.float32 for w in Ws)
-                   and all(b is None or b.dtype == torch.float32 for b in biases))
+    ctx.f32 = _group_f32(x, Ws, biases)
 
 
 def _group_backward(ctx, grads):

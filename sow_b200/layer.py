@@ -55,22 +55,33 @@ class SoWParameter(nn.ParameterList):
 # autograd bridge
 # ---------------------------------------------------------------------------------------------------------
 
-def _bf16c(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+def _halfc(t: Optional[torch.Tensor], dt: torch.dtype) -> Optional[torch.Tensor]:
+    """``t`` as a contiguous tensor of the 16-bit compute dtype ``dt`` (no copy when it already is one)."""
     if t is None:
         return None
-    if t.dtype != torch.bfloat16:
-        t = t.to(torch.bfloat16)
+    if t.dtype != dt:
+        t = t.to(dt)
     return t if t.is_contiguous() else t.contiguous()
 
 
-def _grad_dst(param: Optional[torch.Tensor]):
+def _bf16c(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+    return _halfc(t, torch.bfloat16)
+
+
+def _native_f16(x_dtype: torch.dtype, Ws) -> bool:
+    """The fp16 path: fp16 activations and every dense W of the group fp16 (no W yet counts as fp16)."""
+    return x_dtype == torch.float16 and all(w is None or w.dtype == torch.float16 for w in Ws)
+
+
+def _grad_dst(param: Optional[torch.Tensor], dt: torch.dtype = torch.bfloat16):
     """Where the kernels should write the gradient of a factor: the parameter's view into a flat gradient bucket
     (``_sow_grad_view``, set by parallel.FlatGradSync) when the parameter has no gradient yet -- autograd's AccumulateGrad
-    then adopts the returned view as ``param.grad`` without a copy or an add -- else a fresh tensor."""
+    then adopts the returned view as ``param.grad`` without a copy or an add -- else a fresh tensor.  ``dt``: the dtype
+    the kernels write (bf16, or fp16 on the fp16 path)."""
     if param is None:
         return True
     view = getattr(param, "_sow_grad_view", None)
-    if view is not None and param.grad is None and view.dtype == torch.bfloat16:
+    if view is not None and param.grad is None and view.dtype == dt:
         return view
     return True
 
@@ -81,6 +92,8 @@ class _SoWGroupFn(torch.autograd.Function):
 
     Positional inputs after ``scales``: for each member (W_c or None, A, B, bias or None, W_lo or None).
       * bf16 modules: ``W_c`` is W itself, everything runs in bf16 with fp32 accumulation.
+      * fp16 modules (fp16 x and every dense W fp16): the same in fp16 -- no cast of x, dY or W; factors and biases of
+        another dtype are rounded to fp16 once per call and their gradients returned in their own dtype.
       * fp32 modules (fp32 x, and every dense W given as its two bf16 pieces W_c + W_lo, see SoWLinear._compute_weight):
         the fp32-faithful path -- x and dY are split into two bf16 pieces on the fly, the base products run as bf16x3
         tensor-core contractions, outputs and dX are fp32; the small rank-r factors are rounded to bf16 once.
@@ -104,7 +117,9 @@ class _SoWGroupFn(torch.autograd.Function):
         f32 = (x.dtype == torch.float32 and all((w is None) == (wl is None) for w, wl in zip(Ws, Wlos))
                and all(b is None or b.dtype == torch.float32 for b in biases) and any(w is not None for w in Ws))
         ctx.f32 = f32
-        Bc = [_bf16c(b) for b in Bs]
+        hdt = torch.float16 if (not f32 and _native_f16(x.dtype, Ws)) else torch.bfloat16
+        ctx.hdt = hdt
+        Bc = [_halfc(b, hdt) for b in Bs]
         if f32:
             xf = x.reshape(-1, fin)
             x2, x_lo = ops.split_f32(xf if xf.is_contiguous() else xf.contiguous())
@@ -113,11 +128,11 @@ class _SoWGroupFn(torch.autograd.Function):
                 x2, [(Wc[i], _bf16c(As[i]), Bc[i], None if biases[i] is None else biases[i].contiguous(), scales[i], Wl[i])
                      for i in range(n)], x_lo=x_lo)
         else:
-            x2 = _bf16c(x.reshape(-1, fin))
-            Wc = [_bf16c(w) for w in Ws]
+            x2 = _halfc(x.reshape(-1, fin), hdt)
+            Wc = [_halfc(w, hdt) for w in Ws]
             Wl = [None] * n
             ys, A_cat, t_cat = ops.group_fwd(
-                x2, [(Wc[i], _bf16c(As[i]), Bc[i], _bf16c(biases[i]), scales[i]) for i in range(n)])
+                x2, [(Wc[i], _halfc(As[i], hdt), Bc[i], _halfc(biases[i], hdt), scales[i]) for i in range(n)])
         ctx.has_w = [w is not None for w in Wc]
         ctx.save_for_backward(x2, A_cat, t_cat, *[w for w in Wc if w is not None], *[w for w in Wl if w is not None], *Bc)
         ctx.scales = tuple(float(s) for s in scales)
@@ -163,10 +178,11 @@ class _SoWGroupFn(torch.autograd.Function):
                 dyi = dyi if dyi.dtype == torch.float32 else dyi.float()
                 dy2, dy_lo = ops.split_f32(dyi if dyi.is_contiguous() else dyi.contiguous())
             else:
-                dy2, dy_lo = _bf16c(dyi), None
+                dy2, dy_lo = _halfc(dyi, ctx.hdt), None
             pa, pb = ctx.leaves[i]
-            dA_dst = (_grad_dst(pa) if a_dts[i] == torch.bfloat16 else True) if nA else None
-            dB_dst = (_grad_dst(pb) if b_dts[i] == torch.bfloat16 else True) if nB else None
+            gdt = torch.bfloat16 if ctx.f32 else ctx.hdt          # dtype the kernels write the factor gradients in
+            dA_dst = (_grad_dst(pa, gdt) if a_dts[i] == gdt else True) if nA else None
+            dB_dst = (_grad_dst(pb, gdt) if b_dts[i] == gdt else True) if nB else None
             members.append((Wc[i], Bc[i], dy2, ctx.scales[i], dA_dst, dB_dst, bool(nb) and bias_dts[i] is not None,
                             Wl[i], dy_lo if Wc[i] is not None else None))
         dx, dAs, dBs, dbs = ops.group_bwd(x2, A_cat, t_cat, members, bool(need_x), f32=ctx.f32)
@@ -178,9 +194,9 @@ class _SoWGroupFn(torch.autograd.Function):
         for i in range(n):
             dA, dB, db = dAs[i], dBs[i], dbs[i]
             grads += [None,
-                      None if dA is None else (dA if a_dts[i] == torch.bfloat16 else dA.to(a_dts[i])),
-                      None if dB is None else (dB if b_dts[i] == torch.bfloat16 else dB.to(b_dts[i])),
-                      None if db is None else (db if bias_dts[i] == torch.bfloat16 else db.to(bias_dts[i])),
+                      None if dA is None else (dA if a_dts[i] == dA.dtype else dA.to(a_dts[i])),
+                      None if dB is None else (dB if b_dts[i] == dB.dtype else dB.to(b_dts[i])),
+                      None if db is None else (db if bias_dts[i] == db.dtype else db.to(bias_dts[i])),
                       None]
         return tuple(grads)
 
@@ -273,6 +289,7 @@ class SharedInputGroup:
 
 def _forward_modules(mods: Sequence["SoWLinear"], x: torch.Tensor):
     params, scales = [], []
+    f16 = _native_f16(x.dtype, [m.acc_downweight if m.acc_downweight.numel() != 0 else None for m in mods])
     for m in mods:
         A_list, B_list = list(m.downscale_weights), list(m.upscale_weights)
         if len(A_list) == 1:
@@ -281,7 +298,7 @@ def _forward_modules(mods: Sequence["SoWLinear"], x: torch.Tensor):
             # sum_i (x.A_i).B_i == (x.[A_1|..|A_n]).[B_1;..;B_n]: one fused call; autograd splits the grads
             A = torch.cat(A_list, dim=1)
             B = torch.cat(B_list, dim=0)
-        W_c, W_lo = m._compute_weight()
+        W_c, W_lo = m._compute_weight(native_f16=f16)
         params += [W_c, A, B, m.bias, W_lo]
         scales.append(m.scale)
     return sow_linear_group(x, scales, params)
@@ -342,7 +359,7 @@ class SoWLinear(nn.Module):
             self.bias = nn.Parameter(torch.empty(out_features, **fk))
         else:
             self.register_parameter("bias", None)
-        self._w_shadow = None       # bf16 compute copy of a non-bf16 acc_downweight
+        self._w_shadow = None       # compute copy of acc_downweight: bf16x3 pieces of fp32, bf16 copy of a mixed-dtype W
         self._w_shadow_key = None
         self._group = None          # SharedInputGroup of the projections that read the same input (surgery.group_shared_inputs)
         self._group_index = -1
@@ -367,14 +384,15 @@ class SoWLinear(nn.Module):
             nn.init.zeros_(self.bias)
 
     # ---- forward (sow.py:107-126) ---------------------------------------------------------------------------
-    def _compute_weight(self):
-        """(W_c, W_lo): the operand(s) the kernels read for the frozen accumulation.  bf16 W: (W, None), no copy.  fp32 W:
-        its two bf16 pieces (W ~ W_c + W_lo, 2^-17 relative) for the bf16x3 path, cached until W changes (merge, load).
-        Other dtypes: one bf16 copy (bf16 compute policy)."""
+    def _compute_weight(self, native_f16: bool = False):
+        """(W_c, W_lo): the operand(s) the kernels read for the frozen accumulation.  bf16 W: (W, None), no copy.  fp16 W
+        of a call on the fp16 path (``native_f16``): (W, None), no copy.  fp32 W: its two bf16 pieces (W ~ W_c + W_lo,
+        2^-17 relative) for the bf16x3 path, cached until W changes (merge, load).  Other dtypes: one bf16 copy (bf16
+        compute policy)."""
         W = self.acc_downweight
         if W.numel() == 0:
             return None, None
-        if W.dtype == torch.bfloat16 and W.is_contiguous():
+        if W.is_contiguous() and (W.dtype == torch.bfloat16 or (native_f16 and W.dtype == torch.float16)):
             return W, None
         key = (W.data_ptr(), W._version, W.dtype)
         if self._w_shadow is None or self._w_shadow_key != key:
@@ -433,10 +451,10 @@ class SoWLinear(nn.Module):
 def _merge_dense(mods: List[SoWLinear]) -> None:
     """Dense branch (sow.py:151-153) for all modules: one grouped launch per dtype class (and per 64-wide rank chunk).
 
-    bf16 modules: tcgen05 kernel, W updated IN PLACE (pointer-stable).  fp32 modules: exact fp32 kernel, in place -- the
-    pretrained weights keep their full precision, as in the reference (sow.py:131-153 stays in the parameter dtype).
-    Anything else (mixed dtypes, other devices) goes through a bf16 compute copy and is cast back."""
-    items = {torch.bfloat16: [], torch.float32: []}
+    bf16 and fp16 modules: tcgen05 kernel in the module's dtype, W updated IN PLACE (pointer-stable).  fp32 modules: exact
+    fp32 kernel, in place -- the pretrained weights keep their full precision, as in the reference (sow.py:131-153 stays in
+    the parameter dtype).  Anything else (mixed dtypes, other devices) goes through a bf16 compute copy and is cast back."""
+    items = {torch.bfloat16: [], torch.float16: [], torch.float32: []}
     post = []
     for mod in mods:
         A_list = [a.detach() for a in mod.downscale_weights]

@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import SOWB_BF16, SOWB_F32, MergeEntry, SowB200Error, check
+from ._lib import SOWB_BF16, SOWB_F16, SOWB_F32, MergeEntry, SowB200Error, check
 
 # count of kernel-launching C-ABI calls, for bench.py's `gpu_launches` accounting (approximate kernels per call
 # are listed next to each call site)
@@ -46,7 +46,16 @@ def _dtype_code(dt: torch.dtype) -> int:
         return SOWB_BF16
     if dt == torch.float32:
         return SOWB_F32
+    if dt == torch.float16:
+        return SOWB_F16
     raise SowB200Error(f"unsupported dtype {dt}")
+
+
+def _tt_dtype_code(dt: torch.dtype) -> int:
+    """dtype code of the tensor-train entry points, which take bf16 and fp32 only."""
+    if dt not in (torch.bfloat16, torch.float32):
+        raise SowB200Error(f"unsupported dtype {dt}")
+    return _dtype_code(dt)
 
 
 def workspace(device: torch.device, nbytes: int, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
@@ -87,9 +96,12 @@ def group_rank_fits(ranks) -> bool:
 # SoW linear
 # ---------------------------------------------------------------------------------------------------------
 
-def _check_bf16c(name: str, t: Optional[torch.Tensor]):
-    if t is not None and (t.dtype != torch.bfloat16 or not t.is_contiguous()):
-        raise SowB200Error(f"{name} must be a contiguous bf16 tensor")
+_HALF_NAMES = {torch.bfloat16: "bf16", torch.float16: "fp16"}
+
+
+def _check_bf16c(name: str, t: Optional[torch.Tensor], dt: torch.dtype = torch.bfloat16):
+    if t is not None and (t.dtype != dt or not t.is_contiguous()):
+        raise SowB200Error(f"{name} must be a contiguous {_HALF_NAMES[dt]} tensor")
 
 
 def split_f32(t: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -106,16 +118,18 @@ def split_f32(t: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
 
 
 def group_fwd(x: torch.Tensor, members, x_lo: Optional[torch.Tensor] = None):
-    """Forward of a group of SoW projections that read the same x (T,in) bf16 contiguous (include/sow_b200.h:
-    sow_group_fwd).  members: (W (in,out) or None, A (in,r), B (r,out), bias or None, scale[, W_lo]).
+    """Forward of a group of SoW projections that read the same x (T,in) bf16 or fp16 contiguous (include/sow_b200.h:
+    sow_group_fwd).  members: (W (in,out) or None, A (in,r), B (r,out), bias or None, scale[, W_lo]), all of x's dtype.
     With ``x_lo`` (SOWB_F32 mode) x / x_lo and W / W_lo are the bf16 pieces of fp32 operands, bias is fp32 and the outputs
-    are fp32.  Returns ([y_i (T,out_i)], A_cat (in,R), t_cat (T,R)); A_cat / t_cat are what autograd saves for group_bwd."""
+    are fp32.  Returns ([y_i (T,out_i)], A_cat (in,R), t_cat (T,R)); A_cat / t_cat (x's dtype) are what autograd saves for
+    group_bwd."""
     lib = _lib.load()
     n = len(members)
     T, fin = x.shape
     f32 = x_lo is not None
+    hdt = torch.float16 if (x.dtype == torch.float16 and not f32) else torch.bfloat16
     _require_cuda(x, x_lo)
-    _check_bf16c("x", x)
+    _check_bf16c("x", x, hdt)
     _check_bf16c("x_lo", x_lo)
     arr = (_lib.GroupMember * n)()
     ys = []
@@ -126,27 +140,27 @@ def group_fwd(x: torch.Tensor, members, x_lo: Optional[torch.Tensor] = None):
         W_lo = mem[5] if len(mem) > 5 else None
         _require_cuda(W, A, B, bias, W_lo)
         for nm, t in (("W", W), ("A", A), ("B", B), ("W_lo", W_lo)):
-            _check_bf16c(nm, t)
+            _check_bf16c(nm, t, hdt)
         if f32:
             if bias is not None and (bias.dtype != torch.float32 or not bias.is_contiguous()):
                 raise SowB200Error("group_fwd: fp32 mode needs a contiguous fp32 bias")
             if (W is None) != (W_lo is None):
                 raise SowB200Error("group_fwd: fp32 mode needs both pieces of W")
         else:
-            _check_bf16c("bias", bias)
+            _check_bf16c("bias", bias, hdt)
         r, fout = B.shape
         if A.shape != (fin, r) or (W is not None and tuple(W.shape) != (fin, fout)):
             raise SowB200Error("group_fwd: shape mismatch")
-        y = torch.empty((T, fout), dtype=torch.float32 if f32 else torch.bfloat16, device=x.device)
+        y = torch.empty((T, fout), dtype=torch.float32 if f32 else hdt, device=x.device)
         ys.append(y)
         arr[i].W, arr[i].W_lo, arr[i].A, arr[i].B, arr[i].bias = _p(W), _p(W_lo), _p(A), _p(B), _p(bias)
         arr[i].y = _p(y)
         arr[i].out_features, arr[i].r, arr[i].scale = fout, r, float(scale)
         R += rank_pad(r)
         keep.append((W, W_lo, A, B, bias))
-    A_cat = torch.empty((fin, R), dtype=torch.bfloat16, device=x.device)
-    t_cat = torch.empty((T, R), dtype=torch.bfloat16, device=x.device)
-    rc = lib.sow_group_fwd(_p(x), _p(x_lo), arr, n, _p(A_cat), _p(t_cat), T, fin, SOWB_F32 if f32 else SOWB_BF16,
+    A_cat = torch.empty((fin, R), dtype=hdt, device=x.device)
+    t_cat = torch.empty((T, R), dtype=hdt, device=x.device)
+    rc = lib.sow_group_fwd(_p(x), _p(x_lo), arr, n, _p(A_cat), _p(t_cat), T, fin, SOWB_F32 if f32 else _dtype_code(hdt),
                            _stream_ptr(x.device))
     check(rc, "sow_group_fwd")
     launch_counter["kernels"] += 2 + n
@@ -156,13 +170,18 @@ def group_fwd(x: torch.Tensor, members, x_lo: Optional[torch.Tensor] = None):
 def group_bwd(x: torch.Tensor, A_cat: torch.Tensor, t_cat: torch.Tensor, members, need_dx: bool, f32: bool = False):
     """Backward of a group (sow_group_bwd).  members: (W or None, B (r,out), dy (T,out), scale, dA_dst, dB_dst,
     want_dbias[, W_lo, dy_lo]) where dA_dst / dB_dst are None (not needed), True (allocate) or a preallocated contiguous
-    bf16 tensor of the gradient's shape (e.g. a view into a flat gradient bucket) that the kernels write in place.
+    tensor of the gradient's shape and the 16-bit dtype (e.g. a view into a flat gradient bucket) that the kernels write in
+    place.  The 16-bit dtype is x's: bf16, or fp16 (every operand and gradient fp16).
     ``f32``: W / W_lo and dy / dy_lo are bf16 pieces of fp32 operands and dx is fp32.
     Returns (dx or None, [dA_i], [dB_i], [dbias_i])."""
     lib = _lib.load()
     n = len(members)
     T, fin = x.shape
     dev = x.device
+    hdt = torch.float16 if (x.dtype == torch.float16 and not f32) else torch.bfloat16
+    _check_bf16c("x", x, hdt)
+    _check_bf16c("A_cat", A_cat, hdt)
+    _check_bf16c("t_cat", t_cat, hdt)
     R = t_cat.shape[1]
     arr = (_lib.GroupMember * n)()
     dAs, dBs, dbs = [], [], []
@@ -173,7 +192,7 @@ def group_bwd(x: torch.Tensor, A_cat: torch.Tensor, t_cat: torch.Tensor, members
         dy_lo = mem[8] if len(mem) > 8 else None
         _require_cuda(W, B, dy, W_lo, dy_lo)
         for nm, t in (("W", W), ("B", B), ("dy", dy), ("W_lo", W_lo), ("dy_lo", dy_lo)):
-            _check_bf16c(nm, t)
+            _check_bf16c(nm, t, hdt)
         r, fout = B.shape
         if tuple(dy.shape) != (T, fout):
             raise SowB200Error("group_bwd: dy shape mismatch")
@@ -182,13 +201,14 @@ def group_bwd(x: torch.Tensor, A_cat: torch.Tensor, t_cat: torch.Tensor, members
             if dst is None:
                 return None
             if dst is True:
-                return torch.empty(shape, dtype=torch.bfloat16, device=dev)
-            if tuple(dst.shape) != tuple(shape) or dst.dtype != torch.bfloat16 or not dst.is_contiguous() or dst.device != dev:
-                raise SowB200Error("group_bwd: gradient destination must be a contiguous bf16 tensor of the gradient's shape")
+                return torch.empty(shape, dtype=hdt, device=dev)
+            if tuple(dst.shape) != tuple(shape) or dst.dtype != hdt or not dst.is_contiguous() or dst.device != dev:
+                raise SowB200Error(f"group_bwd: gradient destination must be a contiguous {_HALF_NAMES[hdt]} tensor of the "
+                                   "gradient's shape")
             return dst.detach()          # fresh alias of the same memory: AccumulateGrad can adopt it as param.grad
         dA = out_buf(dA_dst, (fin, r))
         dB = out_buf(dB_dst, (r, fout))
-        db = torch.empty((fout,), dtype=torch.bfloat16, device=dev) if want_dbias else None
+        db = torch.empty((fout,), dtype=hdt, device=dev) if want_dbias else None
         dAs.append(dA)
         dBs.append(dB)
         dbs.append(db)
@@ -197,11 +217,11 @@ def group_bwd(x: torch.Tensor, A_cat: torch.Tensor, t_cat: torch.Tensor, members
         arr[i].dA, arr[i].dB, arr[i].dbias = _p(dA), _p(dB), _p(db)
         arr[i].out_features, arr[i].r, arr[i].scale = fout, r, float(scale)
         keep.append((W, W_lo, B, dy, dy_lo))
-    dt_cat = torch.empty((T, R), dtype=torch.bfloat16, device=dev)
-    dx = torch.empty((T, fin), dtype=torch.float32 if f32 else torch.bfloat16, device=dev) if need_dx else None
+    dt_cat = torch.empty((T, R), dtype=hdt, device=dev)
+    dx = torch.empty((T, fin), dtype=torch.float32 if f32 else hdt, device=dev) if need_dx else None
     nws = lib.sow_group_workspace_bytes(_lib.OP_LINEAR_BWD, T, fin, arr, n)
     ws = workspace(dev, nws)
-    rc = lib.sow_group_bwd(_p(x), _p(A_cat), _p(t_cat), arr, n, _p(dt_cat), _p(dx), T, fin, SOWB_F32 if f32 else SOWB_BF16,
+    rc = lib.sow_group_bwd(_p(x), _p(A_cat), _p(t_cat), arr, n, _p(dt_cat), _p(dx), T, fin, SOWB_F32 if f32 else _dtype_code(hdt),
                            _p(ws), ws.numel(), _stream_ptr(dev))
     check(rc, "sow_group_bwd")
     # K2 (one launch when the members share a cluster size, else n) + split-K dA + finalize + dX + colsum pairs
@@ -230,14 +250,15 @@ def linear_bwd(dy, x, A_pad, t, W, B, scale: float, want_dbias: bool, need_dx: b
 
 def merge_grouped(items: Sequence[Tuple[torch.Tensor, Optional[torch.Tensor], torch.Tensor, torch.Tensor, float]]):
     """items: (W_out (in,out), W_prev or None, A (in,r), B (r,out), scale), all CUDA contiguous on one device and all
-    of ONE dtype: bf16 (tcgen05 path, one launch per 64-wide rank chunk for the whole list) or fp32 (exact fp32 path)."""
+    of ONE dtype: bf16 or fp16 (tcgen05 path, one launch per 64-wide rank chunk for the whole list) or fp32 (exact fp32
+    path)."""
     if not items:
         return
     lib = _lib.load()
     dev = items[0][0].device
     n = len(items)
     dt = items[0][0].dtype
-    if dt not in (torch.bfloat16, torch.float32):
+    if dt not in (torch.bfloat16, torch.float16, torch.float32):
         raise SowB200Error(f"merge_grouped: unsupported dtype {dt}")
     arr = (MergeEntry * n)()
     for i, (W, Wp, A, B, s) in enumerate(items):
@@ -319,7 +340,7 @@ def interleave(src: torch.Tensor, mm: int, nn: int, order: int) -> torch.Tensor:
     src = src.contiguous()
     M, N = src.shape
     out = torch.empty(((mm * nn) ** order,), dtype=torch.float32, device=src.device)
-    rc = lib.tt_interleave(_p(src), M, N, mm, nn, order, _p(out), _dtype_code(src.dtype), _stream_ptr(src.device))
+    rc = lib.tt_interleave(_p(src), M, N, mm, nn, order, _p(out), _tt_dtype_code(src.dtype), _stream_ptr(src.device))
     check(rc, "tt_interleave")
     launch_counter["kernels"] += 1
     return out
@@ -330,7 +351,7 @@ def deinterleave(src: torch.Tensor, M: int, N: int, mm: int, nn: int, order: int
     lib = _lib.load()
     src = src.contiguous()
     out = torch.empty((M, N), dtype=dtype, device=src.device)
-    rc = lib.tt_deinterleave(_p(src), M, N, mm, nn, order, _p(out), _dtype_code(dtype), _stream_ptr(src.device))
+    rc = lib.tt_deinterleave(_p(src), M, N, mm, nn, order, _p(out), _tt_dtype_code(dtype), _stream_ptr(src.device))
     check(rc, "tt_deinterleave")
     launch_counter["kernels"] += 1
     return out
@@ -344,7 +365,7 @@ def decompose2(src: torch.Tensor, mm: int, nn: int, r: int):
     src = src.contiguous()
     M, N = src.shape
     P = mm * nn
-    dt = _dtype_code(src.dtype)
+    dt = _tt_dtype_code(src.dtype)
     st = _stream_ptr(src.device)
     ncols = min(P, (r + 7) // 8 * 8)
     X = torch.empty((P, ncols), dtype=torch.float32, device=src.device)
@@ -367,7 +388,7 @@ def reconstruct2(G1: torch.Tensor, G2: torch.Tensor, M: int, N: int, mm: int, nn
     G2 = G2.contiguous()
     r = G1.shape[1]
     out = torch.empty((M, N), dtype=dtype, device=G1.device)
-    check(lib.tt_reconstruct2(_p(G1), _p(G2), r, _p(out), M, N, mm, nn, _dtype_code(dtype), _stream_ptr(G1.device)),
+    check(lib.tt_reconstruct2(_p(G1), _p(G2), r, _p(out), M, N, mm, nn, _tt_dtype_code(dtype), _stream_ptr(G1.device)),
           "tt_reconstruct2")
     launch_counter["kernels"] += 1
     return out
@@ -406,7 +427,7 @@ def tt_adam_fused2(p, g, cores_m, cores_v, mm, nn, beta1, beta2, eps, step_size,
     g = g.contiguous()
     rc = lib.tt_adam_fused2(_p(p), _p(g), _p(G1m), _p(G2m), _p(G1v), _p(G2v), r, _p(m_out), _p(v_out), M, N, mm, nn,
                             float(beta1), float(beta2), float(eps), float(step_size), float(lr_wd),
-                            1 if first_step else 0, _dtype_code(p.dtype), _stream_ptr(p.device))
+                            1 if first_step else 0, _tt_dtype_code(p.dtype), _stream_ptr(p.device))
     check(rc, "tt_adam_fused2")
     launch_counter["kernels"] += 1
     return m_out, v_out
@@ -432,7 +453,7 @@ def tt_adam2_step(p, g, cores_m, cores_v, mm, nn, r, beta1, beta2, eps, step_siz
     ws = workspace(dev, lib.tt_adam2_workspace_bytes(mm, nn))
     rc = lib.tt_adam2_step(_p(p), _p(g), _p(G1m), _p(G2m), _p(G1v), _p(G2v), r, _p(Q[0]), _p(Q[1]), _p(R[0]), _p(R[1]),
                            M, N, mm, nn, float(beta1), float(beta2), float(eps), float(step_size), float(lr_wd),
-                           1 if first_step else 0, _dtype_code(p.dtype), _p(ws), ws.numel(), _stream_ptr(dev))
+                           1 if first_step else 0, _tt_dtype_code(p.dtype), _p(ws), ws.numel(), _stream_ptr(dev))
     check(rc, "tt_adam2_step")
     launch_counter["kernels"] += 8
     return (Q[0], R[0]), (Q[1], R[1])
@@ -475,7 +496,7 @@ class TTAdam2Plan:
         sp = ctypes.c_void_p(stream.cuda_stream) if stream is not None else _stream_ptr(self.device)
         rc = lib.tt_adam2_step(_p(p), _p(g), g1m, g2m, g1v, g2v, self.r, qm, qv, rm, rv, M, N, self.mm, self.nn,
                                float(beta1), float(beta2), float(eps), float(step_size), float(lr_wd), 1 if first else 0,
-                               _dtype_code(p.dtype), _p(ws), ws.numel(), sp)
+                               _tt_dtype_code(p.dtype), _p(ws), ws.numel(), sp)
         check(rc, "tt_adam2_step")
         launch_counter["kernels"] += 8
         self.cur = out
@@ -499,7 +520,7 @@ def decompose_nd(src: torch.Tensor, mm: int, nn: int, ranks):
     cores = [torch.empty((ranks[k], mm, nn, ranks[k + 1]), dtype=torch.float32, device=src.device) for k in range(order)]
     tab = (ctypes.c_void_p * order)(*[c.data_ptr() for c in cores])
     ws = workspace(src.device, ws_bytes)
-    rc = lib.tt_decompose_nd(_p(src), tab, ranks_c, M, N, mm, nn, order, _dtype_code(src.dtype), _p(ws), ws.numel(),
+    rc = lib.tt_decompose_nd(_p(src), tab, ranks_c, M, N, mm, nn, order, _tt_dtype_code(src.dtype), _p(ws), ws.numel(),
                              _stream_ptr(src.device))
     check(rc, "tt_decompose_nd")
     launch_counter["kernels"] += 1 + 5 * (order - 1)
@@ -521,7 +542,7 @@ def reconstruct_nd(cores, M: int, N: int, mm: int, nn: int, dtype=torch.float32)
     out = torch.empty((M, N), dtype=dtype, device=dev)
     tab = (ctypes.c_void_p * order)(*[c.data_ptr() for c in cs])
     ws = workspace(dev, ws_bytes)
-    rc = lib.tt_reconstruct_nd(tab, ranks_c, _p(out), M, N, mm, nn, order, _dtype_code(dtype), _p(ws), ws.numel(), _stream_ptr(dev))
+    rc = lib.tt_reconstruct_nd(tab, ranks_c, _p(out), M, N, mm, nn, order, _tt_dtype_code(dtype), _p(ws), ws.numel(), _stream_ptr(dev))
     check(rc, "tt_reconstruct_nd")
     launch_counter["kernels"] += order
     return out
@@ -563,7 +584,7 @@ class TTAdamNPlan:
         sp = ctypes.c_void_p(stream.cuda_stream) if stream is not None else _stream_ptr(self.device)
         rc = lib.tt_adam_nd_step(_p(p), _p(g), None if first else self._tab[self.cur], self._tab[out], self._ranks_c, M, N,
                                self.mm, self.nn, self.order, float(beta1), float(beta2), float(eps), float(step_size),
-                               float(lr_wd), 1 if first else 0, _dtype_code(p.dtype), _p(ws), ws.numel(), sp)
+                               float(lr_wd), 1 if first else 0, _tt_dtype_code(p.dtype), _p(ws), ws.numel(), sp)
         check(rc, "tt_adam_nd_step")
         launch_counter["kernels"] += 2 * (self.order - 1) + 1 + 8 * (self.order - 1)
         self.cur = out
@@ -577,7 +598,7 @@ def tt_adam_interleaved(p, g, m, v, mm, nn, order, beta1, beta2, eps, step_size,
     g = g.contiguous()
     M, N = p.shape
     rc = lib.tt_adam_interleaved(_p(p), _p(g), _p(m), _p(v), M, N, mm, nn, order, float(beta1), float(beta2), float(eps),
-                                 float(step_size), float(lr_wd), _dtype_code(p.dtype), _stream_ptr(p.device))
+                                 float(step_size), float(lr_wd), _tt_dtype_code(p.dtype), _stream_ptr(p.device))
     check(rc, "tt_adam_interleaved")
     launch_counter["kernels"] += 1
 
@@ -587,7 +608,7 @@ def tt_adam_dense(p, g, m, v, beta1, beta2, eps, step_size, lr_wd):
     lib = _lib.load()
     g = g.contiguous()
     rc = lib.tt_adam_dense(_p(p), _p(g), _p(m), _p(v), p.numel(), float(beta1), float(beta2), float(eps),
-                           float(step_size), float(lr_wd), _dtype_code(p.dtype), _stream_ptr(p.device))
+                           float(step_size), float(lr_wd), _tt_dtype_code(p.dtype), _stream_ptr(p.device))
     check(rc, "tt_adam_dense")
     launch_counter["kernels"] += 1
 
