@@ -313,6 +313,34 @@ int sow_adam_multi_ex(const void* chunks_dev, int n_chunks, int64_t total_elems,
 int sow_adam_multi_dev(const void* chunks_dev, int n_chunks, int64_t total_elems, double lr, double beta1, double beta2,
                        double eps, double weight_decay, float* step_dev, int decoupled, int dtype, void* stream);
 
+/*
+ * Element-wise glue of the Llama block (HF transformers modeling_llama.py), bit-identical to the eager chains it replaces.
+ * dtype SOWB_BF16 or SOWB_F16; math in fp32, each result rounded to the 16-bit type where eager rounds (see glue.cu).
+ * Pointers 16-byte aligned.  One launch per call.
+ *
+ * Rotary embedding of q and k (apply_rotary_pos_emb):  out = q * cos + rotate_half(q) * sin, the same for k.
+ *   q: (B, Hq, S, D) with element strides q_sb, q_sh, q_ss and a contiguous last dimension; k: (B, Hk, S, D) likewise.
+ *   cos, sin: (B or 1, S, D) contiguous; cs_sb is their batch stride (0 when shared by the batch).
+ *   q_out, k_out: (B, S, H, D) contiguous -- the layout of eager's q_embed seen through its (B, H, S, D) transpose.
+ *   D a multiple of 16, strides multiples of 8.
+ * sow_rope_bwd: dq, dk of the same layout from the upstream gradients gq, gk (strided like q, k); cos / sin as above.
+ */
+int sow_rope_fwd(const void* q, const void* k, const void* cos, const void* sin, void* q_out, void* k_out, int B, int S, int Hq,
+                 int Hk, int D, int64_t q_sb, int64_t q_sh, int64_t q_ss, int64_t k_sb, int64_t k_sh, int64_t k_ss,
+                 int64_t cs_sb, int dtype, void* stream);
+int sow_rope_bwd(const void* gq, const void* gk, const void* cos, const void* sin, void* dq, void* dk, int B, int S, int Hq,
+                 int Hk, int D, int64_t gq_sb, int64_t gq_sh, int64_t gq_ss, int64_t gk_sb, int64_t gk_sh, int64_t gk_ss,
+                 int64_t cs_sb, int dtype, void* stream);
+
+/*
+ * SwiGLU gate of LlamaMLP (act_fn = silu) over n contiguous elements:
+ *   sow_swiglu_fwd: h = silu(gate) * up
+ *   sow_swiglu_bwd: dup = dh * silu(gate),  dgate = silu_backward(dh * up, gate)   (one pass over dh, gate, up)
+ */
+int sow_swiglu_fwd(const void* gate, const void* up, void* h, int64_t n, int dtype, void* stream);
+int sow_swiglu_bwd(const void* dh, const void* gate, const void* up, void* dgate, void* dup, int64_t n, int dtype,
+                   void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1,0 +1,317 @@
+// Element-wise glue of the Llama block: rotary position embedding (q and k) and the SwiGLU gate, forward and backward.
+//
+// Replaces the eager HF chains of transformers/models/llama/modeling_llama.py:
+//     q_embed = (q * cos) + (rotate_half(q) * sin)          (apply_rotary_pos_emb, and the same for k)
+//     h = act_fn(gate_proj(x)) * up_proj(x)                 (LlamaMLP.forward, act_fn = silu)
+// which run as ~12 separate kernels per layer on strided views (mul, neg, cat, add, the zero-filled slice-backward
+// buffers and their copies).  Here each element is read once and written once per pass.
+//
+// The results are bit-identical to the eager chains.  Every rounding eager performs is reproduced in the same place:
+// products and sums are formed in fp32 and rounded to the 16-bit type (round to nearest even) exactly where eager writes
+// a 16-bit tensor.  r() below means that rounding.
+//   rope forward   out[d] = r(r(q[d] cos[d]) + r(-q[d+h] sin[d]))   d <  h = D/2
+//                  out[d] = r(r(q[d] cos[d]) + r( q[d-h] sin[d]))   d >= h
+//   rope backward  a = r(g cos), b = r(g sin)
+//                  dq[d] = r(a[d] + b[d+h]) + 0   d <  h
+//                  dq[d] = r(a[d] - b[d-h]) + 0   d >= h
+//                  (autograd sums the two slice-backward buffers, which are zero outside their half, into the gradient:
+//                  the "+ 0" is that sum, and it turns a -0 into +0)
+//   swiglu forward h = r(r(silu(g)) u),  silu(x) = x / (1 + expf(-x))                 (torch's silu_kernel)
+//   swiglu bwd     du = r(dh r(silu(g))),  dg = r(silu_backward(r(dh u), g))
+//                  silu_backward(dy, x) = dy s (1 + x (1 - s)), s = 1 / (1 + expf(-x))  (torch's silu_backward_kernel)
+// The build does not use --use_fast_math: expf, the divisions and the fp32 products are the IEEE / libdevice ones torch
+// uses.  The one place where FMA contraction decides the bits, 1 + x (1 - s), is pinned to the fused form nvcc emits
+// for torch's expression.
+#include "common.cuh"
+
+#include <cuda_fp16.h>
+
+namespace sowb {
+
+namespace {
+
+template <typename H>
+struct Cvt;
+template <>
+struct Cvt<__nv_bfloat16> {
+  using H2 = __nv_bfloat162;
+  static __device__ __forceinline__ float2 to_f2(H2 v) { return __bfloat1622float2(v); }
+  static __device__ __forceinline__ H2 from_f2(float a, float b) { return __floats2bfloat162_rn(a, b); }
+  static __device__ __forceinline__ float to_f(__nv_bfloat16 v) { return __bfloat162float(v); }
+  static __device__ __forceinline__ __nv_bfloat16 from_f(float v) { return __float2bfloat16_rn(v); }
+};
+template <>
+struct Cvt<__half> {
+  using H2 = __half2;
+  static __device__ __forceinline__ float2 to_f2(H2 v) { return __half22float2(v); }
+  static __device__ __forceinline__ H2 from_f2(float a, float b) { return __floats2half2_rn(a, b); }
+  static __device__ __forceinline__ float to_f(__half v) { return __half2float(v); }
+  static __device__ __forceinline__ __half from_f(float v) { return __float2half_rn(v); }
+};
+
+// r(v): round an fp32 value to the 16-bit type and back
+template <typename H>
+__device__ __forceinline__ float rnd(float v) {
+  return Cvt<H>::to_f(Cvt<H>::from_f(v));
+}
+
+// 8 consecutive 16-bit elements <-> 8 floats (one 16-byte access)
+template <typename H>
+__device__ __forceinline__ void load8(const H* p, float (&f)[8]) {
+  const uint4 v = *reinterpret_cast<const uint4*>(p);
+  const typename Cvt<H>::H2* h2 = reinterpret_cast<const typename Cvt<H>::H2*>(&v);
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float2 t = Cvt<H>::to_f2(h2[j]);
+    f[2 * j] = t.x;
+    f[2 * j + 1] = t.y;
+  }
+}
+template <typename H>
+__device__ __forceinline__ void store8(H* p, const float (&f)[8]) {
+  uint4 v;
+  typename Cvt<H>::H2* h2 = reinterpret_cast<typename Cvt<H>::H2*>(&v);
+#pragma unroll
+  for (int j = 0; j < 4; ++j) h2[j] = Cvt<H>::from_f2(f[2 * j], f[2 * j + 1]);
+  *reinterpret_cast<uint4*>(p) = v;
+}
+
+// One rotary call covers q and k of a layer.  Source (B, H, S, D) with element strides sb / sh / ss and a contiguous last
+// dimension; destination (B, S, H, D) contiguous.  cos / sin: (B or 1, S, D) contiguous, batch stride cs_sb (0 when
+// broadcast).  One thread owns the 8-element chunk c of the first half of a row and the matching chunk of the second half.
+struct RopeSide {
+  const void* src;
+  void* dst;
+  int64_t sb, sh, ss;
+  int heads;
+  int64_t n;   // B * S * heads * (D / 16) threads
+};
+struct RopeArgs {
+  RopeSide t[2];
+  const void* cos;
+  const void* sin;
+  int64_t cs_sb;
+  int S, D;
+};
+
+template <typename H, bool kBackward>
+__global__ void __launch_bounds__(256) rope_kernel(const RopeArgs a) {
+  int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  int side = 0;
+  if (i >= a.t[0].n) {
+    i -= a.t[0].n;
+    side = 1;
+    if (i >= a.t[1].n) return;
+  }
+  const RopeSide& t = a.t[side];
+  const int half = a.D >> 1;
+  const int chunks = half >> 3;
+  const int c = int(i % chunks);
+  int64_t r = i / chunks;
+  const int hh = int(r % t.heads);
+  r /= t.heads;
+  const int s = int(r % a.S);
+  const int64_t b = r / a.S;
+
+  const H* src = static_cast<const H*>(t.src) + b * t.sb + hh * t.sh + s * t.ss + c * 8;
+  H* dst = static_cast<H*>(t.dst) + ((b * a.S + s) * t.heads + hh) * a.D + c * 8;
+  const int64_t co = b * a.cs_sb + int64_t(s) * a.D + c * 8;
+  const H* cs = static_cast<const H*>(a.cos) + co;
+  const H* sn = static_cast<const H*>(a.sin) + co;
+
+  float x1[8], x2[8], c1[8], c2[8], s1[8], s2[8], o1[8], o2[8];
+  load8<H>(src, x1);
+  load8<H>(src + half, x2);
+  load8<H>(cs, c1);
+  load8<H>(cs + half, c2);
+  load8<H>(sn, s1);
+  load8<H>(sn + half, s2);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    if (!kBackward) {
+      o1[j] = rnd<H>(x1[j] * c1[j]) + rnd<H>(-x2[j] * s1[j]);
+      o2[j] = rnd<H>(x2[j] * c2[j]) + rnd<H>(x1[j] * s2[j]);
+    } else {
+      // x = upstream gradient g
+      const float a1 = rnd<H>(x1[j] * c1[j]), a2 = rnd<H>(x2[j] * c2[j]);
+      const float b1 = rnd<H>(x1[j] * s1[j]), b2 = rnd<H>(x2[j] * s2[j]);
+      o1[j] = (a1 + b2) + 0.0f;
+      o2[j] = (a2 - b1) + 0.0f;
+    }
+  }
+  store8<H>(dst, o1);
+  store8<H>(dst + half, o2);
+}
+
+// torch's silu / silu_backward in fp32 (ActivationSiluKernel.cu)
+__device__ __forceinline__ float silu_f(float x) { return x / (1.0f + expf(-x)); }
+__device__ __forceinline__ float silu_bwd_f(float dy, float x) {
+  const float s = 1.0f / (1.0f + expf(-x));
+  return __fmul_rn(__fmul_rn(dy, s), __fmaf_rn(x, 1.0f - s, 1.0f));
+}
+
+template <typename H>
+__device__ __forceinline__ void swiglu_fwd_elem(float g, float u, float& h) {
+  h = rnd<H>(silu_f(g)) * u;
+}
+template <typename H>
+__device__ __forceinline__ void swiglu_bwd_elem(float dh, float g, float u, float& dg, float& du) {
+  du = dh * rnd<H>(silu_f(g));
+  dg = silu_bwd_f(rnd<H>(dh * u), g);
+}
+
+// n elements, contiguous; 8 per thread with 16-byte accesses, the last n % 8 by the first threads one by one
+template <typename H>
+__global__ void __launch_bounds__(256) swiglu_fwd_kernel(const H* __restrict__ gate, const H* __restrict__ up,
+                                                         H* __restrict__ h, int64_t n) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  const int64_t nvec = n >> 3;
+  if (i < nvec) {
+    float g[8], u[8], o[8];
+    load8<H>(gate + i * 8, g);
+    load8<H>(up + i * 8, u);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) swiglu_fwd_elem<H>(g[j], u[j], o[j]);
+    store8<H>(h + i * 8, o);
+  } else if (i - nvec < (n & 7)) {
+    const int64_t e = nvec * 8 + (i - nvec);
+    float o;
+    swiglu_fwd_elem<H>(Cvt<H>::to_f(gate[e]), Cvt<H>::to_f(up[e]), o);
+    h[e] = Cvt<H>::from_f(o);
+  }
+}
+
+template <typename H>
+__global__ void __launch_bounds__(256) swiglu_bwd_kernel(const H* __restrict__ dh, const H* __restrict__ gate,
+                                                         const H* __restrict__ up, H* __restrict__ dgate,
+                                                         H* __restrict__ dup, int64_t n) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  const int64_t nvec = n >> 3;
+  if (i < nvec) {
+    float d[8], g[8], u[8], og[8], ou[8];
+    load8<H>(dh + i * 8, d);
+    load8<H>(gate + i * 8, g);
+    load8<H>(up + i * 8, u);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) swiglu_bwd_elem<H>(d[j], g[j], u[j], og[j], ou[j]);
+    store8<H>(dgate + i * 8, og);
+    store8<H>(dup + i * 8, ou);
+  } else if (i - nvec < (n & 7)) {
+    const int64_t e = nvec * 8 + (i - nvec);
+    float og, ou;
+    swiglu_bwd_elem<H>(Cvt<H>::to_f(dh[e]), Cvt<H>::to_f(gate[e]), Cvt<H>::to_f(up[e]), og, ou);
+    dgate[e] = Cvt<H>::from_f(og);
+    dup[e] = Cvt<H>::from_f(ou);
+  }
+}
+
+inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+int rope_launch(const char* fn, bool backward, const void* q, const void* k, const void* cos, const void* sin, void* q_out,
+                void* k_out, int B, int S, int Hq, int Hk, int D, int64_t q_sb, int64_t q_sh, int64_t q_ss, int64_t k_sb,
+                int64_t k_sh, int64_t k_ss, int64_t cs_sb, int dtype, void* stream_) {
+  SOWB_REQUIRE(dtype == SOWB_BF16 || dtype == SOWB_F16, "%s: dtype %d unsupported (bf16 / fp16)", fn, dtype);
+  SOWB_REQUIRE(q && k && cos && sin && q_out && k_out, "%s: null pointer", fn);
+  SOWB_REQUIRE(aligned16(q) && aligned16(k) && aligned16(cos) && aligned16(sin) && aligned16(q_out) && aligned16(k_out),
+               "%s: pointers must be 16-byte aligned", fn);
+  SOWB_REQUIRE(B >= 0 && S >= 0 && Hq >= 0 && Hk >= 0, "%s: negative size", fn);
+  SOWB_REQUIRE(D > 0 && D % 16 == 0, "%s: head dim %d must be a positive multiple of 16", fn, D);
+  SOWB_REQUIRE(q_sb % 8 == 0 && q_sh % 8 == 0 && q_ss % 8 == 0 && k_sb % 8 == 0 && k_sh % 8 == 0 && k_ss % 8 == 0 &&
+                   cs_sb % 8 == 0 && q_sb >= 0 && q_sh >= 0 && q_ss >= 0 && k_sb >= 0 && k_sh >= 0 && k_ss >= 0 && cs_sb >= 0,
+               "%s: strides must be non-negative multiples of 8 elements", fn);
+  RopeArgs a;
+  a.t[0] = {q, q_out, q_sb, q_sh, q_ss, Hq, int64_t(B) * S * Hq * (D / 16)};
+  a.t[1] = {k, k_out, k_sb, k_sh, k_ss, Hk, int64_t(B) * S * Hk * (D / 16)};
+  a.cos = cos;
+  a.sin = sin;
+  a.cs_sb = cs_sb;
+  a.S = S;
+  a.D = D;
+  const int64_t total = a.t[0].n + a.t[1].n;
+  if (total == 0) return SOWB_OK;
+  const int64_t blocks = (total + 255) / 256;
+  SOWB_REQUIRE(blocks < (int64_t(1) << 31), "%s: tensors too large", fn);
+  if (int rc = ensure_context_for(q)) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (dtype == SOWB_BF16) {
+    if (backward) rope_kernel<__nv_bfloat16, true><<<unsigned(blocks), 256, 0, stream>>>(a);
+    else rope_kernel<__nv_bfloat16, false><<<unsigned(blocks), 256, 0, stream>>>(a);
+  } else {
+    if (backward) rope_kernel<__half, true><<<unsigned(blocks), 256, 0, stream>>>(a);
+    else rope_kernel<__half, false><<<unsigned(blocks), 256, 0, stream>>>(a);
+  }
+  SOWB_CHECK_CUDA(cudaGetLastError());
+  return SOWB_OK;
+}
+
+int swiglu_check(const char* fn, int64_t n, int dtype) {
+  SOWB_REQUIRE(dtype == SOWB_BF16 || dtype == SOWB_F16, "%s: dtype %d unsupported (bf16 / fp16)", fn, dtype);
+  SOWB_REQUIRE(n >= 0, "%s: negative element count", fn);
+  SOWB_REQUIRE((n / 8 + 256) / 256 < (int64_t(1) << 31), "%s: tensors too large", fn);
+  return SOWB_OK;
+}
+
+}  // namespace
+
+}  // namespace sowb
+
+using namespace sowb;
+
+extern "C" {
+
+int sow_rope_fwd(const void* q, const void* k, const void* cos, const void* sin, void* q_out, void* k_out, int B, int S, int Hq,
+                 int Hk, int D, int64_t q_sb, int64_t q_sh, int64_t q_ss, int64_t k_sb, int64_t k_sh, int64_t k_ss,
+                 int64_t cs_sb, int dtype, void* stream) {
+  return rope_launch("sow_rope_fwd", false, q, k, cos, sin, q_out, k_out, B, S, Hq, Hk, D, q_sb, q_sh, q_ss, k_sb, k_sh, k_ss,
+                     cs_sb, dtype, stream);
+}
+
+int sow_rope_bwd(const void* gq, const void* gk, const void* cos, const void* sin, void* dq, void* dk, int B, int S, int Hq,
+                 int Hk, int D, int64_t gq_sb, int64_t gq_sh, int64_t gq_ss, int64_t gk_sb, int64_t gk_sh, int64_t gk_ss,
+                 int64_t cs_sb, int dtype, void* stream) {
+  return rope_launch("sow_rope_bwd", true, gq, gk, cos, sin, dq, dk, B, S, Hq, Hk, D, gq_sb, gq_sh, gq_ss, gk_sb, gk_sh, gk_ss,
+                     cs_sb, dtype, stream);
+}
+
+int sow_swiglu_fwd(const void* gate, const void* up, void* h, int64_t n, int dtype, void* stream_) {
+  if (int rc = swiglu_check("sow_swiglu_fwd", n, dtype)) return rc;
+  SOWB_REQUIRE(gate && up && h, "sow_swiglu_fwd: null pointer");
+  SOWB_REQUIRE(aligned16(gate) && aligned16(up) && aligned16(h), "sow_swiglu_fwd: pointers must be 16-byte aligned");
+  if (n == 0) return SOWB_OK;
+  if (int rc = ensure_context_for(gate)) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const unsigned blocks = unsigned((n / 8 + (n % 8) + 255) / 256);
+  if (dtype == SOWB_BF16)
+    swiglu_fwd_kernel<__nv_bfloat16><<<blocks, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(gate),
+                                                                  static_cast<const __nv_bfloat16*>(up),
+                                                                  static_cast<__nv_bfloat16*>(h), n);
+  else
+    swiglu_fwd_kernel<__half><<<blocks, 256, 0, stream>>>(static_cast<const __half*>(gate), static_cast<const __half*>(up),
+                                                          static_cast<__half*>(h), n);
+  SOWB_CHECK_CUDA(cudaGetLastError());
+  return SOWB_OK;
+}
+
+int sow_swiglu_bwd(const void* dh, const void* gate, const void* up, void* dgate, void* dup, int64_t n, int dtype,
+                   void* stream_) {
+  if (int rc = swiglu_check("sow_swiglu_bwd", n, dtype)) return rc;
+  SOWB_REQUIRE(dh && gate && up && dgate && dup, "sow_swiglu_bwd: null pointer");
+  SOWB_REQUIRE(aligned16(dh) && aligned16(gate) && aligned16(up) && aligned16(dgate) && aligned16(dup),
+               "sow_swiglu_bwd: pointers must be 16-byte aligned");
+  if (n == 0) return SOWB_OK;
+  if (int rc = ensure_context_for(gate)) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const unsigned blocks = unsigned((n / 8 + (n % 8) + 255) / 256);
+  if (dtype == SOWB_BF16)
+    swiglu_bwd_kernel<__nv_bfloat16><<<blocks, 256, 0, stream>>>(
+        static_cast<const __nv_bfloat16*>(dh), static_cast<const __nv_bfloat16*>(gate), static_cast<const __nv_bfloat16*>(up),
+        static_cast<__nv_bfloat16*>(dgate), static_cast<__nv_bfloat16*>(dup), n);
+  else
+    swiglu_bwd_kernel<__half><<<blocks, 256, 0, stream>>>(static_cast<const __half*>(dh), static_cast<const __half*>(gate),
+                                                          static_cast<const __half*>(up), static_cast<__half*>(dgate),
+                                                          static_cast<__half*>(dup), n);
+  SOWB_CHECK_CUDA(cudaGetLastError());
+  return SOWB_OK;
+}
+
+}  // extern "C"

@@ -1,0 +1,150 @@
+"""Native rotary embedding and SwiGLU for HF Llama blocks on the eager training path.
+
+Eager HF code runs ``q * cos + rotate_half(q) * sin`` (for q and k) and ``act_fn(gate) * up`` as about a dozen element-wise
+kernels per layer on strided views, with zero-filled slice-backward buffers in the backward pass.  The kernels of
+``csrc/glue.cu`` do each chain in one pass per direction and reproduce eager's rounding sequence exactly, so the results
+are bit-identical to the stock functions (and a training run is unchanged bit for bit).
+
+``install_llama_glue(model)`` (called by ``prepare_sow``) routes a model's Llama blocks through them:
+  * SwiGLU: every ``LlamaMLP`` with a silu activation gets a per-instance ``forward`` that calls ``gate_proj(x)`` then
+    ``up_proj(x)`` (the order eager uses, which the shared-input SoW group relies on) and the fused gate.
+  * RoPE: HF's attention looks ``apply_rotary_pos_emb`` up in the ``modeling_llama`` module globals; that global is
+    replaced by a dispatcher that keeps the stock function.  Installing twice changes nothing.
+The native path runs only for CUDA bf16 / fp16 tensors of the expected layouts, cos / sin without grad,
+``unsqueeze_dim == 1``, and outside ``torch.compile`` tracing; every other call runs the stock function, so compiled
+models (inductor fuses these chains itself) and fp32 models are exactly as before.
+"""
+from __future__ import annotations
+
+import types
+
+import torch
+import torch.nn as nn
+
+from . import ops
+
+_HALF = (torch.bfloat16, torch.float16)
+
+
+# ---- rotary embedding ----------------------------------------------------------------------------------------------
+
+class _RoPE(torch.autograd.Function):
+    """(q, k, cos, sin) -> (q * cos + rotate_half(q) * sin, the same for k).  Saves only cos / sin, as eager does."""
+
+    @staticmethod
+    def forward(ctx, q, k, cos, sin):
+        ctx.save_for_backward(cos, sin)
+        return ops.rope_fwd(q, k, cos, sin)
+
+    @staticmethod
+    def backward(ctx, gq, gk):
+        cos, sin = ctx.saved_tensors
+        dq, dk = ops.rope_bwd(gq, gk, cos, sin)
+        return dq, dk, None, None
+
+
+def _aligned_rows(t: torch.Tensor) -> bool:
+    return t.stride(-1) == 1 and t.data_ptr() % 16 == 0 and all(s % 8 == 0 for s in t.stride()[:-1])
+
+
+def rope_native_ok(q, k, cos, sin, unsqueeze_dim=1) -> bool:
+    """True when the native kernel computes apply_rotary_pos_emb(q, k, cos, sin, unsqueeze_dim) for these arguments."""
+    if unsqueeze_dim != 1 or not all(isinstance(t, torch.Tensor) for t in (q, k, cos, sin)):
+        return False
+    if not q.is_cuda or q.dtype not in _HALF or not (k.dtype == cos.dtype == sin.dtype == q.dtype):
+        return False
+    if not (k.device == cos.device == sin.device == q.device) or cos.requires_grad or sin.requires_grad:
+        return False
+    if q.dim() != 4 or k.dim() != 4 or cos.dim() != 3:
+        return False
+    B, _, S, D = q.shape
+    if D % 16 or k.shape[0] != B or tuple(k.shape[2:]) != (S, D):
+        return False
+    if cos.shape != sin.shape or tuple(cos.shape) not in ((1, S, D), (B, S, D)):
+        return False
+    if not (cos.is_contiguous() and sin.is_contiguous() and cos.data_ptr() % 16 == 0 and sin.data_ptr() % 16 == 0):
+        return False
+    return _aligned_rows(q) and _aligned_rows(k)
+
+
+def make_rope_dispatcher(stock):
+    """apply_rotary_pos_emb with HF's signature: the native kernel where rope_native_ok holds, ``stock`` otherwise."""
+
+    def apply_rotary_pos_emb(q, k, cos, sin, unsqueeze_dim=1):
+        if not torch.compiler.is_compiling() and rope_native_ok(q, k, cos, sin, unsqueeze_dim):
+            return _RoPE.apply(q, k, cos, sin)
+        return stock(q, k, cos, sin, unsqueeze_dim)
+
+    apply_rotary_pos_emb.__doc__ = getattr(stock, "__doc__", None)
+    apply_rotary_pos_emb.stock = stock
+    return apply_rotary_pos_emb
+
+
+def install_rope(modeling_module) -> bool:
+    """Replace ``modeling_module.apply_rotary_pos_emb`` by the dispatcher (once).  Returns True if it was installed now."""
+    cur = modeling_module.apply_rotary_pos_emb
+    if getattr(cur, "stock", None) is not None:
+        return False
+    modeling_module.apply_rotary_pos_emb = make_rope_dispatcher(cur)
+    return True
+
+
+# ---- SwiGLU ----------------------------------------------------------------------------------------------------------
+
+class _SwiGLU(torch.autograd.Function):
+    """(gate, up) -> silu(gate) * up.  Saves gate and up; eager also keeps silu(gate), one more activation per layer."""
+
+    @staticmethod
+    def forward(ctx, gate, up):
+        ctx.save_for_backward(gate, up)
+        return ops.swiglu_fwd(gate, up)
+
+    @staticmethod
+    def backward(ctx, dh):
+        gate, up = ctx.saved_tensors
+        return ops.swiglu_bwd(dh, gate, up)
+
+
+def swiglu_native_ok(gate, up) -> bool:
+    return (isinstance(gate, torch.Tensor) and isinstance(up, torch.Tensor) and gate.is_cuda and gate.dtype in _HALF
+            and up.dtype == gate.dtype and up.device == gate.device and gate.shape == up.shape
+            and gate.is_contiguous() and up.is_contiguous() and gate.data_ptr() % 16 == 0 and up.data_ptr() % 16 == 0)
+
+
+def _is_silu(act) -> bool:
+    try:
+        from transformers.activations import SiLUActivation
+    except Exception:  # pragma: no cover - older transformers
+        SiLUActivation = ()
+    return isinstance(act, SiLUActivation) or (isinstance(act, nn.SiLU) and not act.inplace)
+
+
+def _llama_mlp_forward(self, x):
+    """LlamaMLP.forward with the silu gate fused: down_proj(silu(gate_proj(x)) * up_proj(x))."""
+    if torch.compiler.is_compiling():
+        return type(self).forward(self, x)
+    gate = self.gate_proj(x)
+    up = self.up_proj(x)
+    h = _SwiGLU.apply(gate, up) if swiglu_native_ok(gate, up) else self.act_fn(gate) * up
+    return self.down_proj(h)
+
+
+# ---- installation ----------------------------------------------------------------------------------------------------
+
+def install_llama_glue(model: nn.Module) -> int:
+    """Route the Llama blocks of ``model`` through the native glue.  Returns the number of MLPs newly switched over."""
+    try:
+        from transformers.models.llama import modeling_llama as ml
+    except Exception:  # pragma: no cover - transformers is optional for the kernels themselves
+        return 0
+    n, has_attention = 0, False
+    for m in model.modules():
+        if isinstance(m, ml.LlamaAttention):
+            has_attention = True
+        elif type(m).forward is ml.LlamaMLP.forward and isinstance(m, ml.LlamaMLP) and _is_silu(m.act_fn):
+            if getattr(m.__dict__.get("forward"), "__func__", None) is not _llama_mlp_forward:
+                m.forward = types.MethodType(_llama_mlp_forward, m)
+                n += 1
+    if has_attention:
+        install_rope(ml)
+    return n

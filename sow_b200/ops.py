@@ -662,6 +662,87 @@ def adam_multi_dev(chunks: torch.Tensor, dtype: torch.dtype, lr, beta1, beta2, e
 
 
 # ---------------------------------------------------------------------------------------------------------
+# Llama block glue: rotary embedding and SwiGLU (bit-identical to the eager HF chains; sow_b200/llama_glue.py)
+# ---------------------------------------------------------------------------------------------------------
+
+def _glue_dtype_code(dt: torch.dtype) -> int:
+    if dt not in (torch.bfloat16, torch.float16):
+        raise SowB200Error(f"the Llama glue kernels take bf16 / fp16 tensors, not {dt}")
+    return _dtype_code(dt)
+
+
+def _rope_strided(t: torch.Tensor) -> torch.Tensor:
+    """(B, H, S, D) in any layout with a contiguous last dim, 16-byte aligned rows; anything else is made contiguous."""
+    if t.stride(-1) == 1 and t.data_ptr() % 16 == 0 and all(s % 8 == 0 for s in t.stride()[:3]):
+        return t
+    return t.contiguous()
+
+
+def _rope_call(fn: str, q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
+    _require_cuda(q, k, cos, sin)
+    B, Hq, S, D = q.shape
+    Hk = k.shape[1]
+    if k.shape != (B, Hk, S, D) or cos.shape != sin.shape or cos.shape not in ((1, S, D), (B, S, D)):
+        raise SowB200Error(f"{fn}: q {tuple(q.shape)}, k {tuple(k.shape)}, cos {tuple(cos.shape)} do not match")
+    if not (q.dtype == k.dtype == cos.dtype == sin.dtype) or not (cos.is_contiguous() and sin.is_contiguous()):
+        raise SowB200Error(f"{fn}: q, k, cos, sin must share one dtype and cos / sin be contiguous")
+    q, k = _rope_strided(q), _rope_strided(k)
+    # outputs (B, S, H, D) contiguous, returned as their (B, H, S, D) transpose: eager q_embed's strides
+    q_out = torch.empty((B, S, Hq, D), dtype=q.dtype, device=q.device).transpose(1, 2)
+    k_out = torch.empty((B, S, Hk, D), dtype=k.dtype, device=k.device).transpose(1, 2)
+    cs_sb = 0 if cos.shape[0] == 1 else S * D
+    rc = getattr(_lib.load(), fn)(_p(q), _p(k), _p(cos), _p(sin), _p(q_out), _p(k_out), B, S, Hq, Hk, D,
+                                  q.stride(0), q.stride(1), q.stride(2), k.stride(0), k.stride(1), k.stride(2), cs_sb,
+                                  _glue_dtype_code(q.dtype), _stream_ptr(q.device))
+    check(rc, fn)
+    launch_counter["kernels"] += 1
+    return q_out, k_out
+
+
+def rope_fwd(q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
+    """q * cos + rotate_half(q) * sin and the same for k, in one launch.  q, k: (B, H, S, D); cos, sin: (B or 1, S, D)."""
+    return _rope_call("sow_rope_fwd", q, k, cos, sin)
+
+
+def rope_bwd(gq: torch.Tensor, gk: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
+    """Gradients of rope_fwd w.r.t. q and k from the upstream gradients gq, gk (either layout), in one launch."""
+    return _rope_call("sow_rope_bwd", gq, gk, cos, sin)
+
+
+def _glue_contig(t: torch.Tensor) -> torch.Tensor:
+    return t if t.is_contiguous() and t.data_ptr() % 16 == 0 else t.contiguous()
+
+
+def swiglu_fwd(gate: torch.Tensor, up: torch.Tensor) -> torch.Tensor:
+    """silu(gate) * up."""
+    _require_cuda(gate, up)
+    if gate.shape != up.shape or gate.dtype != up.dtype:
+        raise SowB200Error("swiglu: gate and up must have the same shape and dtype")
+    gate, up = _glue_contig(gate), _glue_contig(up)
+    h = torch.empty_like(gate, memory_format=torch.contiguous_format)
+    rc = _lib.load().sow_swiglu_fwd(_p(gate), _p(up), _p(h), gate.numel(), _glue_dtype_code(gate.dtype),
+                                    _stream_ptr(gate.device))
+    check(rc, "sow_swiglu_fwd")
+    launch_counter["kernels"] += 1
+    return h
+
+
+def swiglu_bwd(dh: torch.Tensor, gate: torch.Tensor, up: torch.Tensor):
+    """(dgate, dup) of h = silu(gate) * up, in one pass over dh, gate and up."""
+    _require_cuda(dh, gate, up)
+    if not (dh.shape == gate.shape == up.shape) or not (dh.dtype == gate.dtype == up.dtype):
+        raise SowB200Error("swiglu: dh, gate and up must have the same shape and dtype")
+    dh, gate, up = _glue_contig(dh), _glue_contig(gate), _glue_contig(up)
+    dgate = torch.empty_like(gate, memory_format=torch.contiguous_format)
+    dup = torch.empty_like(up, memory_format=torch.contiguous_format)
+    rc = _lib.load().sow_swiglu_bwd(_p(dh), _p(gate), _p(up), _p(dgate), _p(dup), gate.numel(),
+                                    _glue_dtype_code(gate.dtype), _stream_ptr(gate.device))
+    check(rc, "sow_swiglu_bwd")
+    launch_counter["kernels"] += 1
+    return dgate, dup
+
+
+# ---------------------------------------------------------------------------------------------------------
 # live profiling (bench.py)
 # ---------------------------------------------------------------------------------------------------------
 PROF_CLASSES = {"gemm_fwd": 0, "gemm_dx": 1, "gemm_skinny": 2, "gemm_splitk": 3, "merge": 4, "adam": 5, "gemm_k2": 6}

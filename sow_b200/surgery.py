@@ -13,6 +13,7 @@ import torch
 import torch.nn as nn
 
 from .layer import SharedInputGroup, SoWArgs, SoWLinear, accumulate_modules
+from .llama_glue import install_llama_glue
 
 try:  # peft is optional: only the base classes are used by the reference (prepare.py:13)
     from peft import PeftConfig as _PeftConfigBase, PeftModel as _PeftModelBase  # type: ignore
@@ -107,6 +108,8 @@ def prepare_sow(model: nn.Module, config=None, decompose=None, args: Optional[So
         module.weight = None
     if getattr(config, "fuse_shared_input", True):
         group_shared_inputs(model)
+    # rotary embedding and SwiGLU of HF Llama blocks as native kernels (bit-identical to the eager chains)
+    install_llama_glue(model)
     if torch.cuda.is_available():
         torch.cuda.empty_cache()
     return model
