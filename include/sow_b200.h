@@ -314,6 +314,23 @@ int sow_adam_multi_dev(const void* chunks_dev, int n_chunks, int64_t total_elems
                        double eps, double weight_decay, float* step_dev, int decoupled, int dtype, void* stream);
 
 /*
+ * Mixed-precision variant for loss-scaled training (torch.amp.GradScaler):
+ *   state_dtype : dtype of m and v, either `dtype` or SOWB_F32 (fp32 moments for bf16 / fp16 parameters; each chunk-table
+ *                 pointer is offset by its own tensor's element size).  p, g keep `dtype`.
+ *   step_dev    : device step counter as in sow_adam_multi_dev, or NULL to use the host bias corrections (then both > 0).
+ *   grad_scale  : device fp32 scalar or NULL.  g / *grad_scale (IEEE division) is the gradient of the update, and it is
+ *                 written back into g, rounded to `dtype` (torch._fused_adamw_ does the same).
+ *   found_inf   : device fp32 scalar or NULL; requires step_dev.  Non-zero: the update does nothing (p, m, v and g keep
+ *                 every bit) and the step counter does not advance.
+ * Arguments are validated (SOWB_EINVAL) before any work is queued or the CUDA context is touched.
+ * Profiler bytes: (2 e_p + e_g + 4 e_state [+ e_g when grad_scale is given]) per element.
+ */
+int sow_adam_multi_amp(const void* chunks_dev, int n_chunks, int64_t total_elems, double lr, double beta1, double beta2,
+                       double eps, double weight_decay, double bias_correction1, double bias_correction2, float* step_dev,
+                       const float* grad_scale, const float* found_inf, int decoupled, int dtype, int state_dtype,
+                       void* stream);
+
+/*
  * Element-wise glue of the Llama block (HF transformers modeling_llama.py), bit-identical to the eager chains it replaces.
  * dtype SOWB_BF16 or SOWB_F16; math in fp32, each result rounded to the 16-bit type where eager rounds (see glue.cu).
  * Pointers 16-byte aligned.  One launch per call.

@@ -4,7 +4,8 @@
 // mode issues ~8 elementwise kernels per group chunk and, for bf16 parameters, rounds to bf16 after every one
 // of them.  Here each element is read once (p, g, m, v), updated in fp32 registers and written once:
 // 4 reads + 3 writes of the parameter dtype per element -> 14 B/element in bf16, the HBM floor for Adam.
-// State stays per-parameter and in the parameter dtype, exactly where torch keeps it, so
+// State stays per-parameter and by default in the parameter dtype, exactly where torch keeps it (sow_adam_multi_amp can keep
+// fp32 moments for 16-bit parameters: 22 B/element), so
 // scripts/utils/training_utils.py:257-277 (reset_optimizer, which REBINDS exp_avg / exp_avg_sq) keeps working:
 // the host side re-resolves the pointers whenever they change.
 #include "common.cuh"
@@ -37,8 +38,11 @@ __device__ __forceinline__ void adam_update(float& p, float g, float& m, float& 
 
 // CUDA-graph friendly step counter: the bias corrections are derived ON THE DEVICE from a counter that the launch
 // sequence itself advances, so a captured optimizer step replays with the right corrections (host-computed ones would
-// be frozen into the graph).
-__global__ void adam_step_inc_kernel(float* step) { *step += 1.0f; }
+// be frozen into the graph).  A step skipped for found_inf does not advance it (torch's fused AdamW subtracts found_inf
+// from the step it incremented).
+__global__ void adam_step_inc_kernel(float* step, const float* found_inf) {
+  if (found_inf == nullptr || *found_inf == 0.0f) *step += 1.0f;
+}
 
 __device__ __forceinline__ AdamHyper with_device_step(AdamHyper h, const float* __restrict__ step_dev) {
   if (step_dev != nullptr) {
@@ -71,18 +75,69 @@ struct Half16<__half> {
   static __device__ __forceinline__ __half from_f(float v) { return __float2half_rn(v); }
 };
 
-// p, g, m, v of type H (bf16 or fp16): 16-byte vector accesses (8 elements) when all four are 16-byte aligned
+// Moments are either of the parameter type H or fp32 (state_dtype): element conversions for both (Moment<float, float>
+// also serves the fp32 kernel's gradients)
+template <typename H, typename S>
+struct Moment {
+  static __device__ __forceinline__ float to_f(S v) { return Half16<H>::to_f(v); }
+  static __device__ __forceinline__ S from_f(float v) { return Half16<H>::from_f(v); }
+};
 template <typename H>
+struct Moment<H, float> {
+  static __device__ __forceinline__ float to_f(float v) { return v; }
+  static __device__ __forceinline__ float from_f(float v) { return v; }
+};
+
+// Gradient element i as the update reads it.  kAmp with a loss scale: g / scale (IEEE division, as torch's fused Adam
+// divides), and the unscaled value is written back to the gradient, rounded to its type, as torch._fused_adamw_ does.
+template <bool kAmp, typename G, typename C>
+__device__ __forceinline__ float grad_in(G* g, int64_t i, const float* scale) {
+  float x = C::to_f(g[i]);
+  if constexpr (kAmp) {
+    if (scale != nullptr) {
+      x = x / *scale;
+      g[i] = C::from_f(x);
+    }
+  }
+  return x;
+}
+// A packed pair of 16-bit gradients, unscaled in place as grad_in does for one element
+template <bool kAmp, typename C>
+__device__ __forceinline__ void unscale2(float2& gf, typename C::H2& g2, const float* scale) {
+  if constexpr (kAmp) {
+    if (scale != nullptr) {
+      gf.x = gf.x / *scale;
+      gf.y = gf.y / *scale;
+      g2 = C::from_f2(gf.x, gf.y);
+    }
+  }
+}
+
+// kAmp: the launch carries GradScaler's two device scalars.  found_inf != 0 -> the block returns before touching anything
+// (no decay, p / m / v / g keep every bit); grad_scale != NULL -> gradients are unscaled in the kernel.  Without kAmp the
+// pointers are never read, so these instantiations are the plain Adam kernels.
+template <bool kAmp>
+__device__ __forceinline__ bool amp_skip(const float* __restrict__ found_inf) {
+  if constexpr (kAmp) return found_inf != nullptr && *found_inf != 0.0f;
+  return false;
+}
+
+// p, g of type H (bf16 or fp16), m, v of type S (H or fp32): 16-byte vector accesses (8 elements of p and g, one or two
+// 16-byte accesses of m and v) when all four are 16-byte aligned
+template <typename H, typename S, bool kAmp>
 __global__ void __launch_bounds__(256)
-adam_multi_16bit_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0, const float* __restrict__ step_dev) {
+adam_multi_16bit_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0, const float* __restrict__ step_dev,
+                        const float* __restrict__ grad_scale, const float* __restrict__ found_inf) {
   using C = Half16<H>;
+  using M = Moment<H, S>;
   using H2 = typename C::H2;
+  if (amp_skip<kAmp>(found_inf)) return;
   const AdamHyper h = with_device_step(h0, step_dev);
   const AdamChunk c = chunks[blockIdx.x];
   H* p = static_cast<H*>(c.p);
-  const H* g = static_cast<const H*>(c.g);
-  H* m = static_cast<H*>(c.m);
-  H* v = static_cast<H*>(c.v);
+  H* g = static_cast<H*>(const_cast<void*>(c.g));
+  S* m = static_cast<S*>(c.m);
+  S* v = static_cast<S*>(c.v);
   const bool aligned = ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) |
                          reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15) == 0;
   int64_t done = 0;
@@ -90,44 +145,71 @@ adam_multi_16bit_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0
     const int64_t nvec = c.n / 8;
     for (int64_t i = threadIdx.x; i < nvec; i += blockDim.x) {
       uint4 pp = reinterpret_cast<uint4*>(p)[i];
-      const uint4 gg = reinterpret_cast<const uint4*>(g)[i];
-      uint4 mm = reinterpret_cast<uint4*>(m)[i];
-      uint4 vv = reinterpret_cast<uint4*>(v)[i];
+      uint4 gg = reinterpret_cast<const uint4*>(g)[i];
       H2* p2 = reinterpret_cast<H2*>(&pp);
-      const H2* g2 = reinterpret_cast<const H2*>(&gg);
-      H2* m2 = reinterpret_cast<H2*>(&mm);
-      H2* v2 = reinterpret_cast<H2*>(&vv);
+      H2* g2 = reinterpret_cast<H2*>(&gg);
+      if constexpr (std::is_same<S, H>::value) {
+        uint4 mm = reinterpret_cast<uint4*>(m)[i];
+        uint4 vv = reinterpret_cast<uint4*>(v)[i];
+        H2* m2 = reinterpret_cast<H2*>(&mm);
+        H2* v2 = reinterpret_cast<H2*>(&vv);
 #pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        float2 pf = C::to_f2(p2[j]), gf = C::to_f2(g2[j]);
-        float2 mf = C::to_f2(m2[j]), vf = C::to_f2(v2[j]);
-        adam_update(pf.x, gf.x, mf.x, vf.x, h);
-        adam_update(pf.y, gf.y, mf.y, vf.y, h);
-        p2[j] = C::from_f2(pf.x, pf.y);
-        m2[j] = C::from_f2(mf.x, mf.y);
-        v2[j] = C::from_f2(vf.x, vf.y);
+        for (int j = 0; j < 4; ++j) {
+          float2 pf = C::to_f2(p2[j]), gf = C::to_f2(g2[j]);
+          float2 mf = C::to_f2(m2[j]), vf = C::to_f2(v2[j]);
+          unscale2<kAmp, C>(gf, g2[j], grad_scale);
+          adam_update(pf.x, gf.x, mf.x, vf.x, h);
+          adam_update(pf.y, gf.y, mf.y, vf.y, h);
+          p2[j] = C::from_f2(pf.x, pf.y);
+          m2[j] = C::from_f2(mf.x, mf.y);
+          v2[j] = C::from_f2(vf.x, vf.y);
+        }
+        reinterpret_cast<uint4*>(p)[i] = pp;
+        reinterpret_cast<uint4*>(m)[i] = mm;
+        reinterpret_cast<uint4*>(v)[i] = vv;
+      } else {
+        float4 mm[2] = {reinterpret_cast<float4*>(m)[2 * i], reinterpret_cast<float4*>(m)[2 * i + 1]};
+        float4 vv[2] = {reinterpret_cast<float4*>(v)[2 * i], reinterpret_cast<float4*>(v)[2 * i + 1]};
+        float* mf = reinterpret_cast<float*>(mm);
+        float* vf = reinterpret_cast<float*>(vv);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          float2 pf = C::to_f2(p2[j]), gf = C::to_f2(g2[j]);
+          unscale2<kAmp, C>(gf, g2[j], grad_scale);
+          adam_update(pf.x, gf.x, mf[2 * j], vf[2 * j], h);
+          adam_update(pf.y, gf.y, mf[2 * j + 1], vf[2 * j + 1], h);
+          p2[j] = C::from_f2(pf.x, pf.y);
+        }
+        reinterpret_cast<uint4*>(p)[i] = pp;
+        reinterpret_cast<float4*>(m)[2 * i] = mm[0];
+        reinterpret_cast<float4*>(m)[2 * i + 1] = mm[1];
+        reinterpret_cast<float4*>(v)[2 * i] = vv[0];
+        reinterpret_cast<float4*>(v)[2 * i + 1] = vv[1];
       }
-      reinterpret_cast<uint4*>(p)[i] = pp;
-      reinterpret_cast<uint4*>(m)[i] = mm;
-      reinterpret_cast<uint4*>(v)[i] = vv;
+      if constexpr (kAmp) {
+        if (grad_scale != nullptr) reinterpret_cast<uint4*>(g)[i] = gg;
+      }
     }
     done = nvec * 8;
   }
   for (int64_t i = done + threadIdx.x; i < c.n; i += blockDim.x) {
-    float pf = C::to_f(p[i]), mf = C::to_f(m[i]), vf = C::to_f(v[i]);
-    adam_update(pf, C::to_f(g[i]), mf, vf, h);
+    float pf = C::to_f(p[i]), mf = M::to_f(m[i]), vf = M::to_f(v[i]);
+    adam_update(pf, grad_in<kAmp, H, C>(g, i, grad_scale), mf, vf, h);
     p[i] = C::from_f(pf);
-    m[i] = C::from_f(mf);
-    v[i] = C::from_f(vf);
+    m[i] = M::from_f(mf);
+    v[i] = M::from_f(vf);
   }
 }
 
+template <bool kAmp>
 __global__ void __launch_bounds__(256)
-adam_multi_f32_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0, const float* __restrict__ step_dev) {
+adam_multi_f32_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0, const float* __restrict__ step_dev,
+                      const float* __restrict__ grad_scale, const float* __restrict__ found_inf) {
+  if (amp_skip<kAmp>(found_inf)) return;
   const AdamHyper h = with_device_step(h0, step_dev);
   const AdamChunk c = chunks[blockIdx.x];
   float* p = static_cast<float*>(c.p);
-  const float* g = static_cast<const float*>(c.g);
+  float* g = static_cast<float*>(const_cast<void*>(c.g));
   float* m = static_cast<float*>(c.m);
   float* v = static_cast<float*>(c.v);
   const bool aligned = ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) |
@@ -137,7 +219,17 @@ adam_multi_f32_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0, 
     const int64_t nvec = c.n / 4;
     for (int64_t i = threadIdx.x; i < nvec; i += blockDim.x) {
       float4 pp = reinterpret_cast<float4*>(p)[i];
-      const float4 gg = reinterpret_cast<const float4*>(g)[i];
+      float4 gg = reinterpret_cast<const float4*>(g)[i];
+      if constexpr (kAmp) {
+        if (grad_scale != nullptr) {
+          const float s = *grad_scale;
+          gg.x = gg.x / s;
+          gg.y = gg.y / s;
+          gg.z = gg.z / s;
+          gg.w = gg.w / s;
+          reinterpret_cast<float4*>(g)[i] = gg;
+        }
+      }
       float4 mm = reinterpret_cast<float4*>(m)[i];
       float4 vv = reinterpret_cast<float4*>(v)[i];
       adam_update(pp.x, gg.x, mm.x, vv.x, h);
@@ -150,12 +242,24 @@ adam_multi_f32_kernel(const AdamChunk* __restrict__ chunks, const AdamHyper h0, 
     }
     done = nvec * 4;
   }
-  for (int64_t i = done + threadIdx.x; i < c.n; i += blockDim.x) adam_update(p[i], g[i], m[i], v[i], h);
+  for (int64_t i = done + threadIdx.x; i < c.n; i += blockDim.x)
+    adam_update(p[i], grad_in<kAmp, float, Moment<float, float>>(g, i, grad_scale), m[i], v[i], h);
 }
 
 }  // namespace sowb
 
 using namespace sowb;
+
+static int elem_bytes(int dtype) { return dtype == SOWB_F32 ? 4 : 2; }
+
+template <bool kAmp, typename H>
+static void launch_16bit(int n_chunks, const AdamChunk* ch, const AdamHyper& h, const float* step_dev,
+                         const float* grad_scale, const float* found_inf, int state_dtype, cudaStream_t stream) {
+  if (state_dtype == SOWB_F32)
+    adam_multi_16bit_kernel<H, float, true><<<n_chunks, 256, 0, stream>>>(ch, h, step_dev, grad_scale, found_inf);
+  else
+    adam_multi_16bit_kernel<H, H, kAmp><<<n_chunks, 256, 0, stream>>>(ch, h, step_dev, grad_scale, found_inf);
+}
 
 extern "C" {
 
@@ -174,32 +278,52 @@ int sow_adam_multi(const void* chunks_dev, int n_chunks, double lr, double beta1
 
 static int adam_launch(const void* chunks_dev, int n_chunks, int64_t total_elems, double lr, double beta1, double beta2,
                        double eps, double weight_decay, double bias_correction1, double bias_correction2, float* step_dev,
-                       int decoupled, int dtype, void* stream_);
+                       const float* grad_scale, const float* found_inf, bool amp, int decoupled, int dtype,
+                       int state_dtype, void* stream_);
 
 int sow_adam_multi_ex(const void* chunks_dev, int n_chunks, int64_t total_elems, double lr, double beta1, double beta2, double eps,
                       double weight_decay, double bias_correction1, double bias_correction2, int decoupled,
                       int dtype, void* stream_) {
   SOWB_REQUIRE(bias_correction1 > 0.0 && bias_correction2 > 0.0, "sow_adam_multi: bias corrections must be positive");
   return adam_launch(chunks_dev, n_chunks, total_elems, lr, beta1, beta2, eps, weight_decay, bias_correction1,
-                     bias_correction2, nullptr, decoupled, dtype, stream_);
+                     bias_correction2, nullptr, nullptr, nullptr, false, decoupled, dtype, dtype, stream_);
 }
 
 int sow_adam_multi_dev(const void* chunks_dev, int n_chunks, int64_t total_elems, double lr, double beta1, double beta2,
                        double eps, double weight_decay, float* step_dev, int decoupled, int dtype, void* stream_) {
   SOWB_REQUIRE(step_dev != nullptr, "sow_adam_multi_dev: null step counter");
-  return adam_launch(chunks_dev, n_chunks, total_elems, lr, beta1, beta2, eps, weight_decay, 1.0, 1.0, step_dev, decoupled,
-                     dtype, stream_);
+  return adam_launch(chunks_dev, n_chunks, total_elems, lr, beta1, beta2, eps, weight_decay, 1.0, 1.0, step_dev, nullptr,
+                     nullptr, false, decoupled, dtype, dtype, stream_);
+}
+
+int sow_adam_multi_amp(const void* chunks_dev, int n_chunks, int64_t total_elems, double lr, double beta1, double beta2,
+                       double eps, double weight_decay, double bias_correction1, double bias_correction2, float* step_dev,
+                       const float* grad_scale, const float* found_inf, int decoupled, int dtype, int state_dtype,
+                       void* stream_) {
+  SOWB_REQUIRE(dtype == SOWB_BF16 || dtype == SOWB_F16 || dtype == SOWB_F32, "sow_adam_multi_amp: unknown dtype %d", dtype);
+  SOWB_REQUIRE(state_dtype == dtype || state_dtype == SOWB_F32,
+               "sow_adam_multi_amp: state dtype %d unsupported for parameter dtype %d (the parameter's, or fp32)",
+               state_dtype, dtype);
+  SOWB_REQUIRE(found_inf == nullptr || step_dev != nullptr,
+               "sow_adam_multi_amp: found_inf needs the device step counter (a host counter skips on the host)");
+  SOWB_REQUIRE(step_dev != nullptr || (bias_correction1 > 0.0 && bias_correction2 > 0.0),
+               "sow_adam_multi_amp: bias corrections must be positive");
+  return adam_launch(chunks_dev, n_chunks, total_elems, lr, beta1, beta2, eps, weight_decay,
+                     step_dev != nullptr ? 1.0 : bias_correction1, step_dev != nullptr ? 1.0 : bias_correction2, step_dev,
+                     grad_scale, found_inf, true, decoupled, dtype, state_dtype, stream_);
 }
 
 static int adam_launch(const void* chunks_dev, int n_chunks, int64_t total_elems, double lr, double beta1, double beta2,
                        double eps, double weight_decay, double bias_correction1, double bias_correction2, float* step_dev,
-                       int decoupled, int dtype, void* stream_) {
+                       const float* grad_scale, const float* found_inf, bool amp, int decoupled, int dtype,
+                       int state_dtype, void* stream_) {
   if (n_chunks <= 0) return SOWB_OK;
   SOWB_REQUIRE(chunks_dev != nullptr, "sow_adam_multi: null chunk table");
+  SOWB_REQUIRE(dtype == SOWB_BF16 || dtype == SOWB_F16 || dtype == SOWB_F32, "sow_adam_multi: unknown dtype %d", dtype);
   if (int rc0 = ensure_context_for(chunks_dev)) return rc0;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   if (step_dev != nullptr) {
-    adam_step_inc_kernel<<<1, 1, 0, stream>>>(step_dev);
+    adam_step_inc_kernel<<<1, 1, 0, stream>>>(step_dev, found_inf);
     SOWB_CHECK_CUDA(cudaGetLastError());
   }
   AdamHyper h;
@@ -214,16 +338,22 @@ static int adam_launch(const void* chunks_dev, int n_chunks, int64_t total_elems
   h.step_size = float(lr / bias_correction1);
   h.inv_sqrt_bc2 = float(1.0 / sqrt(bias_correction2));
   h.decoupled = decoupled;
-  // algorithmic bytes: p, m, v read+written, g read = 7 accesses of the element size
-  ProfileScope prof(stream, PROF_ADAM, 7.0 * double(total_elems) * (dtype == SOWB_F32 ? 4 : 2));
-  if (dtype == SOWB_BF16)
-    adam_multi_16bit_kernel<__nv_bfloat16><<<n_chunks, 256, 0, stream>>>(static_cast<const AdamChunk*>(chunks_dev), h, step_dev);
-  else if (dtype == SOWB_F16)
-    adam_multi_16bit_kernel<__half><<<n_chunks, 256, 0, stream>>>(static_cast<const AdamChunk*>(chunks_dev), h, step_dev);
-  else if (dtype == SOWB_F32)
-    adam_multi_f32_kernel<<<n_chunks, 256, 0, stream>>>(static_cast<const AdamChunk*>(chunks_dev), h, step_dev);
-  else
-    return set_error(SOWB_EINVAL, "sow_adam_multi: unknown dtype %d", dtype);
+  // algorithmic bytes: p and the moments read + written, g read (and written back when it is unscaled)
+  const int ep = elem_bytes(dtype), es = elem_bytes(state_dtype);
+  ProfileScope prof(stream, PROF_ADAM, double(2 * ep + ep + 4 * es + (grad_scale != nullptr ? ep : 0)) * double(total_elems));
+  const AdamChunk* ch = static_cast<const AdamChunk*>(chunks_dev);
+  if (dtype == SOWB_F32) {
+    if (amp)
+      adam_multi_f32_kernel<true><<<n_chunks, 256, 0, stream>>>(ch, h, step_dev, grad_scale, found_inf);
+    else
+      adam_multi_f32_kernel<false><<<n_chunks, 256, 0, stream>>>(ch, h, step_dev, nullptr, nullptr);
+  } else if (dtype == SOWB_BF16) {
+    if (amp) launch_16bit<true, __nv_bfloat16>(n_chunks, ch, h, step_dev, grad_scale, found_inf, state_dtype, stream);
+    else launch_16bit<false, __nv_bfloat16>(n_chunks, ch, h, step_dev, nullptr, nullptr, state_dtype, stream);
+  } else {
+    if (amp) launch_16bit<true, __half>(n_chunks, ch, h, step_dev, grad_scale, found_inf, state_dtype, stream);
+    else launch_16bit<false, __half>(n_chunks, ch, h, step_dev, nullptr, nullptr, state_dtype, stream);
+  }
   SOWB_CHECK_CUDA(cudaGetLastError());
   return SOWB_OK;
 }

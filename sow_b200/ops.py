@@ -627,11 +627,13 @@ def build_adam_chunks(ps: List[torch.Tensor], gs: List[torch.Tensor], ms: List[t
         _require_cuda(p, g, m, v)
         if not (p.is_contiguous() and g.is_contiguous() and m.is_contiguous() and v.is_contiguous()):
             raise SowB200Error("fused Adam needs contiguous p/g/m/v")
-        es = p.element_size()
         n = p.numel()
+        if not (g.numel() == m.numel() == v.numel() == n):
+            raise SowB200Error("fused Adam needs p/g/m/v of the same size")
+        ep, eg, em, ev = p.element_size(), g.element_size(), m.element_size(), v.element_size()
         for off in range(0, n, ce):
-            rows.append((p.data_ptr() + off * es, g.data_ptr() + off * es, m.data_ptr() + off * es,
-                         v.data_ptr() + off * es, min(ce, n - off)))
+            rows.append((p.data_ptr() + off * ep, g.data_ptr() + off * eg, m.data_ptr() + off * em,
+                         v.data_ptr() + off * ev, min(ce, n - off)))
     table = torch.from_numpy(np.asarray(rows, dtype=np.int64).reshape(-1, 5)).to(ps[0].device, non_blocking=False)
     table._sow_total_elems = int(sum(p.numel() for p in ps))
     return table
@@ -659,6 +661,26 @@ def adam_multi_dev(chunks: torch.Tensor, dtype: torch.dtype, lr, beta1, beta2, e
                                 _stream_ptr(chunks.device))
     check(rc, "sow_adam_multi_dev")
     launch_counter["kernels"] += 2
+
+
+def adam_multi_amp(chunks: torch.Tensor, dtype: torch.dtype, state_dtype: torch.dtype, lr, beta1, beta2, eps, weight_decay,
+                   decoupled, bc1=1.0, bc2=1.0, step_dev: Optional[torch.Tensor] = None,
+                   grad_scale: Optional[torch.Tensor] = None, found_inf: Optional[torch.Tensor] = None):
+    """Fused Adam with moments of ``state_dtype`` (the parameter dtype or fp32) and torch.amp.GradScaler's device scalars:
+    ``grad_scale`` unscales the gradients in the kernel (and writes them back unscaled), ``found_inf`` != 0 skips the step
+    on the device.  ``step_dev`` given: device step counter as in adam_multi_dev (required with ``found_inf``); otherwise
+    the host bias corrections ``bc1``, ``bc2``."""
+    lib = _lib.load()
+    for name, t in (("step", step_dev), ("grad_scale", grad_scale), ("found_inf", found_inf)):
+        if t is not None and not (t.is_cuda and t.dtype == torch.float32 and t.numel() == 1 and t.device == chunks.device):
+            raise SowB200Error(f"adam_multi_amp: {name} must be a single-element fp32 tensor on {chunks.device}")
+    total = getattr(chunks, "_sow_total_elems", 0)
+    rc = lib.sow_adam_multi_amp(_p(chunks), chunks.shape[0], total, float(lr), float(beta1), float(beta2), float(eps),
+                                float(weight_decay), float(bc1), float(bc2), _p(step_dev), _p(grad_scale), _p(found_inf),
+                                1 if decoupled else 0, _dtype_code(dtype), _dtype_code(state_dtype),
+                                _stream_ptr(chunks.device))
+    check(rc, "sow_adam_multi_amp")
+    launch_counter["kernels"] += 1 if step_dev is None else 2
 
 
 # ---------------------------------------------------------------------------------------------------------

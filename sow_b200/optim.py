@@ -319,6 +319,16 @@ class TTSGD(torch.optim.Optimizer):
         return loss
 
 
+def _check_state_dtype(param_dtype: torch.dtype, state_dtype) -> None:
+    """FusedAdamW's moments: the parameter dtype (``None``), or fp32 for bf16 / fp16 parameters."""
+    if state_dtype is None or state_dtype == param_dtype:
+        return
+    if state_dtype == torch.float32 and param_dtype in (torch.bfloat16, torch.float16):
+        return
+    raise SowB200Error(f"FusedAdamW: state_dtype {state_dtype} is not supported for {param_dtype} parameters "
+                       "(None = the parameter dtype, or torch.float32 for bf16 / fp16 parameters)")
+
+
 class FusedAdamW(torch.optim.Optimizer):
     """Multi-tensor AdamW / Adam on one kernel launch per param group (SURVEY.md 8f rank 1).
 
@@ -329,21 +339,78 @@ class FusedAdamW(torch.optim.Optimizer):
     ``capturable=True`` (as in torch.optim.AdamW): ``state[p]["step"]`` lives on the device -- one fp32 counter shared by
     the parameters of a group -- the kernels advance it and derive the bias corrections from it, and ``step()`` performs
     no host-side arithmetic on it, so the whole optimizer step can be captured in a CUDA graph and replayed.
+
+    ``state_dtype`` (per group): ``torch.float32`` keeps ``exp_avg`` / ``exp_avg_sq`` in fp32 for bf16 / fp16
+    parameters.  fp16 moments underflow ((1 - beta2) * g^2 is 0 below |g| ~ 8e-3), so training fp16 weights needs them.
+    Moments that ``reset_optimizer`` rebinds in the parameter dtype are converted back (exactly: they are zeros) on the
+    next step, and ``load_state_dict`` keeps them in fp32.
+
+    torch.amp.GradScaler: ``step()`` takes the ``grad_scale`` / ``found_inf`` tensors GradScaler.step sets on the
+    optimizer (``_step_supports_amp_scaling``).  The kernel unscales the gradients (and writes them back unscaled, as
+    torch's fused AdamW does) and, for capturable groups, skips a step with found_inf on the device: no host sync, so a
+    loss-scaled step can be captured in a CUDA graph.  Non-capturable groups read found_inf once on the host and leave
+    parameters, moments and ``step`` untouched when it is set.
     """
 
+    _step_supports_amp_scaling = True
+
     def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, amsgrad=False,
-                 decoupled=True, capturable=False):
+                 decoupled=True, capturable=False, state_dtype=None):
         if amsgrad:
             raise SowB200Error("FusedAdamW: amsgrad is not implemented")
         defaults = dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay, amsgrad=amsgrad, decoupled=decoupled,
-                        capturable=capturable)
+                        capturable=capturable, state_dtype=state_dtype)
         super().__init__(params, defaults)
         self._tables = {}
 
-    def _step_capturable(self, gi, group):
+    def add_param_group(self, param_group):
+        super().add_param_group(param_group)
+        group = self.param_groups[-1]
+        for p in group["params"]:
+            _check_state_dtype(p.dtype, group.get("state_dtype"))
+
+    def load_state_dict(self, state_dict):
+        """torch's load_state_dict casts every floating-point state tensor to the parameter dtype (through
+        ``Optimizer._process_value_according_to_param_policy``, called by class name, so a subclass cannot override it);
+        the moments of groups with a ``state_dtype`` are taken from the checkpoint in that dtype instead."""
+        keep = {}
+        for group, saved in zip(self.param_groups, state_dict["param_groups"]):
+            sdt = saved.get("state_dtype")
+            if sdt is None:
+                continue
+            for p, pid in zip(group["params"], saved["params"]):
+                st = state_dict["state"].get(pid, {})
+                keep[p] = (sdt, {k: st[k] for k in ("exp_avg", "exp_avg_sq") if isinstance(st.get(k), torch.Tensor)})
+        super().load_state_dict(state_dict)
+        for p, (sdt, moments) in keep.items():
+            for k, v in moments.items():
+                self.state[p][k] = v.to(device=p.device, dtype=sdt)
+
+    @staticmethod
+    def _init_state(p, st, sdt):
+        """Moments of dtype ``sdt``, created on the first step (``step`` None) or converted after reset_optimizer rebound
+        them."""
+        if len(st) == 0 or "exp_avg" not in st:
+            st["step"] = None
+            st["exp_avg"] = torch.zeros_like(p, dtype=sdt, memory_format=torch.preserve_format)
+            st["exp_avg_sq"] = torch.zeros_like(p, dtype=sdt, memory_format=torch.preserve_format)
+        for k in ("exp_avg", "exp_avg_sq"):
+            if st[k].dtype != sdt:
+                st[k] = st[k].to(sdt)
+
+    @staticmethod
+    def _grad(p, grad_scale):
+        if p.grad.dtype == p.dtype:
+            return p.grad
+        if grad_scale is not None:
+            raise SowB200Error("FusedAdamW: loss-scaled gradients must have the parameter dtype (they are unscaled in place)")
+        return p.grad.to(p.dtype)
+
+    def _step_capturable(self, gi, group, grad_scale=None, found_inf=None):
         """One device counter per (group, dtype); parameters whose ``step`` was rebound by reset_optimizer (a fresh zero
         tensor) are folded back onto a shared counter restarted from that value."""
         beta1, beta2 = group["betas"]
+        gsdt = group.get("state_dtype")
         by_dtype = {}
         for p in group["params"]:
             if p.grad is None:
@@ -351,11 +418,8 @@ class FusedAdamW(torch.optim.Optimizer):
             if not p.is_cuda:
                 raise SowB200Error("FusedAdamW needs CUDA parameters (no CPU fallback)")
             st = self.state[p]
-            if len(st) == 0 or "exp_avg" not in st:
-                st["step"] = None
-                st["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
-                st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
-            g = p.grad if p.grad.dtype == p.dtype else p.grad.to(p.dtype)
+            self._init_state(p, st, gsdt or p.dtype)
+            g = self._grad(p, grad_scale)
             by_dtype.setdefault(p.dtype, []).append((p, g, st))
         for dtype, items in by_dtype.items():
             ckey = ("counter", gi, dtype)
@@ -383,8 +447,13 @@ class FusedAdamW(torch.optim.Optimizer):
                                                      [st["exp_avg"] for _, _, st in items],
                                                      [st["exp_avg_sq"] for _, _, st in items]))
                 self._tables[key] = cached
-            ops.adam_multi_dev(cached[1], dtype, group["lr"], beta1, beta2, group["eps"], group["weight_decay"], counter,
-                               group["decoupled"])
+            sdt = items[0][2]["exp_avg"].dtype
+            if sdt == dtype and grad_scale is None and found_inf is None:
+                ops.adam_multi_dev(cached[1], dtype, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
+                                   counter, group["decoupled"])
+            else:
+                ops.adam_multi_amp(cached[1], dtype, sdt, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
+                                   group["decoupled"], step_dev=counter, grad_scale=grad_scale, found_inf=found_inf)
 
     @torch.no_grad()
     def step(self, closure=None):
@@ -392,23 +461,32 @@ class FusedAdamW(torch.optim.Optimizer):
         if closure is not None:
             with torch.enable_grad():
                 loss = closure()
+        # set by torch.amp.GradScaler.step for the duration of this call; grad_scale is None after an explicit unscale_
+        grad_scale = getattr(self, "grad_scale", None)
+        found_inf = getattr(self, "found_inf", None)
+        skip = None                             # found_inf read on the host, once, for the non-capturable groups
         for gi, group in enumerate(self.param_groups):
             if group.get("capturable", False):
-                self._step_capturable(gi, group)
+                self._step_capturable(gi, group, grad_scale, found_inf)
                 continue
+            if found_inf is not None:
+                if skip is None:
+                    skip = bool(found_inf.item())
+                if skip:
+                    continue
             buckets = {}
+            gsdt = group.get("state_dtype")
             for p in group["params"]:
                 if p.grad is None:
                     continue
                 if not p.is_cuda:
                     raise SowB200Error("FusedAdamW needs CUDA parameters (no CPU fallback)")
                 st = self.state[p]
-                if len(st) == 0 or "exp_avg" not in st:
+                self._init_state(p, st, gsdt or p.dtype)
+                if st["step"] is None:
                     st["step"] = torch.zeros((), dtype=torch.float32)
-                    st["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
-                    st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
                 st["step"] += 1
-                g = p.grad if p.grad.dtype == p.dtype else p.grad.to(p.dtype)
+                g = self._grad(p, grad_scale)
                 buckets.setdefault((int(st["step"]), p.dtype), []).append((p, g, st["exp_avg"], st["exp_avg_sq"]))
             beta1, beta2 = group["betas"]
             for (step, dtype), items in buckets.items():
@@ -419,6 +497,12 @@ class FusedAdamW(torch.optim.Optimizer):
                     ps, gs, ms, vs = zip(*items)
                     cached = (sig, ops.build_adam_chunks([p.data for p in ps], list(gs), list(ms), list(vs)))
                     self._tables[key] = cached
-                ops.adam_multi(cached[1], dtype, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
-                               1.0 - beta1 ** step, 1.0 - beta2 ** step, group["decoupled"])
+                sdt = items[0][2].dtype
+                if sdt == dtype and grad_scale is None:
+                    ops.adam_multi(cached[1], dtype, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
+                                   1.0 - beta1 ** step, 1.0 - beta2 ** step, group["decoupled"])
+                else:
+                    ops.adam_multi_amp(cached[1], dtype, sdt, group["lr"], beta1, beta2, group["eps"],
+                                       group["weight_decay"], group["decoupled"], 1.0 - beta1 ** step, 1.0 - beta2 ** step,
+                                       grad_scale=grad_scale)
         return loss

@@ -110,6 +110,10 @@ class TrainConfig:
     compile: bool = False                # torch.compile(model) as scripts/finetune.py:486-487 does (SoW layers = custom ops)
     cuda_graph: bool = False             # capture forward + backward + optimizer step in one CUDA graph and replay it
                                          # (small per-GPU batches are launch-bound: ~5 k launches per step); single GPU
+    optimizer_state_dtype: Optional[torch.dtype] = None   # FusedAdamW moments: None = parameter dtype, or torch.float32
+    loss_scaling: bool = False           # dynamic loss scaling (torch.amp.GradScaler) for fp16 training; capturable optimizer
+    loss_scale_init: float = 2.0 ** 16
+    loss_scale_growth_interval: int = 2000
 
 
 class SoWTrainer:
@@ -119,6 +123,15 @@ class SoWTrainer:
                  targets: Optional[list] = None):
         """``model``: an already built (and possibly already SoW-prepared) module to train instead of the named config;
         ``targets``: its SoW target module names."""
+        if cfg.loss_scaling and not cfg.fused_optimizer:
+            raise ValueError("loss_scaling needs the fused optimizer (GradScaler cannot unscale fp16 gradients for "
+                             "torch.optim.AdamW)")
+        if cfg.loss_scaling and cfg.dtype == torch.bfloat16:
+            raise ValueError("loss_scaling is not available for bf16 models: torch.amp.GradScaler has no bf16 inf / nan "
+                             "check, and bf16 has fp32's exponent range, so its gradients need no scaling")
+        if cfg.loss_scaling and cfg.grad_clipping != 0.0:
+            raise ValueError("loss_scaling with grad_clipping is not supported (the norm of scaled fp16 gradients "
+                             "overflows)")
         self.cfg = cfg
         self.device = device
         self.is_classifier = cfg.model.startswith("roberta")
@@ -164,8 +177,14 @@ class SoWTrainer:
         groups.append({"params": self.special, "lr": cfg.sow_lr, "weight_decay": cfg.weight_decay})
         if cfg.cuda_graph and not cfg.fused_optimizer:
             raise ValueError("cuda_graph needs the fused optimizer (device-side step counter)")
-        self.optimizer = (FusedAdamW(groups, capturable=cfg.cuda_graph) if cfg.fused_optimizer
+        self.optimizer = (FusedAdamW(groups, capturable=cfg.cuda_graph or cfg.loss_scaling,
+                                     state_dtype=cfg.optimizer_state_dtype) if cfg.fused_optimizer
                           else torch.optim.AdamW(groups))                                               # :502-506
+        # loss scaling: found_inf is computed inside scaler.step, after the bucket all-reduce, so every rank skips alike;
+        # the capturable optimizer unscales and skips on the device (no host sync, so the step can be graphed)
+        self.scaler = (torch.amp.GradScaler(device.type, init_scale=cfg.loss_scale_init,
+                                            growth_interval=cfg.loss_scale_growth_interval)
+                       if cfg.loss_scaling else None)
         broadcast_parameters(model)                                                # DDP ctor semantics (:566-572)
         self.grad_sync = FlatGradSync(self.trainable + self.special, overlap=cfg.overlap_grad_sync, direct=self.special)
         self.global_step = 0
@@ -240,7 +259,10 @@ class SoWTrainer:
             labels = input_ids
         kw = {} if attention_mask is None else {"attention_mask": attention_mask}
         loss = self.forward_fn(input_ids=input_ids, labels=labels, **kw).loss      # simple_train.py:611 / run_glue.py:978
-        (loss / cfg.gradient_accumulation).backward()                              # :612-613 (+ overlapped all-reduce)
+        if self.scaler is not None:
+            self.scaler.scale(loss / cfg.gradient_accumulation).backward()
+        else:
+            (loss / cfg.gradient_accumulation).backward()                          # :612-613 (+ overlapped all-reduce)
         accumulation_step = int(cfg.gradient_accumulation * cfg.sow_accumulation)
         G = cfg.gradient_accumulation
         capturing = torch.cuda.is_current_stream_capturing()
@@ -261,7 +283,11 @@ class SoWTrainer:
             return loss.detach()
         if cfg.grad_clipping != 0.0:
             torch.nn.utils.clip_grad_norm_(self.trainable, cfg.grad_clipping)      # :631
-        self.optimizer.step()                                                      # :646
+        if self.scaler is not None:
+            self.scaler.step(self.optimizer)   # a skipped step (inf / nan gradients) still counts as an update step
+            self.scaler.update()
+        else:
+            self.optimizer.step()                                                  # :646
         self.grad_sync.zero_grad()                                                 # :647 (one memset per bucket)
         if not capturing:
             self.update_step += 1
