@@ -331,6 +331,31 @@ int sow_adam_multi_amp(const void* chunks_dev, int n_chunks, int64_t total_elems
                        void* stream);
 
 /*
+ * Gradient clipping by the global 2-norm (torch.nn.utils.clip_grad_norm_, norm type 2), on the device and without atomics:
+ *   sow_grad_norm_partials : one fp32 partial sum of squares per row of an Adam chunk table (reads g and n of each row;
+ *                            dtype is the gradients' type), written to partials[0 .. n_chunks).  grad_scale: NULL, or
+ *                            GradScaler's device scale, in which case each element is round_dtype(g / *grad_scale) -- the
+ *                            value sow_adam_multi_amp's unscale writes back.  The tables of one param group write to
+ *                            consecutive ranges of one partials buffer.
+ *   sow_grad_norm_finalize : *total_norm = float(sqrt(sum of partials in fp64)), and the clip coefficient exactly as torch
+ *                            computes it on an fp32 tensor: r = 1.0f / (total_norm + 1e-6f), c = r * (float)max_norm,
+ *                            *clip_coef = min(c, 1) with NaN propagated.  An inf norm gives 0, a NaN norm NaN.
+ *   sow_adam_multi_clip    : sow_adam_multi_amp with the gradient round(round(g / scale) * *clip_coef) (the unscale only when
+ *                            grad_scale is given), which is also written back into g.  found_inf still skips everything.
+ * Every result is bit-reproducible.  Arguments are validated (SOWB_EINVAL) before any work is queued or the CUDA context
+ * is touched: unknown dtypes, n_chunks < 0, NULL pointers where a value is needed, n_partials < 1, max_norm not finite or
+ * not > 0, and the dtype combinations sow_adam_multi_amp rejects.
+ */
+int sow_grad_norm_partials(const void* chunks_dev, int n_chunks, int dtype, const float* grad_scale, float* partials,
+                           void* stream);
+int sow_grad_norm_finalize(const float* partials, int n_partials, double max_norm, float* total_norm, float* clip_coef,
+                           void* stream);
+int sow_adam_multi_clip(const void* chunks_dev, int n_chunks, int64_t total_elems, double lr, double beta1, double beta2,
+                        double eps, double weight_decay, double bias_correction1, double bias_correction2, float* step_dev,
+                        const float* grad_scale, const float* found_inf, const float* clip_coef, int decoupled, int dtype,
+                        int state_dtype, void* stream);
+
+/*
  * Element-wise glue of the Llama block (HF transformers modeling_llama.py), bit-identical to the eager chains it replaces.
  * dtype SOWB_BF16 or SOWB_F16; math in fp32, each result rounded to the 16-bit type where eager rounds (see glue.cu).
  * Pointers 16-byte aligned.  One launch per call.

@@ -107,6 +107,9 @@ SIGNATURES = {
     "sow_adam_multi": (_i, [_vp, _i, _d, _d, _d, _d, _d, _d, _d, _i, _i, _vp]),
     "sow_adam_multi_dev": (_i, [_vp, _i, _i64, _d, _d, _d, _d, _d, _vp, _i, _i, _vp]),
     "sow_adam_multi_amp": (_i, [_vp, _i, _i64, _d, _d, _d, _d, _d, _d, _d, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    "sow_adam_multi_clip": (_i, [_vp, _i, _i64, _d, _d, _d, _d, _d, _d, _d, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    "sow_grad_norm_partials": (_i, [_vp, _i, _i, _vp, _vp, _vp]),
+    "sow_grad_norm_finalize": (_i, [_vp, _i, _d, _vp, _vp, _vp]),
     "sow_rope_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i, _vp]),
     "sow_rope_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i, _vp]),
     "sow_swiglu_fwd": (_i, [_vp, _vp, _vp, _i64, _i, _vp]),

@@ -683,6 +683,63 @@ def adam_multi_amp(chunks: torch.Tensor, dtype: torch.dtype, state_dtype: torch.
     launch_counter["kernels"] += 1 if step_dev is None else 2
 
 
+def _check_scalar(fn: str, name: str, t: Optional[torch.Tensor], device: torch.device):
+    if t is not None and not (t.is_cuda and t.dtype == torch.float32 and t.numel() == 1 and t.device == device):
+        raise SowB200Error(f"{fn}: {name} must be a single-element fp32 tensor on {device}")
+
+
+def grad_norm(tables: Sequence[Tuple[torch.Tensor, torch.dtype]], partials: torch.Tensor, total_norm: torch.Tensor,
+              clip_coef: torch.Tensor, max_norm: float, grad_scale: Optional[torch.Tensor] = None):
+    """Global 2-norm of the gradients of several Adam chunk tables ``(chunks, gradient dtype)`` -- one partial per chunk
+    row into consecutive ranges of ``partials`` (fp32, at least one element per row in total), then one finalize -- and
+    the clip coefficient ``min(max_norm / (total_norm + 1e-6), 1)`` as torch computes it.  ``grad_scale``: the norm is
+    that of the unscaled gradients.  Writes ``total_norm`` and ``clip_coef`` (single-element fp32 device tensors)."""
+    lib = _lib.load()
+    dev = partials.device
+    _require_cuda(partials)
+    if partials.dtype != torch.float32 or not partials.is_contiguous():
+        raise SowB200Error("grad_norm: partials must be a contiguous fp32 tensor")
+    for name, t in (("total_norm", total_norm), ("clip_coef", clip_coef), ("grad_scale", grad_scale)):
+        _check_scalar("grad_norm", name, t, dev)
+    rows = sum(chunks.shape[0] for chunks, _ in tables)
+    if partials.numel() < max(rows, 1):
+        raise SowB200Error(f"grad_norm: {partials.numel()} partials for {rows} chunk rows")
+    off = 0
+    for chunks, dtype in tables:
+        if chunks.device != dev:
+            raise SowB200Error(f"grad_norm: chunk table on {chunks.device}, partials on {dev}")
+        n = chunks.shape[0]
+        if n:
+            rc = lib.sow_grad_norm_partials(_p(chunks), n, _dtype_code(dtype), _p(grad_scale),
+                                            ctypes.c_void_p(partials.data_ptr() + 4 * off), _stream_ptr(dev))
+            check(rc, "sow_grad_norm_partials")
+            launch_counter["kernels"] += 1
+        off += n
+    rc = lib.sow_grad_norm_finalize(_p(partials), max(rows, 1), float(max_norm), _p(total_norm), _p(clip_coef),
+                                    _stream_ptr(dev))
+    check(rc, "sow_grad_norm_finalize")
+    launch_counter["kernels"] += 1
+
+
+def adam_multi_clip(chunks: torch.Tensor, dtype: torch.dtype, state_dtype: torch.dtype, lr, beta1, beta2, eps, weight_decay,
+                    decoupled, clip_coef: torch.Tensor, bc1=1.0, bc2=1.0, step_dev: Optional[torch.Tensor] = None,
+                    grad_scale: Optional[torch.Tensor] = None, found_inf: Optional[torch.Tensor] = None):
+    """adam_multi_amp with the gradients multiplied by the device scalar ``clip_coef`` (after the unscale, each product
+    rounded to the gradient dtype) and written back, as ``unscale_`` + ``clip_grad_norm_`` leave them."""
+    lib = _lib.load()
+    if clip_coef is None:
+        raise SowB200Error("adam_multi_clip: clip_coef is required")
+    for name, t in (("step", step_dev), ("grad_scale", grad_scale), ("found_inf", found_inf), ("clip_coef", clip_coef)):
+        _check_scalar("adam_multi_clip", name, t, chunks.device)
+    total = getattr(chunks, "_sow_total_elems", 0)
+    rc = lib.sow_adam_multi_clip(_p(chunks), chunks.shape[0], total, float(lr), float(beta1), float(beta2), float(eps),
+                                 float(weight_decay), float(bc1), float(bc2), _p(step_dev), _p(grad_scale), _p(found_inf),
+                                 _p(clip_coef), 1 if decoupled else 0, _dtype_code(dtype), _dtype_code(state_dtype),
+                                 _stream_ptr(chunks.device))
+    check(rc, "sow_adam_multi_clip")
+    launch_counter["kernels"] += 1 if step_dev is None else 2
+
+
 # ---------------------------------------------------------------------------------------------------------
 # Llama block glue: rotary embedding and SwiGLU (bit-identical to the eager HF chains; sow_b200/llama_glue.py)
 # ---------------------------------------------------------------------------------------------------------

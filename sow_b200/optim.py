@@ -329,6 +329,16 @@ def _check_state_dtype(param_dtype: torch.dtype, state_dtype) -> None:
                        "(None = the parameter dtype, or torch.float32 for bf16 / fp16 parameters)")
 
 
+def _check_max_grad_norm(max_grad_norm):
+    """FusedAdamW's per-group clipping threshold: ``None`` (no clipping) or a finite number > 0, returned as a float."""
+    if max_grad_norm is None:
+        return None
+    if (isinstance(max_grad_norm, bool) or not isinstance(max_grad_norm, (int, float)) or not math.isfinite(max_grad_norm)
+            or max_grad_norm <= 0):
+        raise SowB200Error(f"FusedAdamW: max_grad_norm must be None or a finite float > 0, not {max_grad_norm!r}")
+    return float(max_grad_norm)
+
+
 class FusedAdamW(torch.optim.Optimizer):
     """Multi-tensor AdamW / Adam on one kernel launch per param group (SURVEY.md 8f rank 1).
 
@@ -350,24 +360,55 @@ class FusedAdamW(torch.optim.Optimizer):
     torch's fused AdamW does) and, for capturable groups, skips a step with found_inf on the device: no host sync, so a
     loss-scaled step can be captured in a CUDA graph.  Non-capturable groups read found_inf once on the host and leave
     parameters, moments and ``step`` untouched when it is set.
+
+    ``max_grad_norm`` (per group): clip the group's gradients by their global 2-norm before the update, as
+    ``torch.nn.utils.clip_grad_norm_(params, max_grad_norm)`` would, with the norm and the coefficient computed on the
+    device (fp32 sums of squares, reduced in a fixed order: bit-reproducible, no host sync, graph-capturable).  The norm
+    covers every gradient of the group and, under GradScaler, is that of the unscaled gradients; the clipped (and unscaled)
+    gradients are written back to ``p.grad``.  ``grad_norm(group_index)`` returns the pre-clip norm of the last step.
     """
 
     _step_supports_amp_scaling = True
 
     def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, amsgrad=False,
-                 decoupled=True, capturable=False, state_dtype=None):
+                 decoupled=True, capturable=False, state_dtype=None, max_grad_norm=None):
         if amsgrad:
             raise SowB200Error("FusedAdamW: amsgrad is not implemented")
         defaults = dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay, amsgrad=amsgrad, decoupled=decoupled,
-                        capturable=capturable, state_dtype=state_dtype)
+                        capturable=capturable, state_dtype=state_dtype, max_grad_norm=max_grad_norm)
         super().__init__(params, defaults)
         self._tables = {}
+        self._clip = {}                         # group index -> partials buffer, total_norm and clip_coef (device)
 
     def add_param_group(self, param_group):
         super().add_param_group(param_group)
         group = self.param_groups[-1]
         for p in group["params"]:
             _check_state_dtype(p.dtype, group.get("state_dtype"))
+        _check_max_grad_norm(group.get("max_grad_norm"))
+
+    def grad_norm(self, group_index: int):
+        """The total 2-norm of group ``group_index``'s gradients before clipping, at its last clipped step (unscaled under
+        GradScaler; what ``clip_grad_norm_`` returns), as a 0-dim fp32 device tensor that the next clipped step overwrites.
+        No host sync.  ``None`` before the group's first clipped step."""
+        st = self._clip.get(group_index)
+        return None if st is None else st["total_norm"]
+
+    def _clip_coef(self, gi, tables, max_norm, grad_scale):
+        """Norm of the group's gradients over all its chunk tables ``(chunks, dtype)`` and the clip coefficient, into
+        per-group device buffers that are reused from step to step (a captured step keeps their addresses; the partials
+        are reallocated only when the row count changes, which rebuilds the chunk tables too)."""
+        device = tables[0][0].device
+        rows = max(1, sum(t.shape[0] for t, _ in tables))
+        st = self._clip.get(gi)
+        if st is None or st["total_norm"].device != device:
+            st = {"total_norm": torch.zeros((), dtype=torch.float32, device=device),
+                  "clip_coef": torch.ones((), dtype=torch.float32, device=device), "partials": None}
+            self._clip[gi] = st
+        if st["partials"] is None or st["partials"].numel() != rows:
+            st["partials"] = torch.zeros(rows, dtype=torch.float32, device=device)
+        ops.grad_norm(tables, st["partials"], st["total_norm"], st["clip_coef"], max_norm, grad_scale)
+        return st["clip_coef"]
 
     def load_state_dict(self, state_dict):
         """torch's load_state_dict casts every floating-point state tensor to the parameter dtype (through
@@ -399,11 +440,14 @@ class FusedAdamW(torch.optim.Optimizer):
                 st[k] = st[k].to(sdt)
 
     @staticmethod
-    def _grad(p, grad_scale):
+    def _grad(p, grad_scale, clip=False):
         if p.grad.dtype == p.dtype:
             return p.grad
         if grad_scale is not None:
             raise SowB200Error("FusedAdamW: loss-scaled gradients must have the parameter dtype (they are unscaled in place)")
+        if clip:
+            raise SowB200Error("FusedAdamW: the gradients of a max_grad_norm group must have the parameter dtype (they are "
+                               "clipped in place)")
         return p.grad.to(p.dtype)
 
     def _step_capturable(self, gi, group, grad_scale=None, found_inf=None):
@@ -411,6 +455,7 @@ class FusedAdamW(torch.optim.Optimizer):
         tensor) are folded back onto a shared counter restarted from that value."""
         beta1, beta2 = group["betas"]
         gsdt = group.get("state_dtype")
+        max_norm = _check_max_grad_norm(group.get("max_grad_norm"))
         by_dtype = {}
         for p in group["params"]:
             if p.grad is None:
@@ -419,8 +464,9 @@ class FusedAdamW(torch.optim.Optimizer):
                 raise SowB200Error("FusedAdamW needs CUDA parameters (no CPU fallback)")
             st = self.state[p]
             self._init_state(p, st, gsdt or p.dtype)
-            g = self._grad(p, grad_scale)
+            g = self._grad(p, grad_scale, max_norm is not None)
             by_dtype.setdefault(p.dtype, []).append((p, g, st))
+        launches = []
         for dtype, items in by_dtype.items():
             ckey = ("counter", gi, dtype)
             counter = self._tables.get(ckey)
@@ -447,12 +493,19 @@ class FusedAdamW(torch.optim.Optimizer):
                                                      [st["exp_avg"] for _, _, st in items],
                                                      [st["exp_avg_sq"] for _, _, st in items]))
                 self._tables[key] = cached
-            sdt = items[0][2]["exp_avg"].dtype
-            if sdt == dtype and grad_scale is None and found_inf is None:
-                ops.adam_multi_dev(cached[1], dtype, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
+            launches.append((dtype, items[0][2]["exp_avg"].dtype, counter, cached[1]))
+        # clipping: the norm spans every dtype bucket of the group, so it is complete before the first update
+        clip = (self._clip_coef(gi, [(t, d) for d, _, _, t in launches], max_norm, grad_scale)
+                if max_norm is not None and launches else None)
+        for dtype, sdt, counter, table in launches:
+            if clip is not None:
+                ops.adam_multi_clip(table, dtype, sdt, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
+                                    group["decoupled"], clip, step_dev=counter, grad_scale=grad_scale, found_inf=found_inf)
+            elif sdt == dtype and grad_scale is None and found_inf is None:
+                ops.adam_multi_dev(table, dtype, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
                                    counter, group["decoupled"])
             else:
-                ops.adam_multi_amp(cached[1], dtype, sdt, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
+                ops.adam_multi_amp(table, dtype, sdt, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
                                    group["decoupled"], step_dev=counter, grad_scale=grad_scale, found_inf=found_inf)
 
     @torch.no_grad()
@@ -476,6 +529,7 @@ class FusedAdamW(torch.optim.Optimizer):
                     continue
             buckets = {}
             gsdt = group.get("state_dtype")
+            max_norm = _check_max_grad_norm(group.get("max_grad_norm"))
             for p in group["params"]:
                 if p.grad is None:
                     continue
@@ -486,9 +540,10 @@ class FusedAdamW(torch.optim.Optimizer):
                 if st["step"] is None:
                     st["step"] = torch.zeros((), dtype=torch.float32)
                 st["step"] += 1
-                g = self._grad(p, grad_scale)
+                g = self._grad(p, grad_scale, max_norm is not None)
                 buckets.setdefault((int(st["step"]), p.dtype), []).append((p, g, st["exp_avg"], st["exp_avg_sq"]))
             beta1, beta2 = group["betas"]
+            launches = []
             for (step, dtype), items in buckets.items():
                 sig = tuple((p.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), p.numel()) for p, g, m, v in items)
                 key = (gi, dtype, len(items))
@@ -497,12 +552,19 @@ class FusedAdamW(torch.optim.Optimizer):
                     ps, gs, ms, vs = zip(*items)
                     cached = (sig, ops.build_adam_chunks([p.data for p in ps], list(gs), list(ms), list(vs)))
                     self._tables[key] = cached
-                sdt = items[0][2].dtype
-                if sdt == dtype and grad_scale is None:
-                    ops.adam_multi(cached[1], dtype, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
+                launches.append((step, dtype, items[0][2].dtype, cached[1]))
+            clip = (self._clip_coef(gi, [(t, d) for _, d, _, t in launches], max_norm, grad_scale)
+                    if max_norm is not None and launches else None)
+            for step, dtype, sdt, table in launches:
+                if clip is not None:
+                    ops.adam_multi_clip(table, dtype, sdt, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
+                                        group["decoupled"], clip, 1.0 - beta1 ** step, 1.0 - beta2 ** step,
+                                        grad_scale=grad_scale)
+                elif sdt == dtype and grad_scale is None:
+                    ops.adam_multi(table, dtype, group["lr"], beta1, beta2, group["eps"], group["weight_decay"],
                                    1.0 - beta1 ** step, 1.0 - beta2 ** step, group["decoupled"])
                 else:
-                    ops.adam_multi_amp(cached[1], dtype, sdt, group["lr"], beta1, beta2, group["eps"],
+                    ops.adam_multi_amp(table, dtype, sdt, group["lr"], beta1, beta2, group["eps"],
                                        group["weight_decay"], group["decoupled"], 1.0 - beta1 ** step, 1.0 - beta2 ** step,
                                        grad_scale=grad_scale)
         return loss

@@ -114,6 +114,7 @@ class TrainConfig:
     loss_scaling: bool = False           # dynamic loss scaling (torch.amp.GradScaler) for fp16 training; capturable optimizer
     loss_scale_init: float = 2.0 ** 16
     loss_scale_growth_interval: int = 2000
+    fused_grad_clipping: bool = False    # grad_clipping inside FusedAdamW (device norm: works with loss scaling and cuda_graph)
 
 
 class SoWTrainer:
@@ -129,7 +130,9 @@ class SoWTrainer:
         if cfg.loss_scaling and cfg.dtype == torch.bfloat16:
             raise ValueError("loss_scaling is not available for bf16 models: torch.amp.GradScaler has no bf16 inf / nan "
                              "check, and bf16 has fp32's exponent range, so its gradients need no scaling")
-        if cfg.loss_scaling and cfg.grad_clipping != 0.0:
+        if cfg.fused_grad_clipping and not cfg.fused_optimizer:
+            raise ValueError("fused_grad_clipping needs the fused optimizer (the norm is computed inside FusedAdamW.step)")
+        if cfg.loss_scaling and cfg.grad_clipping != 0.0 and not cfg.fused_grad_clipping:
             raise ValueError("loss_scaling with grad_clipping is not supported (the norm of scaled fp16 gradients "
                              "overflows)")
         self.cfg = cfg
@@ -173,6 +176,8 @@ class SoWTrainer:
         groups = []
         if self.trainable:
             groups.append({"params": self.trainable, "lr": cfg.lr, "weight_decay": cfg.weight_decay})
+            if cfg.fused_grad_clipping and cfg.grad_clipping != 0.0:
+                groups[-1]["max_grad_norm"] = cfg.grad_clipping       # the set clip_grad_norm_ clips (:631); not the factors
         self.sow_group_id = len(groups)
         groups.append({"params": self.special, "lr": cfg.sow_lr, "weight_decay": cfg.weight_decay})
         if cfg.cuda_graph and not cfg.fused_optimizer:
@@ -201,7 +206,9 @@ class SoWTrainer:
     # ---- CUDA-graph replay of the whole micro-step ------------------------------------------------------------
     def _graph_ok(self, attention_mask) -> bool:
         cfg = self.cfg
-        if not cfg.cuda_graph or attention_mask is not None or cfg.gradient_accumulation != 1 or cfg.grad_clipping != 0.0:
+        if not cfg.cuda_graph or attention_mask is not None or cfg.gradient_accumulation != 1:
+            return False
+        if cfg.grad_clipping != 0.0 and not cfg.fused_grad_clipping:
             return False
         nxt = self.update_step                 # a merge fires inside step() when this is a multiple of sow_accumulation
         return not (nxt > 0 and nxt % int(cfg.sow_accumulation) == 0)
@@ -281,8 +288,10 @@ class SoWTrainer:
             self.grad_sync.synchronize()      # DDP semantics: gradients are averaged on every micro-step (no no_sync)
         if self.global_step % G != 0:                                              # :628
             return loss.detach()
-        if cfg.grad_clipping != 0.0:
+        if cfg.grad_clipping != 0.0 and not cfg.fused_grad_clipping:
             torch.nn.utils.clip_grad_norm_(self.trainable, cfg.grad_clipping)      # :631
+        # fused_grad_clipping: the trainable group's norm and clip run inside optimizer.step, on the averaged gradients
+        # (after grad_sync.synchronize above), so every rank computes the same coefficient
         if self.scaler is not None:
             self.scaler.step(self.optimizer)   # a skipped step (inf / nan gradients) still counts as an update step
             self.scaler.update()
