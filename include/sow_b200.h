@@ -383,6 +383,19 @@ int sow_swiglu_fwd(const void* gate, const void* up, void* h, int64_t n, int dty
 int sow_swiglu_bwd(const void* dh, const void* gate, const void* up, void* dgate, void* dup, int64_t n, int dtype,
                    void* stream);
 
+/*
+ * LlamaRMSNorm over rows x width contiguous elements, bit-identical to the eager HF forward and its autograd backward:
+ *   sow_rmsnorm_fwd: rs = rsqrt(mean(x^2) + eps) per row (fp32, rows values), y = w * (x * rs)
+ *   sow_rmsnorm_bwd: dx from dy, x, w and the saved rs; when p is not null also p = dy * (x * rs), the per-element
+ *                    product whose sum over the rows is dw.
+ * width one of 128, 256, 512, 768, 1024, 2048, 3072, 4096; rows >= 16 unless width == 128 (torch's row sums take
+ * another order below that); x, w, y, dy, dx, p 16-byte aligned.  rows == 0 does nothing.
+ */
+int sow_rmsnorm_fwd(const void* x, const void* w, void* y, float* rs, int64_t rows, int width, float eps, int dtype,
+                    void* stream);
+int sow_rmsnorm_bwd(const void* dy, const void* x, const void* w, const float* rs, void* dx, void* p, int64_t rows,
+                    int width, int dtype, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -114,6 +114,8 @@ SIGNATURES = {
     "sow_rope_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i, _vp]),
     "sow_swiglu_fwd": (_i, [_vp, _vp, _vp, _i64, _i, _vp]),
     "sow_swiglu_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _vp]),
+    "sow_rmsnorm_fwd": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _f, _i, _vp]),
+    "sow_rmsnorm_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _vp]),
 }
 
 _lock = threading.Lock()

@@ -205,6 +205,166 @@ __global__ void __launch_bounds__(256) swiglu_bwd_kernel(const H* __restrict__ d
   }
 }
 
+// ---- RMSNorm (LlamaRMSNorm.forward and its autograd backward) ------------------------------------------------------
+//
+// Eager runs, per row of H elements (xf = f32(x), r16() = rounding to the 16-bit type, every other op an fp32 op):
+//   forward   ms = sum(xf * xf) * factor          (mean: torch's MeanOps multiplies by float(rows) / float(rows * H))
+//             rs = rsqrtf(ms + eps),  hb = r16(xf * rs),  y = r16(w * hb)
+//   backward  dh = f32(r16(dy * w)),  s = sum(dh * xf)
+//             gv = (s * -0.5) * ((rs * rs) * rs)              (rsqrt backward; pow(rs, 3) is rs * rs * rs)
+//             d2 = gv * (1 / H)                               (mean backward: torch divides by a scalar as a product
+//                                                             with its reciprocal)
+//             dx = r16(dh * rs + d2 * (xf * 2))               (the two gradients of xf, each product rounded to fp32)
+//             p  = r16(dy * hb), reduced over the rows to dw by torch itself (sum_to_size), as eager's engine does
+// The two row sums are torch's inner-dimension fp32 reductions, and at the shapes dispatched here (H a multiple of 128
+// up to 4096 and rows >= 16, or H == 128) their order is fixed (ATen/native/cuda/Reduce.cuh, setReduceConfig with
+// vectorised input): one warp per row, lane t keeps four accumulators j = 0..3 over the elements 128 k + 4 t + j in
+// ascending k, combines them as ((a0 + a1) + a2) + a3, then a shfl_down tree with offsets 16, 8, 4, 2, 1.  The kernels
+// below use exactly that mapping, with the row held in registers.  Every product is written with __fmul_rn / __fadd_rn
+// so that nvcc cannot contract a product and a sum into one FMA where eager rounds the product first.
+
+template <typename H>
+__device__ __forceinline__ void unpack4(uint2 v, float (&f)[4]) {
+  const typename Cvt<H>::H2* h2 = reinterpret_cast<const typename Cvt<H>::H2*>(&v);
+  const float2 a = Cvt<H>::to_f2(h2[0]), b = Cvt<H>::to_f2(h2[1]);
+  f[0] = a.x;
+  f[1] = a.y;
+  f[2] = b.x;
+  f[3] = b.y;
+}
+template <typename H>
+__device__ __forceinline__ uint2 pack4(const float (&f)[4]) {
+  uint2 v;
+  typename Cvt<H>::H2* h2 = reinterpret_cast<typename Cvt<H>::H2*>(&v);
+  h2[0] = Cvt<H>::from_f2(f[0], f[1]);
+  h2[1] = Cvt<H>::from_f2(f[2], f[3]);
+  return v;
+}
+
+// torch's row sum from the four per-lane accumulators; the result in every lane
+__device__ __forceinline__ float warp_row_sum(const float (&a)[4]) {
+  float v = __fadd_rn(__fadd_rn(__fadd_rn(a[0], a[1]), a[2]), a[3]);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = __fadd_rn(v, __shfl_down_sync(0xffffffffu, v, o));
+  return __shfl_sync(0xffffffffu, v, 0);
+}
+
+constexpr int kNormRowsPerBlock = 8;   // one warp per row
+
+// NK = H / 128: lane t holds the 4 NK elements 128 k + 4 t + j of its row
+template <typename H, int NK>
+__global__ void __launch_bounds__(32 * kNormRowsPerBlock) rmsnorm_fwd_kernel(const H* __restrict__ x,
+                                                                             const H* __restrict__ w, H* __restrict__ y,
+                                                                             float* __restrict__ rs_out, int64_t rows,
+                                                                             float factor, float eps) {
+  const int64_t row = int64_t(blockIdx.x) * kNormRowsPerBlock + (threadIdx.x >> 5);
+  if (row >= rows) return;
+  const int lane = threadIdx.x & 31;
+  const int64_t base = row * (NK * 128) + lane * 4;
+  uint2 xv[NK];
+#pragma unroll
+  for (int k = 0; k < NK; ++k) xv[k] = *reinterpret_cast<const uint2*>(x + base + k * 128);
+  float a[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+  for (int k = 0; k < NK; ++k) {
+    float f[4];
+    unpack4<H>(xv[k], f);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) a[j] = __fadd_rn(a[j], __fmul_rn(f[j], f[j]));
+  }
+  const float rs = rsqrtf(__fadd_rn(__fmul_rn(warp_row_sum(a), factor), eps));
+#pragma unroll
+  for (int k = 0; k < NK; ++k) {
+    float f[4], wf[4], o[4];
+    unpack4<H>(xv[k], f);
+    unpack4<H>(*reinterpret_cast<const uint2*>(w + lane * 4 + k * 128), wf);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) o[j] = __fmul_rn(wf[j], rnd<H>(__fmul_rn(f[j], rs)));
+    *reinterpret_cast<uint2*>(y + base + k * 128) = pack4<H>(o);
+  }
+  if (lane == 0) rs_out[row] = rs;
+}
+
+// p (the per-element weight-gradient product) is written only when it is not null
+template <typename H, int NK>
+__global__ void __launch_bounds__(32 * kNormRowsPerBlock) rmsnorm_bwd_kernel(const H* __restrict__ dy,
+                                                                             const H* __restrict__ x,
+                                                                             const H* __restrict__ w,
+                                                                             const float* __restrict__ rs_in,
+                                                                             H* __restrict__ dx, H* __restrict__ p,
+                                                                             int64_t rows, float inv_h) {
+  const int64_t row = int64_t(blockIdx.x) * kNormRowsPerBlock + (threadIdx.x >> 5);
+  if (row >= rows) return;
+  const int lane = threadIdx.x & 31;
+  const int64_t base = row * (NK * 128) + lane * 4;
+  uint2 xv[NK], dv[NK];
+#pragma unroll
+  for (int k = 0; k < NK; ++k) {
+    xv[k] = *reinterpret_cast<const uint2*>(x + base + k * 128);
+    dv[k] = *reinterpret_cast<const uint2*>(dy + base + k * 128);
+  }
+  const float rs = rs_in[row];
+  float a[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+  for (int k = 0; k < NK; ++k) {
+    float f[4], d[4], wf[4], dh[4];
+    unpack4<H>(xv[k], f);
+    unpack4<H>(dv[k], d);
+    unpack4<H>(*reinterpret_cast<const uint2*>(w + lane * 4 + k * 128), wf);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      dh[j] = rnd<H>(__fmul_rn(d[j], wf[j]));
+      a[j] = __fadd_rn(a[j], __fmul_rn(dh[j], f[j]));
+    }
+    if (p != nullptr) {
+      float pf[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) pf[j] = __fmul_rn(d[j], rnd<H>(__fmul_rn(f[j], rs)));
+      *reinterpret_cast<uint2*>(p + base + k * 128) = pack4<H>(pf);
+    }
+    dv[k] = pack4<H>(dh);   // dh is a 16-bit value: from here on dv holds it instead of dy
+  }
+  const float gv = __fmul_rn(__fmul_rn(warp_row_sum(a), -0.5f), __fmul_rn(__fmul_rn(rs, rs), rs));
+  const float d2 = __fmul_rn(gv, inv_h);
+#pragma unroll
+  for (int k = 0; k < NK; ++k) {
+    float f[4], dh[4], o[4];
+    unpack4<H>(xv[k], f);
+    unpack4<H>(dv[k], dh);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) o[j] = __fadd_rn(__fmul_rn(dh[j], rs), __fmul_rn(d2, __fmul_rn(f[j], 2.0f)));
+    *reinterpret_cast<uint2*>(dx + base + k * 128) = pack4<H>(o);
+  }
+}
+
+// calls f(std::integral_constant<int, H / 128>{}) for the widths that have kernels; false for any other width
+template <typename F>
+bool with_norm_width(int width, F&& f) {
+  switch (width) {
+    case 128: f(std::integral_constant<int, 1>{}); return true;
+    case 256: f(std::integral_constant<int, 2>{}); return true;
+    case 512: f(std::integral_constant<int, 4>{}); return true;
+    case 768: f(std::integral_constant<int, 6>{}); return true;
+    case 1024: f(std::integral_constant<int, 8>{}); return true;
+    case 2048: f(std::integral_constant<int, 16>{}); return true;
+    case 3072: f(std::integral_constant<int, 24>{}); return true;
+    case 4096: f(std::integral_constant<int, 32>{}); return true;
+    default: return false;
+  }
+}
+
+int rmsnorm_check(const char* fn, int64_t rows, int width, int dtype) {
+  SOWB_REQUIRE(dtype == SOWB_BF16 || dtype == SOWB_F16, "%s: dtype %d unsupported (bf16 / fp16)", fn, dtype);
+  SOWB_REQUIRE(rows >= 0, "%s: negative row count", fn);
+  SOWB_REQUIRE(with_norm_width(width, [](auto) {}),
+               "%s: width %d has no kernel (128, 256, 512, 768, 1024, 2048, 3072, 4096)", fn, width);
+  // below 16 rows torch's reduction uses wider blocks and another summation order (one row is the same for H == 128)
+  SOWB_REQUIRE(rows == 0 || rows >= 16 || width == 128, "%s: %lld rows: at least 16 are needed for width %d", fn,
+               static_cast<long long>(rows), width);
+  SOWB_REQUIRE(rows / kNormRowsPerBlock < (int64_t(1) << 31) - 1, "%s: too many rows", fn);
+  return SOWB_OK;
+}
+
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 int rope_launch(const char* fn, bool backward, const void* q, const void* k, const void* cos, const void* sin, void* q_out,
@@ -310,6 +470,57 @@ int sow_swiglu_bwd(const void* dh, const void* gate, const void* up, void* dgate
     swiglu_bwd_kernel<__half><<<blocks, 256, 0, stream>>>(static_cast<const __half*>(dh), static_cast<const __half*>(gate),
                                                           static_cast<const __half*>(up), static_cast<__half*>(dgate),
                                                           static_cast<__half*>(dup), n);
+  SOWB_CHECK_CUDA(cudaGetLastError());
+  return SOWB_OK;
+}
+
+int sow_rmsnorm_fwd(const void* x, const void* w, void* y, float* rs, int64_t rows, int width, float eps, int dtype,
+                    void* stream_) {
+  if (int rc = rmsnorm_check("sow_rmsnorm_fwd", rows, width, dtype)) return rc;
+  SOWB_REQUIRE(x && w && y && rs, "sow_rmsnorm_fwd: null pointer");
+  SOWB_REQUIRE(aligned16(x) && aligned16(w) && aligned16(y), "sow_rmsnorm_fwd: pointers must be 16-byte aligned");
+  if (rows == 0) return SOWB_OK;
+  if (int rc = ensure_context_for(x)) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const unsigned blocks = unsigned((rows + kNormRowsPerBlock - 1) / kNormRowsPerBlock);
+  const float factor = float(rows) / float(rows * width);   // torch's mean: float(outputs) / numel
+  with_norm_width(width, [&](auto nk) {
+    constexpr int NK = decltype(nk)::value;
+    if (dtype == SOWB_BF16)
+      rmsnorm_fwd_kernel<__nv_bfloat16, NK><<<blocks, 32 * kNormRowsPerBlock, 0, stream>>>(
+          static_cast<const __nv_bfloat16*>(x), static_cast<const __nv_bfloat16*>(w), static_cast<__nv_bfloat16*>(y), rs,
+          rows, factor, eps);
+    else
+      rmsnorm_fwd_kernel<__half, NK><<<blocks, 32 * kNormRowsPerBlock, 0, stream>>>(
+          static_cast<const __half*>(x), static_cast<const __half*>(w), static_cast<__half*>(y), rs, rows, factor, eps);
+  });
+  SOWB_CHECK_CUDA(cudaGetLastError());
+  return SOWB_OK;
+}
+
+int sow_rmsnorm_bwd(const void* dy, const void* x, const void* w, const float* rs, void* dx, void* p, int64_t rows,
+                    int width, int dtype, void* stream_) {
+  if (int rc = rmsnorm_check("sow_rmsnorm_bwd", rows, width, dtype)) return rc;
+  SOWB_REQUIRE(dy && x && w && rs && dx, "sow_rmsnorm_bwd: null pointer");
+  SOWB_REQUIRE(aligned16(dy) && aligned16(x) && aligned16(w) && aligned16(dx) && aligned16(p),
+               "sow_rmsnorm_bwd: pointers must be 16-byte aligned");
+  if (rows == 0) return SOWB_OK;
+  if (int rc = ensure_context_for(x)) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const unsigned blocks = unsigned((rows + kNormRowsPerBlock - 1) / kNormRowsPerBlock);
+  const float inv_h = 1.0f / float(width);   // torch's division by a scalar: a product with its reciprocal
+  with_norm_width(width, [&](auto nk) {
+    constexpr int NK = decltype(nk)::value;
+    if (dtype == SOWB_BF16)
+      rmsnorm_bwd_kernel<__nv_bfloat16, NK><<<blocks, 32 * kNormRowsPerBlock, 0, stream>>>(
+          static_cast<const __nv_bfloat16*>(dy), static_cast<const __nv_bfloat16*>(x),
+          static_cast<const __nv_bfloat16*>(w), rs, static_cast<__nv_bfloat16*>(dx), static_cast<__nv_bfloat16*>(p), rows,
+          inv_h);
+    else
+      rmsnorm_bwd_kernel<__half, NK><<<blocks, 32 * kNormRowsPerBlock, 0, stream>>>(
+          static_cast<const __half*>(dy), static_cast<const __half*>(x), static_cast<const __half*>(w), rs,
+          static_cast<__half*>(dx), static_cast<__half*>(p), rows, inv_h);
+  });
   SOWB_CHECK_CUDA(cudaGetLastError());
   return SOWB_OK;
 }

@@ -129,10 +129,71 @@ def _llama_mlp_forward(self, x):
     return self.down_proj(h)
 
 
+# ---- RMSNorm ---------------------------------------------------------------------------------------------------------
+
+_NORM_WIDTHS = (128, 256, 512, 768, 1024, 2048, 3072, 4096)   # the widths csrc/glue.cu has kernels for
+
+
+def _stock_rmsnorm(x, w, eps):
+    """LlamaRMSNorm.forward, op for op."""
+    h = x.to(torch.float32)
+    h = h * torch.rsqrt(h.pow(2).mean(-1, keepdim=True) + eps)
+    return w * h.to(x.dtype)
+
+
+class _RMSNorm(torch.autograd.Function):
+    """(x, w) -> w * (x * rsqrt(mean(x^2) + eps)) in one pass each way.  Saves x, w and one fp32 value per row, where
+    eager saves several fp32 copies of x."""
+
+    @staticmethod
+    def forward(ctx, x, w, eps):
+        y, rs = ops.rmsnorm_fwd(x, w, eps)
+        ctx.save_for_backward(x, w, rs)
+        ctx.eps = eps
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        x, w, rs = ctx.saved_tensors
+        want_w = ctx.needs_input_grad[1]
+        if not (dy.is_contiguous() and dy.data_ptr() % 16 == 0):
+            # eager's row sums follow the layout of dy: replay the stock chain for such a gradient
+            with torch.enable_grad():
+                xd, wd = x.detach().requires_grad_(True), w.detach().requires_grad_(want_w)
+                ins = (xd, wd) if want_w else (xd,)
+                gs = torch.autograd.grad(_stock_rmsnorm(xd, wd, ctx.eps), ins, dy)
+            return gs[0], gs[1] if want_w else None, None
+        dx, p = ops.rmsnorm_bwd(dy, x, w, rs, want_p=want_w)
+        # dw as eager's engine forms it: torch's own reduction of the bf16 / fp16 product over the leading dims
+        return dx, p.sum_to_size(w.shape) if want_w else None, None
+
+
+def rmsnorm_native_ok(x, w, eps) -> bool:
+    """True when the native kernels compute LlamaRMSNorm (weight w, epsilon eps) of x bit for bit."""
+    if not (isinstance(x, torch.Tensor) and isinstance(w, torch.Tensor) and isinstance(eps, (float, int))):
+        return False
+    if not x.is_cuda or x.dtype not in _HALF or w.dtype != x.dtype or w.device != x.device or w.dim() != 1:
+        return False
+    H = x.shape[-1] if x.dim() else 0
+    if H not in _NORM_WIDTHS or w.shape[0] != H or not (x.is_contiguous() and w.is_contiguous()):
+        return False
+    rows = x.numel() // H
+    # below 16 rows torch's row sums take another order (except at H = 128, where the order is the same)
+    return (rows >= 16 or H == 128) and x.data_ptr() % 16 == 0 and w.data_ptr() % 16 == 0
+
+
+def _llama_rmsnorm_forward(self, hidden_states):
+    """LlamaRMSNorm.forward through the native kernels where rmsnorm_native_ok holds."""
+    if not torch.compiler.is_compiling() and rmsnorm_native_ok(hidden_states, self.weight, self.variance_epsilon):
+        return _RMSNorm.apply(hidden_states, self.weight, self.variance_epsilon)
+    return type(self).forward(self, hidden_states)
+
+
 # ---- installation ----------------------------------------------------------------------------------------------------
 
 def install_llama_glue(model: nn.Module) -> int:
-    """Route the Llama blocks of ``model`` through the native glue.  Returns the number of MLPs newly switched over."""
+    """Route the Llama blocks of ``model`` through the native glue.  Returns the number of MLPs newly switched over
+    (the RMSNorms are switched over as well, uncounted)."""
     try:
         from transformers.models.llama import modeling_llama as ml
     except Exception:  # pragma: no cover - transformers is optional for the kernels themselves
@@ -145,6 +206,9 @@ def install_llama_glue(model: nn.Module) -> int:
             if getattr(m.__dict__.get("forward"), "__func__", None) is not _llama_mlp_forward:
                 m.forward = types.MethodType(_llama_mlp_forward, m)
                 n += 1
+        elif type(m).forward is ml.LlamaRMSNorm.forward and isinstance(m, ml.LlamaRMSNorm):
+            if getattr(m.__dict__.get("forward"), "__func__", None) is not _llama_rmsnorm_forward:
+                m.forward = types.MethodType(_llama_rmsnorm_forward, m)
     if has_attention:
         install_rope(ml)
     return n

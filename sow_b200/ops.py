@@ -821,6 +821,43 @@ def swiglu_bwd(dh: torch.Tensor, gate: torch.Tensor, up: torch.Tensor):
     return dgate, dup
 
 
+def _norm_args(fn: str, x: torch.Tensor, w: torch.Tensor, *others: torch.Tensor):
+    _require_cuda(x, w, *others)
+    if w.dim() != 1 or x.dim() < 1 or x.shape[-1] != w.shape[0] or any(t.shape != x.shape for t in others):
+        raise SowB200Error(f"{fn}: x {tuple(x.shape)} and w {tuple(w.shape)} do not match")
+    if any(t.dtype != x.dtype for t in (w, *others)):
+        raise SowB200Error(f"{fn}: x, w and the gradients must share one dtype")
+    return (_glue_contig(t) for t in (x, w, *others))
+
+
+def rmsnorm_fwd(x: torch.Tensor, w: torch.Tensor, eps: float):
+    """LlamaRMSNorm forward over the last dim: (y = w * (x * rs), rs = rsqrt(mean(x^2) + eps)), rs fp32 of shape
+    x.shape[:-1]."""
+    x, w = _norm_args("sow_rmsnorm_fwd", x, w)
+    y = torch.empty_like(x)
+    rs = torch.empty(x.shape[:-1], dtype=torch.float32, device=x.device)
+    rc = _lib.load().sow_rmsnorm_fwd(_p(x), _p(w), _p(y), _p(rs), rs.numel(), x.shape[-1], eps,
+                                     _glue_dtype_code(x.dtype), _stream_ptr(x.device))
+    check(rc, "sow_rmsnorm_fwd")
+    launch_counter["kernels"] += 1
+    return y, rs
+
+
+def rmsnorm_bwd(dy: torch.Tensor, x: torch.Tensor, w: torch.Tensor, rs: torch.Tensor, want_p: bool = True):
+    """(dx, p) of rmsnorm_fwd from the upstream gradient dy and the saved rs; p = dy * (x * rs) is the per-element
+    product whose sum over the rows is dw (None unless want_p)."""
+    x, w, dy = _norm_args("sow_rmsnorm_bwd", x, w, dy)
+    if rs.dtype != torch.float32 or rs.shape != x.shape[:-1] or not rs.is_contiguous():
+        raise SowB200Error("sow_rmsnorm_bwd: rs must be contiguous fp32 of shape x.shape[:-1]")
+    dx = torch.empty_like(x)
+    p = torch.empty_like(x) if want_p else None
+    rc = _lib.load().sow_rmsnorm_bwd(_p(dy), _p(x), _p(w), _p(rs), _p(dx), _p(p), rs.numel(), x.shape[-1],
+                                     _glue_dtype_code(x.dtype), _stream_ptr(x.device))
+    check(rc, "sow_rmsnorm_bwd")
+    launch_counter["kernels"] += 1
+    return dx, p
+
+
 # ---------------------------------------------------------------------------------------------------------
 # live profiling (bench.py)
 # ---------------------------------------------------------------------------------------------------------

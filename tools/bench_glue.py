@@ -1,12 +1,13 @@
 #!/usr/bin/env python
-"""Stock HF vs native (csrc/glue.cu) rotary embedding and SwiGLU of one Llama layer, forward and backward, at the bench
-shape (Llama-350M: batch 128 x seq 256, 16 heads of 64, intermediate 2736, bf16).
+"""Stock HF vs native (csrc/glue.cu) rotary embedding, SwiGLU and RMSNorm of one Llama layer, forward and backward, at the
+bench shape (Llama-350M: batch 128 x seq 256, hidden 1024 = 16 heads of 64, intermediate 2736, bf16).
 
     python tools/bench_glue.py [--batch 128] [--seq 256] [--iters 20] [--dtype bf16] [--out FILE]
 
 Each pass is timed with CUDA events over --iters repetitions after a warm-up.  The working set of every pass (>= 268 MB)
 is larger than the 126 MB L2, so each repetition reads from HBM.  Achieved bandwidth = the bytes the pass must move at
-least (every input read once, every output written once; cos / sin counted once) over its time, set against the HBM
+least (every input read once, every output written once; cos / sin and the norm weight counted once; the RMSNorm
+backward's bf16 product for the weight gradient, and torch's reduction of it, are not counted) over its time, set against the HBM
 peak: MEASURED_PEAKS.json when present, otherwise the rate of a 2 GiB device-to-device copy measured here.
 Prints one JSON line per pass plus one with the card, its power limit and the peak used.
 """
@@ -71,7 +72,7 @@ def main():
     import torch
     import torch.nn.functional as F
     from transformers.models.llama import modeling_llama as ml
-    from sow_b200.llama_glue import _RoPE, _SwiGLU
+    from sow_b200.llama_glue import _RMSNorm, _RoPE, _SwiGLU
 
     assert torch.cuda.is_available(), "bench_glue.py measures on the GPU"
     dt = torch.bfloat16 if args.dtype == "bf16" else torch.float16
@@ -96,6 +97,10 @@ def main():
     gate = torch.randn(B, S, I, device="cuda", generator=g).to(dt).requires_grad_(True)
     up = torch.randn(B, S, I, device="cuda", generator=g).to(dt).requires_grad_(True)
     dh = torch.randn(B, S, I, device="cuda", generator=g).to(dt)
+    norm = ml.LlamaRMSNorm(H * D, eps=1e-6).to("cuda", dt)
+    xn = torch.randn(B, S, H * D, device="cuda", generator=g).to(dt).requires_grad_(True)
+    dyn = torch.randn(B, S, H * D, device="cuda", generator=g).to(dt)
+    norm_n = B * S * H * D
     ops = {
         "rope": {
             "stock": lambda: stock_rope(q, k, cos, sin),
@@ -108,6 +113,13 @@ def main():
             "native": lambda: _SwiGLU.apply(gate, up),
             "bwd": lambda out: torch.autograd.grad(out, (gate, up), dh),
             "bytes": (3 * swi_n * 2, 5 * swi_n * 2),     # fwd: gate, up -> h; bwd: dh, gate, up -> dgate, dup
+        },
+        "rmsnorm": {
+            "stock": lambda: ml.LlamaRMSNorm.forward(norm, xn),
+            "native": lambda: _RMSNorm.apply(xn, norm.weight, norm.variance_epsilon),
+            "bwd": lambda out: torch.autograd.grad(out, (xn, norm.weight), dyn),
+            "bytes": (2 * norm_n * 2, 3 * norm_n * 2),   # fwd: x -> y; bwd: dy, x -> dx
+            "per_step": 2 * 24 + 1,
         },
     }
     for name, o in ops.items():
@@ -126,9 +138,12 @@ def main():
             lines.append(row)
         st, nat = lines[-2], lines[-1]
         nat["speedup_fwd_bwd"] = st["fwd_bwd_ms"] / nat["fwd_bwd_ms"]
+    # per step of Llama-350M: 24 layers, one rotary and one SwiGLU call each, two norms each plus the final norm
+    per_step = [o.get("per_step", 24) for o in ops.values()]
     lines.append({"card": card(), "hbm_peak_gbs": peak, "hbm_peak_source": peak_src, "iters": args.iters,
-                  "per_step_layers": 24,
-                  "per_step_saving_ms": 24 * sum(lines[i]["fwd_bwd_ms"] - lines[i + 1]["fwd_bwd_ms"] for i in (0, 2))})
+                  "per_step_calls": dict(zip(ops, per_step)),
+                  "per_step_saving_ms": sum(n * (lines[2 * i]["fwd_bwd_ms"] - lines[2 * i + 1]["fwd_bwd_ms"])
+                                            for i, n in enumerate(per_step))})
     for ln in lines:
         s = json.dumps(ln)
         print(s, flush=True)
