@@ -396,6 +396,21 @@ int sow_rmsnorm_fwd(const void* x, const void* w, void* y, float* rs, int64_t ro
 int sow_rmsnorm_bwd(const void* dy, const void* x, const void* w, const float* rs, void* dx, void* p, int64_t rows,
                     int width, int dtype, void* stream);
 
+/*
+ * Cross-entropy of rows x vocab contiguous 16-bit logits against int64 targets, bit-identical to torch's fp32
+ * log_softmax of the upcast logits and the backward of log_softmax + the upcast:
+ *   sow_ce_fwd: per row, fp32 row_max = max_j x_j, row_logsum = log(sum_j exp(x_j - row_max)) and
+ *               logp_t = (x_t - row_max) - row_logsum; logp_t = 0 for a target outside [0, vocab), whose row is not gathered
+ *   sow_ce_bwd: grad = d(sum_i dlogp_t[i] * logp_t[i]) / d logits (16-bit, the logits' shape) from the forward's row_max
+ *               and row_logsum; dlogp_t[i] is the NLL gradient of row i (0 for an ignored row)
+ * vocab a multiple of 8 in [16384, 32768] (torch's log_softmax reduces other widths in another order); logits and grad
+ * 16-byte aligned.  rows == 0 does nothing.
+ */
+int sow_ce_fwd(const void* logits, const int64_t* target, float* row_max, float* row_logsum, float* logp_t, int64_t rows,
+               int vocab, int dtype, void* stream);
+int sow_ce_bwd(const void* logits, const float* row_max, const float* row_logsum, const int64_t* target,
+               const float* dlogp_t, void* grad, int64_t rows, int vocab, int dtype, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

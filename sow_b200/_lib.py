@@ -116,6 +116,8 @@ SIGNATURES = {
     "sow_swiglu_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _vp]),
     "sow_rmsnorm_fwd": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _f, _i, _vp]),
     "sow_rmsnorm_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _vp]),
+    "sow_ce_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _vp]),
+    "sow_ce_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _vp]),
 }
 
 _lock = threading.Lock()

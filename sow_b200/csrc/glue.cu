@@ -26,6 +26,8 @@
 
 #include <cuda_fp16.h>
 
+#include <cfloat>
+
 namespace sowb {
 
 namespace {
@@ -337,6 +339,145 @@ __global__ void __launch_bounds__(32 * kNormRowsPerBlock) rmsnorm_bwd_kernel(con
   }
 }
 
+// ---- causal-LM cross-entropy (HF ForCausalLMLoss: F.cross_entropy(logits.float(), labels)) --------------------------
+//
+// Eager upcasts the (N, V) logits to fp32 and runs torch's log_softmax, nll_loss and their backwards over fp32 copies.
+// The kernels below read the 16-bit logits directly (the upcast is exact) and reproduce torch's fp32 results bit for bit.
+// Per row (x = f32(logits[i]), t = target, v = the NLL gradient of the row: -grad_loss / total_weight, or +0 if ignored):
+//   forward   m = max_j x_j,  s = sum_j expf(x_j - m),  ls = logf(s),  logp_t = (x_t - m) - ls
+//   backward  g_j = r16(fma(expf((x_j - m) - ls), -(0 + v), j == t ? v : +0))
+// torch's cunn_SoftMaxForward<ILP = 4> with its LogSoftMaxForwardEpilogue (ATen/native/cuda/SoftMax.cu) does the forward
+// sums; for fp32 rows of 16384 <= V <= 32768 it runs with one 1024-thread block per row (smaller rows take its warp,
+// register or shared-memory variants, which sum in other orders).  Its order, which ce_fwd_kernel copies:
+//   * thread t folds the float4 groups t + 1024 k (k < V / 4096) lane by lane, then the scalars V - V % 4096 + t + 1024 m;
+//   * m: fmaxf per thread from -FLT_MAX, then the block tree below; the order does not change a max;
+//   * s: from 0, s = s + expf(x - m), where nvcc fuses the last product of expf (2^i * ex2(f)) and the add into one FFMA,
+//     as in torch's build;
+//   * block tree: shfl_down 16, 8, 4, 2, 1 in each warp, warp totals through shared memory, the same tree in warp 0.
+// The NLL reduction over the rows is torch's own (nll_loss of the gathered (N, 1) logp_t, see llama_glue.py): its order
+// depends on N only.  In the backward torch's row sum of the NLL gradient is 0 + v (one non-zero entry; -0 becomes +0),
+// and its LogSoftMaxBackwardEpilogue, grad - expf(logp) * sum, compiles to a rounded expf and one FFMA: the __fmaf_rn
+// below.  The fp32 gradient is rounded to the 16-bit type as the backward of `.float()` does.  No --use_fast_math: expf
+// and logf are the libdevice ones torch calls.
+
+constexpr int kCeThreads = 1024;
+constexpr int kCeMaxVocab = 32768;
+constexpr int kCeMaxVec = kCeMaxVocab / (4 * kCeThreads);   // float4 groups per thread
+constexpr int kCeMaxTail = 4;                                // scalars per thread from the V % 4096 tail
+
+// torch's cuda_utils::BlockReduce followed by blockReduceWarp's broadcast of thread 0's value
+template <typename Op>
+__device__ __forceinline__ float ce_block_reduce(float v, float* smem, Op op, float identity) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = op(v, __shfl_down_sync(0xffffffffu, v, o));
+  __syncthreads();   // smem is reused by the next reduction
+  if (lane == 0) smem[warp] = v;
+  __syncthreads();
+  if (warp == 0) {
+    v = threadIdx.x < kCeThreads / 32 ? smem[lane] : identity;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = op(v, __shfl_down_sync(0xffffffffu, v, o));
+  }
+  if (threadIdx.x == 0) smem[0] = v;
+  __syncthreads();
+  return smem[0];
+}
+
+// one block per row, the row held in registers (at most 32 values per thread); writes the row's max, logf(sum) and
+// logp at the target (0 when the target is outside [0, V): ignored rows, which read nothing more)
+template <typename H>
+__global__ void __launch_bounds__(kCeThreads) ce_fwd_kernel(const H* __restrict__ logits, const int64_t* __restrict__ target,
+                                                           float* __restrict__ row_max, float* __restrict__ row_logsum,
+                                                           float* __restrict__ logp_t, int V) {
+  __shared__ float smem[kCeThreads / 32];
+  const int t = threadIdx.x;
+  const H* x = logits + int64_t(blockIdx.x) * V;
+  const int nvec = V / (4 * kCeThreads);
+  const int tail = nvec * 4 * kCeThreads;
+  uint2 xv[kCeMaxVec];
+  float xs[kCeMaxTail] = {};
+#pragma unroll
+  for (int k = 0; k < kCeMaxVec; ++k)
+    if (k < nvec) xv[k] = *reinterpret_cast<const uint2*>(x + 4 * (t + k * kCeThreads));
+#pragma unroll
+  for (int m = 0; m < kCeMaxTail; ++m)
+    if (tail + t + m * kCeThreads < V) xs[m] = Cvt<H>::to_f(x[tail + t + m * kCeThreads]);
+
+  float mx = -FLT_MAX;
+#pragma unroll
+  for (int k = 0; k < kCeMaxVec; ++k)
+    if (k < nvec) {
+      float f[4];
+      unpack4<H>(xv[k], f);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) mx = fmaxf(mx, f[j]);
+    }
+#pragma unroll
+  for (int m = 0; m < kCeMaxTail; ++m)
+    if (tail + t + m * kCeThreads < V) mx = fmaxf(mx, xs[m]);
+  mx = ce_block_reduce(mx, smem, [](float a, float b) { return a < b ? b : a; }, -FLT_MAX);
+
+  float s = 0.0f;
+#pragma unroll
+  for (int k = 0; k < kCeMaxVec; ++k)
+    if (k < nvec) {
+      float f[4];
+      unpack4<H>(xv[k], f);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) s = s + expf(f[j] - mx);
+    }
+#pragma unroll
+  for (int m = 0; m < kCeMaxTail; ++m)
+    if (tail + t + m * kCeThreads < V) s = s + expf(xs[m] - mx);
+  s = ce_block_reduce(s, smem, [](float a, float b) { return a + b; }, 0.0f);
+
+  if (t == 0) {
+    const float ls = logf(s);
+    const int64_t tg = target[blockIdx.x];
+    row_max[blockIdx.x] = mx;
+    row_logsum[blockIdx.x] = ls;
+    logp_t[blockIdx.x] = (tg >= 0 && tg < V) ? (Cvt<H>::to_f(x[tg]) - mx) - ls : 0.0f;
+  }
+}
+
+constexpr int kCeBwdThreads = 256;   // 8 elements (16 bytes) per thread; a row takes ceil(V / 2048) blocks
+
+template <typename H>
+__global__ void __launch_bounds__(kCeBwdThreads) ce_bwd_kernel(const H* __restrict__ logits,
+                                                              const float* __restrict__ row_max,
+                                                              const float* __restrict__ row_logsum,
+                                                              const int64_t* __restrict__ target,
+                                                              const float* __restrict__ dlogp_t, H* __restrict__ grad, int V,
+                                                              int blocks_per_row) {
+  const int row = blockIdx.x / blocks_per_row;
+  const int c = (blockIdx.x - row * blocks_per_row) * kCeBwdThreads + threadIdx.x;
+  if (c * 8 >= V) return;
+  const float mx = row_max[row], ls = row_logsum[row], v = dlogp_t[row];
+  const float sum = 0.0f + v;
+  const int64_t tg = target[row];
+  const int64_t off = int64_t(row) * V + c * 8;
+  float f[8];
+  load8<H>(logits + off, f);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    const float go = (c * 8 + j == tg) ? v : 0.0f;
+    f[j] = __fmaf_rn(expf((f[j] - mx) - ls), -sum, go);
+  }
+  store8<H>(grad + off, f);
+}
+
+int ce_check(const char* fn, int64_t rows, int vocab, int dtype) {
+  SOWB_REQUIRE(dtype == SOWB_BF16 || dtype == SOWB_F16, "%s: dtype %d unsupported (bf16 / fp16)", fn, dtype);
+  SOWB_REQUIRE(rows >= 0, "%s: negative row count", fn);
+  // below 16384 torch's log_softmax reduces in another order; above 32768 a row does not fit the registers
+  SOWB_REQUIRE(vocab >= 16384 && vocab <= kCeMaxVocab && vocab % 8 == 0,
+               "%s: vocabulary %d unsupported (a multiple of 8 in [16384, %d])", fn, vocab, kCeMaxVocab);
+  SOWB_REQUIRE(rows < (int64_t(1) << 31) / ((vocab + 8 * kCeBwdThreads - 1) / (8 * kCeBwdThreads)), "%s: too many rows",
+               fn);
+  return SOWB_OK;
+}
+
 // calls f(std::integral_constant<int, H / 128>{}) for the widths that have kernels; false for any other width
 template <typename F>
 bool with_norm_width(int width, F&& f) {
@@ -521,6 +662,45 @@ int sow_rmsnorm_bwd(const void* dy, const void* x, const void* w, const float* r
           static_cast<const __half*>(dy), static_cast<const __half*>(x), static_cast<const __half*>(w), rs,
           static_cast<__half*>(dx), static_cast<__half*>(p), rows, inv_h);
   });
+  SOWB_CHECK_CUDA(cudaGetLastError());
+  return SOWB_OK;
+}
+
+int sow_ce_fwd(const void* logits, const int64_t* target, float* row_max, float* row_logsum, float* logp_t, int64_t rows,
+               int vocab, int dtype, void* stream_) {
+  if (int rc = ce_check("sow_ce_fwd", rows, vocab, dtype)) return rc;
+  SOWB_REQUIRE(logits && target && row_max && row_logsum && logp_t, "sow_ce_fwd: null pointer");
+  SOWB_REQUIRE(aligned16(logits), "sow_ce_fwd: logits must be 16-byte aligned");
+  if (rows == 0) return SOWB_OK;
+  if (int rc = ensure_context_for(logits)) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (dtype == SOWB_BF16)
+    ce_fwd_kernel<__nv_bfloat16><<<unsigned(rows), kCeThreads, 0, stream>>>(
+        static_cast<const __nv_bfloat16*>(logits), target, row_max, row_logsum, logp_t, vocab);
+  else
+    ce_fwd_kernel<__half><<<unsigned(rows), kCeThreads, 0, stream>>>(static_cast<const __half*>(logits), target, row_max,
+                                                                     row_logsum, logp_t, vocab);
+  SOWB_CHECK_CUDA(cudaGetLastError());
+  return SOWB_OK;
+}
+
+int sow_ce_bwd(const void* logits, const float* row_max, const float* row_logsum, const int64_t* target,
+               const float* dlogp_t, void* grad, int64_t rows, int vocab, int dtype, void* stream_) {
+  if (int rc = ce_check("sow_ce_bwd", rows, vocab, dtype)) return rc;
+  SOWB_REQUIRE(logits && row_max && row_logsum && target && dlogp_t && grad, "sow_ce_bwd: null pointer");
+  SOWB_REQUIRE(aligned16(logits) && aligned16(grad), "sow_ce_bwd: logits and grad must be 16-byte aligned");
+  if (rows == 0) return SOWB_OK;
+  if (int rc = ensure_context_for(logits)) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const int bpr = (vocab + 8 * kCeBwdThreads - 1) / (8 * kCeBwdThreads);
+  const unsigned blocks = unsigned(rows * bpr);
+  if (dtype == SOWB_BF16)
+    ce_bwd_kernel<__nv_bfloat16><<<blocks, kCeBwdThreads, 0, stream>>>(
+        static_cast<const __nv_bfloat16*>(logits), row_max, row_logsum, target, dlogp_t,
+        static_cast<__nv_bfloat16*>(grad), vocab, bpr);
+  else
+    ce_bwd_kernel<__half><<<blocks, kCeBwdThreads, 0, stream>>>(static_cast<const __half*>(logits), row_max, row_logsum,
+                                                                target, dlogp_t, static_cast<__half*>(grad), vocab, bpr);
   SOWB_CHECK_CUDA(cudaGetLastError());
   return SOWB_OK;
 }

@@ -10,16 +10,21 @@ are bit-identical to the stock functions (and a training run is unchanged bit fo
     ``up_proj(x)`` (the order eager uses, which the shared-input SoW group relies on) and the fused gate.
   * RoPE: HF's attention looks ``apply_rotary_pos_emb`` up in the ``modeling_llama`` module globals; that global is
     replaced by a dispatcher that keeps the stock function.  Installing twice changes nothing.
+  * RMSNorm: every ``LlamaRMSNorm`` gets a per-instance ``forward``.
+  * Loss: every ``LlamaForCausalLM`` whose ``loss_function`` is HF's ``ForCausalLMLoss`` gets ``CausalLMLoss`` (which
+    keeps the stock function as ``.stock``) through the ``loss_function`` setter.
 The native path runs only for CUDA bf16 / fp16 tensors of the expected layouts, cos / sin without grad,
 ``unsqueeze_dim == 1``, and outside ``torch.compile`` tracing; every other call runs the stock function, so compiled
 models (inductor fuses these chains itself) and fp32 models are exactly as before.
 """
 from __future__ import annotations
 
+import os
 import types
 
 import torch
 import torch.nn as nn
+import torch.nn.functional as F
 
 from . import ops
 
@@ -189,11 +194,98 @@ def _llama_rmsnorm_forward(self, hidden_states):
     return type(self).forward(self, hidden_states)
 
 
+# ---- causal-LM loss --------------------------------------------------------------------------------------------------
+
+_LOSS_VOCAB = (16384, 32768)   # widths (multiples of 8) whose torch log_softmax sums in ce_fwd_kernel's order (glue.cu)
+
+
+class _CausalLMLoss(torch.autograd.Function):
+    """(logits (N, V) bf16 / fp16, targets (N,) int64) -> logp_t (N, 1) fp32, log_softmax(logits.float()) at each row's
+    target.  Saves the logits and two fp32 values per row, where eager keeps an fp32 copy of the logits and their fp32
+    log_softmax."""
+
+    @staticmethod
+    def forward(ctx, logits, targets):
+        row_max, row_logsum, logp_t = ops.ce_fwd(logits, targets)
+        ctx.save_for_backward(logits, targets, row_max, row_logsum)
+        return logp_t.unsqueeze(1)
+
+    @staticmethod
+    def backward(ctx, g):
+        logits, targets, row_max, row_logsum = ctx.saved_tensors
+        return ops.ce_bwd(logits, row_max, row_logsum, targets, g[:, 0]), None
+
+
+def loss_native_ok(logits, labels, vocab_size, ignore_index=-100, shifted=False) -> bool:
+    """True when the native kernels compute ForCausalLMLoss(logits, labels, vocab_size, ignore_index=ignore_index) bit
+    for bit (``shifted``: labels are the already shifted ``shift_labels``)."""
+    if not (isinstance(logits, torch.Tensor) and isinstance(labels, torch.Tensor) and isinstance(vocab_size, int)
+            and isinstance(ignore_index, int)):
+        return False
+    if not logits.is_cuda or logits.dtype not in _HALF or labels.dtype != torch.int64 or logits.dim() < 2:
+        return False
+    V = logits.shape[-1]
+    if V != vocab_size or V % 8 or not _LOSS_VOCAB[0] <= V <= _LOSS_VOCAB[1] or 0 <= ignore_index < V:
+        return False
+    if labels.numel() != logits.numel() // V or (not shifted and labels.shape != logits.shape[:-1]):
+        return False
+    return logits.is_contiguous() and logits.data_ptr() % 16 == 0
+
+
+class CausalLMLoss:
+    """ForCausalLMLoss with HF's signature: the native kernels where loss_native_ok holds (and SOWB_NATIVE_LOSS is not
+    0), ``stock`` otherwise.
+
+    The native path shifts the labels as HF does, gathers logp_t = log_softmax(logits.float())[i, t_i] for every row
+    (ops.ce_fwd) and hands that (N, 1) column to torch's own nll_loss, with target 0 for a valid row and the label itself
+    otherwise.  nll_loss sums over the rows in an order that depends on N only, so the loss, its total weight and the
+    per-row gradient it passes back are torch's, bit for bit; ops.ce_bwd turns that gradient into the logits' gradient."""
+
+    def __init__(self, stock):
+        self.stock = stock
+
+    def __call__(self, logits, labels, vocab_size, num_items_in_batch=None, ignore_index=-100, shift_labels=None,
+                 **kwargs):
+        if (torch.compiler.is_compiling() or os.environ.get("SOWB_NATIVE_LOSS", "1") == "0"
+                or not loss_native_ok(logits, labels if shift_labels is None else shift_labels, vocab_size,
+                                      ignore_index, shifted=shift_labels is not None)):
+            return self.stock(logits, labels, vocab_size, num_items_in_batch=num_items_in_batch,
+                              ignore_index=ignore_index, shift_labels=shift_labels, **kwargs)
+        if shift_labels is None:
+            labels = F.pad(labels, (0, 1), value=ignore_index)
+            shift_labels = labels[..., 1:].contiguous()
+        logits = logits.view(-1, vocab_size)
+        targets = shift_labels.view(-1).to(logits.device)
+        logp_t = _CausalLMLoss.apply(logits, targets)
+        # a label outside [0, V) is ignore_index (ignored here too) or invalid (nll_loss rejects it, as it does in eager)
+        nll_targets = torch.where((targets >= 0) & (targets < vocab_size), 0, targets)
+        reduction = "sum" if num_items_in_batch is not None else "mean"
+        loss = F.nll_loss(logp_t, nll_targets, ignore_index=ignore_index, reduction=reduction)
+        if reduction == "sum":
+            if torch.is_tensor(num_items_in_batch):
+                num_items_in_batch = num_items_in_batch.to(loss.device)
+            loss = loss / num_items_in_batch
+        return loss
+
+
+def install_loss(model: nn.Module) -> bool:
+    """Route ``model.loss_function`` (HF's ForCausalLMLoss) through CausalLMLoss, once.  Returns True if installed now."""
+    try:
+        from transformers.loss.loss_utils import ForCausalLMLoss
+    except Exception:  # pragma: no cover - older transformers
+        return False
+    cur = model.loss_function
+    if cur is not ForCausalLMLoss:    # another loss, or already installed
+        return False
+    model.loss_function = CausalLMLoss(cur)
+    return True
+
+
 # ---- installation ----------------------------------------------------------------------------------------------------
 
 def install_llama_glue(model: nn.Module) -> int:
     """Route the Llama blocks of ``model`` through the native glue.  Returns the number of MLPs newly switched over
-    (the RMSNorms are switched over as well, uncounted)."""
+    (the RMSNorms and the causal-LM loss are switched over as well, uncounted)."""
     try:
         from transformers.models.llama import modeling_llama as ml
     except Exception:  # pragma: no cover - transformers is optional for the kernels themselves
@@ -202,6 +294,8 @@ def install_llama_glue(model: nn.Module) -> int:
     for m in model.modules():
         if isinstance(m, ml.LlamaAttention):
             has_attention = True
+        elif isinstance(m, ml.LlamaForCausalLM):
+            install_loss(m)
         elif type(m).forward is ml.LlamaMLP.forward and isinstance(m, ml.LlamaMLP) and _is_silu(m.act_fn):
             if getattr(m.__dict__.get("forward"), "__func__", None) is not _llama_mlp_forward:
                 m.forward = types.MethodType(_llama_mlp_forward, m)

@@ -858,6 +858,41 @@ def rmsnorm_bwd(dy: torch.Tensor, x: torch.Tensor, w: torch.Tensor, rs: torch.Te
     return dx, p
 
 
+def _ce_args(fn: str, logits: torch.Tensor, target: torch.Tensor, *rows: torch.Tensor):
+    _require_cuda(logits, target, *rows)
+    if logits.dim() != 2 or target.shape != logits.shape[:1] or any(t.shape != target.shape for t in rows):
+        raise SowB200Error(f"{fn}: logits {tuple(logits.shape)} and targets {tuple(target.shape)} do not match")
+    if target.dtype != torch.int64 or any(t.dtype != torch.float32 for t in rows):
+        raise SowB200Error(f"{fn}: targets must be int64 and the row values fp32")
+    return _glue_contig(logits), target.contiguous(), *(t.contiguous() for t in rows)
+
+
+def ce_fwd(logits: torch.Tensor, target: torch.Tensor):
+    """Row statistics of log_softmax(logits.float()) for (N, V) logits and (N,) int64 targets: fp32 (row_max, row_logsum,
+    logp_t), logp_t[i] = log_softmax(logits)[i, target[i]] (0 where the target is outside [0, V))."""
+    logits, target = _ce_args("sow_ce_fwd", logits, target)
+    N, V = logits.shape
+    row_max, row_logsum, logp_t = (torch.empty(N, dtype=torch.float32, device=logits.device) for _ in range(3))
+    rc = _lib.load().sow_ce_fwd(_p(logits), _p(target), _p(row_max), _p(row_logsum), _p(logp_t), N, V,
+                                _glue_dtype_code(logits.dtype), _stream_ptr(logits.device))
+    check(rc, "sow_ce_fwd")
+    launch_counter["kernels"] += 1
+    return row_max, row_logsum, logp_t
+
+
+def ce_bwd(logits: torch.Tensor, row_max: torch.Tensor, row_logsum: torch.Tensor, target: torch.Tensor,
+           dlogp_t: torch.Tensor) -> torch.Tensor:
+    """Gradient w.r.t. the logits (their dtype, (N, V)) of sum_i dlogp_t[i] * logp_t[i], with ce_fwd's row statistics."""
+    logits, target, row_max, row_logsum, dlogp_t = _ce_args("sow_ce_bwd", logits, target, row_max, row_logsum, dlogp_t)
+    N, V = logits.shape
+    grad = torch.empty_like(logits)
+    rc = _lib.load().sow_ce_bwd(_p(logits), _p(row_max), _p(row_logsum), _p(target), _p(dlogp_t), _p(grad), N, V,
+                                _glue_dtype_code(logits.dtype), _stream_ptr(logits.device))
+    check(rc, "sow_ce_bwd")
+    launch_counter["kernels"] += 1
+    return grad
+
+
 # ---------------------------------------------------------------------------------------------------------
 # live profiling (bench.py)
 # ---------------------------------------------------------------------------------------------------------
