@@ -164,14 +164,48 @@ struct Segment {
   int K;
 };
 
+// resident clusters of the CTA-pair GEMM (sow_gemm_pair_kernel) on the current device; every instantiation has the same
+// resources, so one query serves all of them
+static int pair_max_clusters() {
+  static std::mutex mu;
+  static int cache[64] = {0};
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
+  std::lock_guard<std::mutex> lk(mu);
+  if (cache[dev] == 0) {
+    int n = 0;
+    set_max_smem_once(sow_gemm_pair_kernel<true, false>, size_t(GemmPairSmem::kTotal));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(2 * num_sms());
+    cfg.blockDim = dim3(kGemmThreads);
+    cfg.dynamicSmemBytes = GemmPairSmem::kTotal;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = 2;
+    at[0].val.clusterDim.y = 1;
+    at[0].val.clusterDim.z = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = 1;
+    if (cudaOccupancyMaxActiveClusters(&n, sow_gemm_pair_kernel<true, false>, &cfg) != cudaSuccess || n <= 0) {
+      cudaGetLastError();
+      n = std::max(1, num_sms() / 2);
+    }
+    cache[dev] = n;
+  }
+  return cache[dev];
+}
+
 // Operand A of D = A.B: logical [M, K].  K-major  <=> stored [M rows, K cols];  MN-major <=> stored [K rows, M cols].
 // Operand B of D = A.B: logical [K, N].  K-major  <=> stored [N rows, K cols];  MN-major <=> stored [K rows, N cols].
 // f16: the 16-bit operands (and a 16-bit C / bias) are fp16, else bf16.
-template <int BN, bool A_MN, bool B_MN, int EPI, int MT = 1>
+// PAIR: the work item is a 256 x 256 tile computed by a cluster of two CTAs (sow_gemm_pair_kernel); BN = 256, MT = 1,
+// A K-major, EPI_BF16_TMA only.
+template <int BN, bool A_MN, bool B_MN, int EPI, int MT = 1, bool PAIR = false>
 static int launch_gemm(const Segment* segs, int nseg, void* C_bf16, float* C_f32, int ldc, int M, int N,
                        const float* alpha_blocks, int n_alpha, const void* bias, bool split_k, bool f16, cudaStream_t stream,
                        int prof_class, double alg_flops, int* splits_out = nullptr) {
   using S = GemmSmem<BN, MT>;
+  static_assert(!PAIR || (BN == 256 && MT == 1 && !A_MN && EPI == EPI_BF16_TMA), "pair tiles: 256 wide, A K-major, 16-bit out");
   if (nseg < 1 || nseg > kMaxSeg) return set_error(SOWB_EINVAL, "launch_gemm: %d segments (max %d)", nseg, kMaxSeg);
   GemmMaps maps;
   GemmParams p;
@@ -182,7 +216,7 @@ static int launch_gemm(const Segment* segs, int nseg, void* C_bf16, float* C_f32
     const Segment& sg = segs[s < nseg ? s : 0];
     rc = make_tensor_map_2d(&maps.a[s], sg.A.ptr, sg.A.cols, sg.A.rows, sg.A.pitch_elems * 2, 64, A_MN ? 64 : kBM, t16);
     if (rc) return rc;
-    rc = make_tensor_map_2d(&maps.b[s], sg.B.ptr, sg.B.cols, sg.B.rows, sg.B.pitch_elems * 2, 64, B_MN ? 64 : BN, t16);
+    rc = make_tensor_map_2d(&maps.b[s], sg.B.ptr, sg.B.cols, sg.B.rows, sg.B.pitch_elems * 2, 64, B_MN ? 64 : (PAIR ? BN / 2 : BN), t16);
     if (rc) return rc;
     if (s < nseg) kb += ceil_div(sg.K, kBK);
     p.kb_end[s] = kb;
@@ -198,7 +232,7 @@ static int launch_gemm(const Segment* segs, int nseg, void* C_bf16, float* C_f32
   p.M = M;
   p.N = N;
   p.nseg = nseg;
-  p.m_tiles = ceil_div(M, kBM * MT);      // work rows: MT tiles of 128 rows each
+  p.m_tiles = ceil_div(M, kBM * MT * (PAIR ? 2 : 1));      // work rows: MT tiles of 128 rows each (two CTAs' for PAIR)
   p.n_tiles = ceil_div(N, BN);
   const int kb_total = kb;
   const int sms = num_sms();
@@ -220,6 +254,26 @@ static int launch_gemm(const Segment* segs, int nseg, void* C_bf16, float* C_f32
   if (splits_out) *splits_out = p.splits;
   const int total = p.m_tiles * p.n_tiles * p.splits;
   if (total <= 0 || kb_total <= 0) return SOWB_OK;
+  if constexpr (PAIR) {
+    auto kern = f16 ? sow_gemm_pair_kernel<B_MN, true> : sow_gemm_pair_kernel<B_MN, false>;
+    SOWB_CHECK_CUDA(set_max_smem_once(kern, size_t(GemmPairSmem::kTotal)));
+    const int clusters = std::min(total, pair_max_clusters());
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(2 * clusters);
+    cfg.blockDim = dim3(kGemmThreads);
+    cfg.dynamicSmemBytes = GemmPairSmem::kTotal;
+    cfg.stream = stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = 2;
+    at[0].val.clusterDim.y = 1;
+    at[0].val.clusterDim.z = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = 1;
+    ProfileScope prof(stream, prof_class, alg_flops);
+    SOWB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, maps, p));
+    return SOWB_OK;
+  }
   auto kern = sow_gemm_kernel<BN, A_MN, B_MN, EPI, MT, false>;
   if constexpr (EPI != EPI_F32_TMA) {   // the bf16x3 path of fp32 modules has bf16 operands only
     if (f16) kern = sow_gemm_kernel<BN, A_MN, B_MN, EPI, MT, true>;
@@ -250,6 +304,19 @@ static bool use_big_tiles(int M, int N, int kb_total) {
   const int sms = num_sms();
   const int waves = ceil_div(items, sms);
   return kb_total >= 32 && items >= 2 * sms && double(items) / (double(waves) * sms) >= 0.93;
+}
+
+// CTA-pair 256 x 256 tiles (sow_gemm_pair_kernel) take every 16-bit forward y_i and group dX that the rules above leave on the
+// 128 x 256 tile.  They keep the same number of SMs busy as the 128 x 256 tiles (a pair tile is two CTAs) with a third less
+// operand traffic per MAC, so they are used at every size (small T was not timed separately).  Measured at T = 32768
+// (tools/bench_group.py): 7-18 % less time per launch for every Llama-350M forward and dX.  SOWB_GEMM_PAIR=0 restores the
+// 128 x 256 tile (for A/B runs).
+static bool use_pair_tiles() {
+  static const bool on = []() {
+    const char* e = getenv("SOWB_GEMM_PAIR");
+    return e == nullptr || atoi(e) != 0;
+  }();
+  return on;
 }
 
 // number of split-K partials launch_gemm<BN, ..., EPI_F32_PARTIAL> produces for an [M x N] output contracted over K
@@ -508,6 +575,9 @@ int sow_group_fwd(const void* x, const void* x_lo, const sowb_group_member* m, i
     else if (use_big_tiles(static_cast<int>(T), m[i].out, ceil_div(in, kBK) * (m[i].W != nullptr) + L.rpad[i] / kBK))
       rc = launch_gemm<256, false, true, EPI_BF16_TMA, 2>(segs, ns, m[i].y, nullptr, m[i].out, static_cast<int>(T), m[i].out,
                                                           &one, 1, m[i].bias, false, f16, stream, PROF_GEMM_FWD, fl);
+    else if (use_pair_tiles())
+      rc = launch_gemm<256, false, true, EPI_BF16_TMA, 1, true>(segs, ns, m[i].y, nullptr, m[i].out, static_cast<int>(T), m[i].out,
+                                                                &one, 1, m[i].bias, false, f16, stream, PROF_GEMM_FWD, fl);
     else
       rc = launch_gemm<256, false, true, EPI_BF16_TMA>(segs, ns, m[i].y, nullptr, m[i].out, static_cast<int>(T), m[i].out,
                                                        &one, 1, m[i].bias, false, f16, stream, PROF_GEMM_FWD, fl);
@@ -743,6 +813,9 @@ int sow_group_bwd(const void* x, const void* A_cat, const void* t_cat, const sow
     else if (use_big_tiles(Ti, in, static_cast<int>(kalg) / kBK))
       rc = launch_gemm<256, false, false, EPI_BF16_TMA, 2>(segs, ns, dx, nullptr, in, Ti, in, &one, 1, nullptr, false, f16, stream,
                                                            PROF_GEMM_DX, 2.0 * double(T) * double(in) * kalg);
+    else if (use_pair_tiles())
+      rc = launch_gemm<256, false, false, EPI_BF16_TMA, 1, true>(segs, ns, dx, nullptr, in, Ti, in, &one, 1, nullptr, false, f16,
+                                                                 stream, PROF_GEMM_DX, 2.0 * double(T) * double(in) * kalg);
     else
       rc = launch_gemm<256, false, false, EPI_BF16_TMA>(segs, ns, dx, nullptr, in, Ti, in, &one, 1, nullptr, false, f16, stream,
                                                         PROF_GEMM_DX, 2.0 * double(T) * double(in) * kalg);

@@ -196,6 +196,52 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
                : "memory");
 }
 
+// ---- CTA pairs (cta_group::2): two CTAs of a cluster (ranks 2j, 2j+1) share one MMA -------------------------------------
+// Allocation and deallocation are collective over one warp of EACH CTA of the pair; both get the same TMEM address.
+__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_dst, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)),
+               "r"(ncols)
+               : "memory");
+}
+__device__ __forceinline__ void tmem_relinquish_pair() {
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+// Issued by one thread of the even CTA: A (M = 256) is rows 0..127 from the even CTA's smem and 128..255 from the odd CTA's,
+// B's N columns are split in halves the same way (the descriptors are offsets valid in both CTAs); D is each CTA's own
+// 128 TMEM lanes x N columns at tmem_d.
+__device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                               uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// Arrive once on the mbarrier at the same smem offset in every CTA of cta_mask, when all earlier pair MMAs have completed.
+__device__ __forceinline__ void umma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
+  asm volatile(
+      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+          smem_u32(bar)),
+      "h"(cta_mask)
+      : "memory");
+}
+// 2-D tiled load into THIS CTA's smem whose completed bytes are counted on `cluster_bar`, a shared::cluster address that
+// may be the peer CTA's barrier (the even CTA of the pair counts both CTAs' bytes).
+__device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const CUtensorMap* m, uint32_t cluster_bar, int32_t c0,
+                                                 int32_t c1) {
+  asm volatile(
+      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+      ::"r"(smem_u32(smem_dst)),
+      "l"(reinterpret_cast<uint64_t>(m)), "r"(cluster_bar), "r"(c0), "r"(c1)
+      : "memory");
+}
+
 // TMEM -> registers: this warp's 32 lanes x 32 consecutive fp32 columns.
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
   asm volatile(
